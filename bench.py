@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the hot path (BASELINE.json): Mrays/s over all logical ray types and frame ms,
 bun69k 4K (3840x2160) 16 spp, on N B200s, beside the CPU restatement of the reference on the host cores.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one full frame of the workload through the wavefront kernels.
   value    : whole-job throughput with the scene resident in HBM and the frame left on rank 0's device (NCCL chunk gather included for N>1)
@@ -52,6 +52,7 @@ METRIC = WORKLOAD["metric"]
 CHUNK_ROWS = 8
 SAMPLE_STRIDE = 16            # bounded CPU sample = every 16th 8-row chunk of the frame (the pixel set of rank 0 of 16)
 ACCEL_NAMES = ["reference-topology literal", "reference-topology fast", "lbvh"]
+DUMP_PIXELS = 1 << 21         # --dump-outputs: pixels kept of a larger frame (4 float32 channels + a float64 index: 48 MiB)
 
 
 def make_config(w, world, accel, has_photons):
@@ -111,6 +112,20 @@ class ClockSampler:
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None, "reasons": reasons, "samples": len(self.rows)}
 
 
+def dump_outputs(out_dir, frame_host, ray_types):
+    """What the timed step hands its caller, as .npy files for comparing two builds output for output: the frame's A, R, G, B channels
+    (float32; when the frame has more than DUMP_PIXELS pixels, the same seeded sample of them every run, their indices in frame_pixel_index)
+    and the logical ray counts of the step (float64, in the order of ray_types_per_frame)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n = frame_host.size
+    idx = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(0).choice(n, DUMP_PIXELS, replace=False))
+    px = frame_host.astype(np.uint32)[idx]
+    np.save(os.path.join(out_dir, "frame_argb.npy"), np.stack([(px >> s) & 255 for s in (24, 16, 8, 0)], axis=1).astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "ray_counts.npy"), np.array(list(ray_types.values()), dtype=np.float64))
+
+
 def oracle_scene():
     from oracle import orc
     orc.build()
@@ -168,6 +183,7 @@ def main():
     ap.add_argument("--photons", type=int, default=None, help="photons cast per light for the photon workloads (sweep 1M..64M)")
     ap.add_argument("--res", default=None, help="COLSxROWS override")
     ap.add_argument("--spp", type=int, default=None)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the frame and ray counts of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
     global METRIC
     if args.workload == "synth":
@@ -257,6 +273,8 @@ def main():
         import zlib
         frame_host = frame.cpu().numpy()
         frame_crc = "%08x" % (zlib.crc32(frame_host.tobytes()) & 0xffffffff)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, frame_host, ray_types)
     ms_per_step = sum(gpu_ms) / len(gpu_ms)
     value = rays / (ms_per_step / 1e3) / 1e6
 
