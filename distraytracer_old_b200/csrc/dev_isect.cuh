@@ -26,8 +26,10 @@ struct alignas(16) Hit {
 };
 // what a primitive test reports; the caller fills the Hit record only for candidates that win
 struct PHit { double t; int32_t arg0, arg1, state, boxRaw; };
+// pad0 during a closest-hit search: 2 (list child index + 1) + boxRaw, where the winner came from (closestHitT forms loc / rawDir from it)
 __device__ __forceinline__ void takeHit(const DScene& S, Hit& dst, const PHit& ph, int primIdx, const Ray& r, D3 rawDir, int hitXform) {
   dst.t = ph.t; dst.prim = primIdx; dst.arg0 = ph.arg0; dst.arg1 = ph.arg1; dst.state = ph.state; dst.hitXform = hitXform; dst.shaderOverride = -1; dst.inst = -1;
+  dst.pad0 = ph.boxRaw ? 1 : 0;
   dst.loc = d3((r.d.x * ph.t) + r.o.x, (r.d.y * ph.t) + r.o.y, (r.d.z * ph.t) + r.o.z);       // transRay.pointOnRay(t), myRay.java:82-87
   // rendered box: the direction recorded in the hit is CTM x transformed direction (myGeomBase.java:160)
   dst.rawDir = ph.boxRaw ? xfVector(S.xforms[S.prims[primIdx].xform].m, r.d) : rawDir;
@@ -681,11 +683,12 @@ __device__ __noinline__ double boxStdEntry(const double* __restrict__ box6, doub
 // may be skipped against the best hit only if te * tScale >= bestT.  1 when |ba| >= 1 (te itself is then the conservative bound).
 __device__ __forceinline__ float leanScale(double len2) { return len2 >= 1.0 ? 1.0f : __double2float_rd(sqrt(len2)) * 0.999999f; }
 template <int CAP>
-__device__ DRT_LEAN_INLINE int leanClosest32(const DScene& S, const FBvh& B, const D3 bo, const D3 ba, const D3 binv, const D3 to, const D3 td, const D3 rawDir, Hit& out, const float tScale = 1.0f) {
+__device__ DRT_LEAN_INLINE int leanClosest32(const DScene& S, const FBvh& B, const D3 bo, const D3 ba, const D3 binv, const D3 to, const D3 td, const D3 rawDir, Hit& out, const double bound, const float tScale = 1.0f) {
   const Lean32 L = makeLean32(B, bo.x, bo.y, bo.z, binv);
   const bool stdBox = S.accelMode == 2;
   uint2 stkE[CAP]; int sp = 0; bool overflow = false;
-  double bestT = DRT_DMAX; float bestTf = __int_as_float(0x7f800000);        // bestTf = bestT / tScale rounded UP: te_lb >= bestTf implies te * tScale >= bestT
+  // bestTf = bestT / tScale rounded UP: te_lb >= bestTf implies te * tScale >= bestT (the callers without a bound fold this to +inf)
+  double bestT = bound; float bestTf = bound < DRT_DMAX ? __fdiv_ru(__double2float_ru(bound), tScale) : __int_as_float(0x7f800000);
   int bestTri = -1, bestRank = 0x7fffffff, bestSt = 0;
   int32_t ref = B.fastRoot; bool alive = true;
   auto popNext = [&]() { alive = false; while (sp > 0) { const uint2 e = stkE[--sp]; if (__uint_as_float(e.y) < bestTf) { ref = (int32_t)e.x; alive = true; break; } } };
@@ -728,8 +731,8 @@ __device__ DRT_LEAN_INLINE int leanClosest32(const DScene& S, const FBvh& B, con
     popNext();
   }
   if (overflow) return -1;
-  if (bestTri < 0) return 0;
-  out.t = bestT; out.prim = S.tris[bestTri].prim; out.arg0 = 0; out.arg1 = 0; out.state = bestSt; out.hitXform = B.triHitXform; out.shaderOverride = -1; out.inst = -1;
+  if (bestTri < 0 || !(bestT < bound)) return 0;
+  out.t = bestT; out.prim = S.tris[bestTri].prim; out.arg0 = 0; out.arg1 = 0; out.state = bestSt; out.hitXform = B.triHitXform; out.shaderOverride = -1; out.inst = -1; out.pad0 = 0;
   out.loc = d3((td.x * bestT) + to.x, (td.y * bestT) + to.y, (td.z * bestT) + to.z); out.rawDir = rawDir; return 1;
 }
 template <int CAP>
@@ -792,14 +795,14 @@ struct Frame { int32_t node; double tL; };     // node >= 0: "after left" of tha
 // closest hit.  Every function returns 1 (hit), 0 (miss) or -1 (this kernel variant cannot serve the ray: defer it)
 // ---------------------------------------------------------------------------------------------------------------
 template <int F, int LVL>
-__device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int idx, Ray& _ray, const Ray& trans, int transXf, double time, Hit& out, TraceCounters* tc);
+__device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int idx, Ray& _ray, const Ray& trans, int transXf, double time, Hit& out, TraceCounters* tc, double bound);
 // the generic variant keeps one outlined copy per level (code size); the lean variants inline everything so that ray / hit records stay in registers
 template <int F, int LVL>
-__device__ __noinline__ int accelClosestOut(const DScene& S, int kind, int idx, Ray& _ray, const Ray& trans, int transXf, double time, Hit& out, TraceCounters* tc) { return accelClosestImpl<F, LVL>(S, kind, idx, _ray, trans, transXf, time, out, tc); }
+__device__ __noinline__ int accelClosestOut(const DScene& S, int kind, int idx, Ray& _ray, const Ray& trans, int transXf, double time, Hit& out, TraceCounters* tc, double bound) { return accelClosestImpl<F, LVL>(S, kind, idx, _ray, trans, transXf, time, out, tc, bound); }
 template <int F, int LVL>
-__device__ __forceinline__ int accelClosest(const DScene& S, int kind, int idx, Ray& _ray, const Ray& trans, int transXf, double time, Hit& out, TraceCounters* tc) {
-  if constexpr (F == TF_ALL) return accelClosestOut<F, LVL>(S, kind, idx, _ray, trans, transXf, time, out, tc);
-  else return accelClosestImpl<F, LVL>(S, kind, idx, _ray, trans, transXf, time, out, tc);
+__device__ __forceinline__ int accelClosest(const DScene& S, int kind, int idx, Ray& _ray, const Ray& trans, int transXf, double time, Hit& out, TraceCounters* tc, double bound) {
+  if constexpr (F == TF_ALL) return accelClosestOut<F, LVL>(S, kind, idx, _ray, trans, transXf, time, out, tc, bound);
+  else return accelClosestImpl<F, LVL>(S, kind, idx, _ray, trans, transXf, time, out, tc, bound);
 }
 
 // myGeomList.traverseStruct: every child gets a fresh transform of `_ray`; first strictly smaller t wins;
@@ -811,25 +814,25 @@ __device__ __forceinline__ const Ray& xfRayCached(const DScene& S, Ray& _ray, in
   return xc.r;
 }
 template <int F, int LVL>
-__device__ __forceinline__ double leafClosest(const DScene& S, int listIdx, Ray& _ray, double time, Hit& res, TraceCounters* tc, XfCache& xc, bool& defer) {
+__device__ __forceinline__ double leafClosest(const DScene& S, int listIdx, Ray& _ray, double time, Hit& res, TraceCounters* tc, XfCache& xc, bool& defer, double bound) {
   const FList L = S.lists[listIdx];
-  double clsT = DRT_DMAX;
+  double clsT = bound;
   for (int i = 0; i < L.childCount; ++i) {
     const FObjRef c = S.children[L.childStart + i];
     Ray r = xfRayCached(S, _ray, c.xform, xc);
     if (c.kind == OK_PRIM) {
       PHit ph; if (tc) ++tc->prim;
-      if (primTest(S, c.idx, r, time, ph) && ph.t < clsT) { clsT = ph.t; takeHit(S, res, ph, c.idx, r, _ray.d, c.hitXform); }
+      if (primTest(S, c.idx, r, time, ph) && ph.t < clsT) { clsT = ph.t; takeHit(S, res, ph, c.idx, r, _ray.d, c.hitXform); res.pad0 += 2 * (L.childStart + i + 1); }
     } else {   // instance: the already transformed ray is forwarded as both rays (mySceneObject.java:123-127)
       const FInstance I = S.instances[c.idx];
       if (I.baseKind == OK_PRIM) {
         PHit ph; if (tc) ++tc->prim;
-        if (primTest(S, I.baseIdx, r, time, ph) && ph.t < clsT) { clsT = ph.t; takeHit(S, res, ph, I.baseIdx, r, r.d, c.hitXform); if (I.shader >= 0) res.shaderOverride = I.shader; res.inst = I.serial; }
+        if (primTest(S, I.baseIdx, r, time, ph) && ph.t < clsT) { clsT = ph.t; takeHit(S, res, ph, I.baseIdx, r, r.d, c.hitXform); res.pad0 += 2 * (L.childStart + i + 1); if (I.shader >= 0) res.shaderOverride = I.shader; res.inst = I.serial; }
       } else if constexpr (LVL == 1) {
         if constexpr (!(F & TF_LITERAL1)) { defer = true; return clsT; }
         else {
           Hit h; hitReset(h);
-          const int got = accelClosest<F, 2>(S, I.baseKind, I.baseIdx, r, r, -1, time, h, tc);
+          const int got = accelClosest<F, 2>(S, I.baseKind, I.baseIdx, r, r, -1, time, h, tc, DRT_DMAX);
           if (got < 0) { defer = true; return clsT; }
           if (got && h.t < clsT) {
             clsT = h.t; res.t = h.t; res.prim = h.prim; res.arg0 = h.arg0; res.arg1 = h.arg1; res.state = h.state; res.loc = h.loc; res.rawDir = h.rawDir;
@@ -848,7 +851,7 @@ __device__ __forceinline__ double leafClosest(const DScene& S, int listIdx, Ray&
 // combines with "min, left wins ties", the overall winner is the DFS-first minimum over all visited leaves; the
 // per-subtree minima needed for the pruning decisions live on an explicit frame stack.
 template <int F, int LVL>
-__device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int idx, Ray& _ray, const Ray& trans, int transXf, double time, Hit& out, TraceCounters* tc) {
+__device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int idx, Ray& _ray, const Ray& trans, int transXf, double time, Hit& out, TraceCounters* tc, double bound) {
   constexpr bool LITERAL = (LVL == 1) ? ((F & TF_LITERAL1) != 0) : ((F & TF_LEVEL2) != 0);      // literal recursion compiled in at this level?
   constexpr bool NONLEAN = (LVL == 1) ? ((F & TF_NONLEAN) != 0) : ((F & TF_LEVEL2) != 0);
   const D3 inv = rayInv(trans);
@@ -857,9 +860,9 @@ __device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int i
     if (tc) ++tc->box;
     if (!boxHit(L.bmin, L.bmax, trans, inv)) return 0;
     XfCache xc; xc.xf = -1; bool defer = false;
-    double t = leafClosest<F, LVL>(S, idx, _ray, time, out, tc, xc, defer);
+    double t = leafClosest<F, LVL>(S, idx, _ray, time, out, tc, xc, defer, bound);
     if (defer) return -1;
-    return t < DRT_DMAX ? 1 : 0;
+    return t < bound ? 1 : 0;
   }
   const FBvh& B = S.bvhs[idx];
   if (tc) ++tc->box;
@@ -883,8 +886,8 @@ __device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int i
           return got;
         } else {
 #if DRT_LEAN32
-          if constexpr ((F & TF_LITERAL1) != 0) return leanClosest32<DRT_LSTACK>(S, B, trans.o, trans.a, inv, r.o, r.d, _ray.d, out, leanScale(len2));
-          else { if (!one) return -1; return leanClosest32<DRT_LSTACK>(S, B, trans.o, trans.a, inv, trans.o, trans.a, _ray.d, out); }      // flat scenes: one ray, one register set
+          if constexpr ((F & TF_LITERAL1) != 0) return leanClosest32<DRT_LSTACK>(S, B, trans.o, trans.a, inv, r.o, r.d, _ray.d, out, bound, leanScale(len2));
+          else { if (!one) return -1; return leanClosest32<DRT_LSTACK>(S, B, trans.o, trans.a, inv, trans.o, trans.a, _ray.d, out, bound); }      // flat scenes: one ray, one register set
 #else
           if constexpr ((F & TF_LITERAL1) != 0) return leanClosest<false, DRT_LSTACK>(S, B, trans.o, trans.a, r.o, r.d, _ray.d, out, tc);
           else { if (!one) return -1; return leanClosest<true, DRT_LSTACK>(S, B, trans.o, trans.a, r.o, r.d, _ray.d, out, tc); }
@@ -907,7 +910,7 @@ __device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int i
     bool ret = false;
     int32_t afterLeftOf = -1;
     if (node < 0) {                    // leaf
-      tCur = leafClosest<F, LVL>(S, ~node, _ray, time, leaf, tc, xc, defer);
+      tCur = leafClosest<F, LVL>(S, ~node, _ray, time, leaf, tc, xc, defer, DRT_DMAX);
       if (defer) return -1;
       if (tCur < best.t) { best.t = leaf.t; best.prim = leaf.prim; best.arg0 = leaf.arg0; best.arg1 = leaf.arg1; best.state = leaf.state; best.hitXform = leaf.hitXform;
         best.shaderOverride = leaf.shaderOverride; best.inst = leaf.inst; best.loc = leaf.loc; best.rawDir = leaf.rawDir; }
@@ -938,13 +941,21 @@ __device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int i
   }
 }
 
-// myScene.findClosestRayHit: linear scan of the top-level list, first-inserted wins among equal t
+// myScene.findClosestRayHit: linear scan of the top-level list, first-inserted wins among equal t.
+// The accel searches take `bound`: they write their winner to the record they are given only if it is strictly closer than bound -- the same
+// decision as "h.t < best.t" on a separate record.  The flat lean variants (no literal recursion, no generic descent: every search they reach
+// honours bound) pass `best` itself, so a single Hit lives across the BVH walk instead of two, and they carry only the winner's key across
+// it: which top-level object (wTop) and, in best.pad0, which list child produced it.  Its hit point and recorded direction are formed once,
+// after the loop, from the same transformed ray the winning test used: getTransformedRay is a pure function of (unit-length ray, CTM), so the
+// recomputed ray has the bits the loop had.
 template <int F>
 __device__ __forceinline__ int closestHitT(const DScene& S, Ray& ray, double time, Hit& best, TraceCounters* tc) {
+  constexpr bool IN_PLACE = DRT_LEAN && DRT_LEAN32 && (F & (TF_LITERAL1 | TF_NONLEAN)) == 0;
   hitReset(best);
-  Hit h; hitReset(h);
+  Hit h; if constexpr (!IN_PLACE) hitReset(h);
   Ray tr; int trXf = -1;        // consecutive top-level objects often share one CTM (a polygon soup read under one transform): the transformed
                                 // ray is a pure function of (ray, CTM), and `ray` is already unit length here, so it is formed once per run
+  int wTop = -1;
   for (int i = 0; i < S.g.numTop; ++i) {
     const FObjRef o = S.top[i];
     if (o.xform != trXf || o.kind != OK_PRIM) { tr = xfRay(ray, S.xforms[o.xform].inv); trXf = (o.kind == OK_PRIM) ? o.xform : -1; }
@@ -953,24 +964,47 @@ __device__ __forceinline__ int closestHitT(const DScene& S, Ray& ray, double tim
       const int triIdx = (S.accelMode != 0) ? S.prims[o.idx].pad0 : -1;      // packed record of a plain top-level triangle (fast modes)
       if (triIdx >= 0) {
         int32_t rank; ph.arg0 = 0; ph.arg1 = 0; ph.boxRaw = 0;
-        if (leanTri(S.tris + triIdx, tr.o.x, tr.o.y, tr.o.z, tr.d.x, tr.d.y, tr.d.z, best.t, ph.t, ph.state, rank) && ph.t < best.t) takeHit(S, best, ph, o.idx, tr, ray.d, o.xform);
-      } else if (primTest(S, o.idx, tr, time, ph) && ph.t < best.t) takeHit(S, best, ph, o.idx, tr, ray.d, o.xform);
+        if (leanTri(S.tris + triIdx, tr.o.x, tr.o.y, tr.o.z, tr.d.x, tr.d.y, tr.d.z, best.t, ph.t, ph.state, rank) && ph.t < best.t) { takeHit(S, best, ph, o.idx, tr, ray.d, o.xform); wTop = i; }
+      } else if (primTest(S, o.idx, tr, time, ph) && ph.t < best.t) { takeHit(S, best, ph, o.idx, tr, ray.d, o.xform); wTop = i; }
     } else {
       int got; int shader = -1, serial = -1;
       if (o.kind == OK_INSTANCE) {
         const FInstance I = S.instances[o.idx]; shader = I.shader; serial = I.serial;
         if (I.baseKind == OK_PRIM) {
           PHit ph; if (tc) ++tc->prim;
-          if (primTest(S, I.baseIdx, tr, time, ph) && ph.t < best.t) { takeHit(S, best, ph, I.baseIdx, tr, tr.d, o.xform); if (shader >= 0) best.shaderOverride = shader; best.inst = serial; }
+          if (primTest(S, I.baseIdx, tr, time, ph) && ph.t < best.t) { takeHit(S, best, ph, I.baseIdx, tr, tr.d, o.xform); if (shader >= 0) best.shaderOverride = shader; best.inst = serial; wTop = i; }
           continue;
         }
-        got = accelClosest<F, 1>(S, I.baseKind, I.baseIdx, tr, tr, -1, time, h, tc);
-      } else got = accelClosest<F, 1>(S, o.kind, o.idx, ray, tr, o.xform, time, h, tc);
+        if constexpr (IN_PLACE) got = accelClosest<F, 1>(S, I.baseKind, I.baseIdx, tr, tr, -1, time, best, tc, best.t);
+        else got = accelClosest<F, 1>(S, I.baseKind, I.baseIdx, tr, tr, -1, time, h, tc, DRT_DMAX);
+      } else if constexpr (IN_PLACE) got = accelClosest<F, 1>(S, o.kind, o.idx, ray, tr, o.xform, time, best, tc, best.t);
+      else got = accelClosest<F, 1>(S, o.kind, o.idx, ray, tr, o.xform, time, h, tc, DRT_DMAX);
       if (got < 0) return -1;
-      if (got && h.t < best.t) {
+      if constexpr (IN_PLACE) {
+        if (got) { if (shader >= 0) best.shaderOverride = shader; if (serial >= 0 && best.inst < 0) best.inst = serial; wTop = i; }
+      } else if (got && h.t < best.t) {
         best.t = h.t; best.prim = h.prim; best.arg0 = h.arg0; best.arg1 = h.arg1; best.state = h.state; best.hitXform = h.hitXform; best.loc = h.loc; best.rawDir = h.rawDir;
         best.shaderOverride = (shader >= 0) ? shader : h.shaderOverride; best.inst = (serial >= 0 && h.inst < 0) ? serial : h.inst;
       }
+    }
+  }
+  if constexpr (IN_PLACE) {
+    best.loc = d3(0, 0, 0); best.rawDir = d3(0, 0, 0);
+    if (wTop >= 0) {
+      const FObjRef o = S.top[wTop];
+      Ray tr0 = xfRay(ray, S.xforms[o.xform].inv);
+      const int child = (best.pad0 >> 1) - 1; const bool boxRaw = (best.pad0 & 1) != 0;
+      Ray rt = tr0; D3 raw;
+      if (child >= 0) {           // primitive of a list (leafClosest): the list's ray -- renormalised in place through an instance -- under the child's CTM
+        Ray& src = (o.kind == OK_INSTANCE) ? tr0 : ray;
+        const FObjRef c = S.children[child];
+        rt = xfRay(src, S.xforms[c.xform].inv);
+        raw = (c.kind == OK_PRIM) ? src.d : rt.d;
+      } else if (o.kind == OK_INSTANCE) {
+        raw = (S.instances[o.idx].baseKind == OK_PRIM) ? tr0.d : norm3(tr0.d);    // instanced mesh: the lean search saw the renormalised ray
+      } else raw = ray.d;
+      best.loc = pointOnRay(rt, best.t);
+      best.rawDir = boxRaw ? xfVector(S.xforms[S.prims[best.prim].xform].m, rt.d) : raw;
     }
   }
   return best.t < DRT_DMAX ? 1 : 0;

@@ -72,6 +72,7 @@ __device__ __forceinline__ double urange(double u, double origin, double bound) 
 struct DScene {
   const FXform* xforms; const FPrim* prims; const double* pdata; const FObjRef* top; const FObjRef* children;
   const FInstance* instances; const FList* lists; const FBvh* bvhs; const FNode* nodes; const FLight* lights;
+  const double* lightPos;           // xfPoint(CTM, origin) of every light, 3 doubles each: formed on the device once per upload (k_light_pos)
   const FShader* shaders; const FTexture* textures; const double* texColors; const FImage* images; const int32_t* texels;
   // fast-BVH view: packed triangles and the node array their fastRoot indexes (== nodes, or the GPU-built LBVH nodes); accelMode = drt.h DRT_ACCEL_*
   const FTri* tris; const FNode* fnodes; const FNode32* fnodes32; int32_t accelMode; int32_t padA;

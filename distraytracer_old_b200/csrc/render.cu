@@ -31,7 +31,8 @@ struct alignas(16) SurfRec { double loc[3], n[3], rawDir[3], tex[3]; int32_t sha
 struct alignas(16) NodeRec { double local[3], cA[3], cB[3], w[3]; int32_t parent, slot; int32_t pad[2]; };
 
 // compact pixel index -> absolute pixel (row-major). Identity for single-GPU; interleaved row chunks for multi-GPU tiles.
-struct PixMap { long long chunkPix, totalPix; int world, rank; };
+// narrow != 0: the host checked that every ray index, pixel index and absolute pixel of the launch is below 2^31 (see renderChunks)
+struct PixMap { long long chunkPix, totalPix; int world, rank, narrow; };
 __host__ __device__ __forceinline__ long long absPixel(const PixMap& m, long long p) { return ((p / m.chunkPix) * m.world + m.rank) * m.chunkPix + (p % m.chunkPix); }
 
 // primaryS / shadowS: the two counters every warp bumps are spread over 64 slots (block index & 63) and summed on the host -- one address for
@@ -93,12 +94,25 @@ __device__ __forceinline__ void deferAppend(bool doIt, uint32_t idx, unsigned lo
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// primary ray of (pixel, sample) index i of the batch -- generated where it is needed (k_trace and k_shade at level 0) instead of being
-// written to and re-read from HBM
+// absolute pixel and sample of primary-ray index i of the batch.  With pm.narrow the divisions run on 32-bit integers (a 64-bit division is a
+// long subroutine, and there are up to four per ray): the same quotients, since every operand fits
+struct PixKey { long long pix; uint32_t smp; };
+__device__ __forceinline__ PixKey pixelOf(const FGlobals& g, const PixMap& pm, long long pix0, long long i) {
+  const int spp = g.spp < 1 ? 1 : g.spp; PixKey k;
+  if (pm.narrow) {
+    const uint32_t ii = (uint32_t)i, p = (uint32_t)pix0 + ii / (uint32_t)spp, c = (uint32_t)pm.chunkPix;
+    k.pix = (pm.world == 1) ? p : ((p / c) * (uint32_t)pm.world + (uint32_t)pm.rank) * c + p % c; k.smp = ii % (uint32_t)spp;
+  } else { k.pix = absPixel(pm, pix0 + i / spp); k.smp = (uint32_t)(i % spp); }
+  return k;
+}
+// primary ray of (pixel, sample) index i of the batch -- generated where it is needed (k_trace; k_shade only for a skydome miss) instead of
+// being written to and re-read from HBM
 __device__ __forceinline__ void primaryRay(const DScene& S, const PixMap& pm, long long pix0, long long i, RayRec& r) {
   const FGlobals& g = S.g; int spp = g.spp < 1 ? 1 : g.spp;
-  long long pix = absPixel(pm, pix0 + i / spp); uint32_t smp = (uint32_t)(i % spp);
-  int row = (int)(pix / g.cols), col = (int)(pix % g.cols);
+  const PixKey k = pixelOf(g, pm, pix0, i); const long long pix = k.pix; const uint32_t smp = k.smp;
+  int row, col;
+  if (pm.narrow) { row = (int)((uint32_t)pix / (uint32_t)g.cols); col = (int)((uint32_t)pix % (uint32_t)g.cols); }
+  else { row = (int)(pix / g.cols); col = (int)(pix % g.cols); }
   r.kt0 = 1; r.kt1 = 1; r.ka = (uint32_t)pix; r.kb = smp; r.kc = 1; r.stream = STREAM_PIXEL; r.gen = 0; r.valid = 1; r.pad[0] = r.pad[1] = 0;
   D3 o = d3(g.eye[0], g.eye[1], g.eye[2]), d = d3(0, 0, -1);
   auto U = [&](uint32_t dim) { return philoxU01(g.seed, STREAM_PIXEL, (uint32_t)pix, smp, 1, dim); };
@@ -174,6 +188,7 @@ k_trace(const __grid_constant__ DScene S, Wave w, PixMap pm, long long pix0, con
         Ray ray = makeRay(d3(r.o[0], r.o[1], r.o[2]), d3(r.d[0], r.d[1], r.d[2]));
         const int got = closestHitT<F>(S, ray, rayTime(S, r.stream, r.ka, r.kb, r.kc, r.stream == STREAM_PIXEL ? DIM_TIME : 0xFFFFu), h, COUNT ? &tc : nullptr);
         if (F != TF_ALL && got < 0) { defer = true; hitReset(h); }
+        h.pad0 = 1;            // the ray's valid flag: k_shade reads it at level 0 instead of generating the primary ray again
       }
       if (!defer) storeHit(hits + i, h);
     }
@@ -205,14 +220,17 @@ __device__ inline D3 skyColor(const DScene& S, D3 o, D3 d) {
 }
 
 // Surface pass. One thread per ray of the level; children go to the next level's queue (its length lives on the device: levelCount[level+1]).
-// rays == null: level 0 -- the primary ray is regenerated from the index and the node record is written whole (no k_raygen pass).
+// PRIMARY (level 0, rays == null): the ray's keys are functions of the index, its valid flag is in the hit record (Hit::pad0), origin and
+// direction are only needed for a skydome lookup (a hit uses h.rawDir); the node record is written whole (no k_raygen pass).  One instance per
+// case, so that the bounce levels carry none of the primary-ray code in their register allocation.
 #ifndef DRT_SHADE_MINBLOCKS
 #define DRT_SHADE_MINBLOCKS 4
 #endif
+template <bool PRIMARY>
 __global__ void __launch_bounds__(128, DRT_SHADE_MINBLOCKS) k_shade(const __grid_constant__ DScene S, Wave w, PixMap pm, long long pix0, const RayRec* __restrict__ rays, const Hit* __restrict__ hits,
                                                SurfRec* __restrict__ surf, NodeRec* __restrict__ nodesBase, RayRec* __restrict__ nextRays, Counters* ctr) {
   const long long n = waveCount(w, ctr);
-  const long long off = (w.level == 0) ? 0 : waveNodeOffset(w, ctr, w.level), offNext = off + n;
+  const long long off = PRIMARY ? 0 : waveNodeOffset(w, ctr, w.level), offNext = off + n;
   NodeRec* __restrict__ nodes = nodesBase + off; NodeRec* __restrict__ nextNodes = nodesBase + offNext;
   const long long nextCap = (w.nodeCap - offNext) < w.rayCap ? (w.nodeCap - offNext) : w.rayCap;
   const unsigned lane = threadIdx.x & 31;
@@ -224,8 +242,11 @@ __global__ void __launch_bounds__(128, DRT_SHADE_MINBLOCKS) k_shade(const __grid
   uint32_t cka = 0, ckb = 0, ckc = 0, cstream = 0; int32_t cgen = 0;
   bool cPrimary = false, cRefl = false, cRefr = false;
   if (i < n) {
-    RayRec r; if (rays) r = rays[i]; else primaryRay(S, pm, pix0, i, r);
     const Hit h = hits[i];
+    RayRec r;
+    if constexpr (!PRIMARY) r = rays[i];
+    else if (S.g.hasSky && h.prim < 0) primaryRay(S, pm, pix0, i, r);
+    else { const PixKey k = pixelOf(S.g, pm, pix0, i); r.ka = (uint32_t)k.pix; r.kb = k.smp; r.kc = 1; r.stream = STREAM_PIXEL; r.gen = 0; r.valid = h.pad0; r.kt0 = 1; r.kt1 = 1; }
     SurfRec s; s.valid = 0; s.shader = -1; s.ka = r.ka; s.kb = r.kb; s.kc = r.kc; s.stream = r.stream; s.gen = r.gen; s.pad = 0;
     D3 local = d3(0, 0, 0);
     if (r.valid) {
@@ -269,7 +290,7 @@ __global__ void __launch_bounds__(128, DRT_SHADE_MINBLOCKS) k_shade(const __grid
       }
     }
     surf[i] = s;
-    if (rays) { nodes[i].local[0] = local.x; nodes[i].local[1] = local.y; nodes[i].local[2] = local.z; }
+    if constexpr (!PRIMARY) { nodes[i].local[0] = local.x; nodes[i].local[1] = local.y; nodes[i].local[2] = local.z; }
     else { NodeRec nd; nd.parent = -1; nd.slot = 0; nd.pad[0] = nd.pad[1] = 0; nd.local[0] = local.x; nd.local[1] = local.y; nd.local[2] = local.z;
       for (int k = 0; k < 3; ++k) { nd.cA[k] = 0; nd.cB[k] = 0; nd.w[k] = 1; } nodes[i] = nd; }
   }
@@ -306,6 +327,10 @@ __global__ void __launch_bounds__(128, DRT_SHADE_MINBLOCKS) k_shade(const __grid
 // Light pass: literal calcShadowColor, one thread per shaded hit, lights in list order, shadow rays traced in-thread.
 // F / work / deferOut as in k_trace: a lean variant that meets a shadow ray it cannot serve leaves the WHOLE record to the generic pass
 // (the record's light sum is formed by one thread in list order either way).
+// Register budget: only what the shadow ray needs (hit point, keys, running sum) is held across the BVH walk; the normal, texture colour,
+// ray direction and shader / light constants of the shading that follows are read from the (L1/L2-resident) records after the walk.  Held
+// across it at the 80-register cap, they were spilled to local memory and written back through L2 on every light.
+__device__ __forceinline__ D3 ldgD3(const double* p) { return d3(__ldg(p), __ldg(p + 1), __ldg(p + 2)); }
 template <bool COUNT, int F>
 __global__ void __launch_bounds__(128, (F == TF_ALL) ? DRT_LIGHT_MINBLOCKS : (F == TF_LITERAL1) ? DRT_L1_MINBLOCKS : DRT_LLIGHT_MINBLOCKS)
 k_light(const __grid_constant__ DScene S, Wave w, const SurfRec* __restrict__ surf, NodeRec* __restrict__ nodesBase, Counters* ctr, const uint32_t* __restrict__ work, uint32_t* __restrict__ deferOut) {
@@ -317,40 +342,47 @@ k_light(const __grid_constant__ DScene S, Wave w, const SurfRec* __restrict__ su
     long long i = base + threadIdx.x; bool defer = false;
     if (i < n) {
       if (work) i = work[i];
-      const SurfRec s = surf[i];
-      if (s.valid) {
-        const FShader sh = S.shaders[s.shader];
-        D3 hitLoc = d3(s.loc[0], s.loc[1], s.loc[2]), N = d3(s.n[0], s.n[1], s.n[2]), rawDir = d3(s.rawDir[0], s.rawDir[1], s.rawDir[2]);
+      const SurfRec* __restrict__ s = surf + i;
+      const int4 sv = __ldg(reinterpret_cast<const int4*>(&s->shader));            // shader, valid, ka, kb
+      if (sv.y) {
+        const int2 sk = __ldg(reinterpret_cast<const int2*>(&s->kc));               // kc, stream
+        const uint32_t ka = (uint32_t)sv.z, kb = (uint32_t)sv.w, kc = (uint32_t)sk.x, stream = (uint32_t)sk.y;
+        const FShader& sh = S.shaders[sv.x];
+        const D3 hitLoc = ldgD3(s->loc);
         double r = 0, g = 0, b = 0; unsigned nShadow = 0;
         for (int li = 0; li < S.g.numLights; ++li) {
-          const FLight L = S.lights[li]; const FXform& LX = S.xforms[L.xform];
+          const FLight& L = S.lights[li];
           const uint32_t dim = DIM_LIGHT_BASE + DIM_LIGHT_STRIDE * li;
+          const int type = L.type;
           D3 lo = d3(L.origin[0], L.origin[1], L.origin[2]), orient = d3(L.orient[0], L.orient[1], L.orient[2]);
           auto diskPos = [&](uint32_t d0) {           // myDiskLight.getRandomDiskPos (:251-258)
-            double ua = philoxU01(S.g.seed, s.stream, s.ka, s.kb, s.kc, d0), ur = philoxU01(S.g.seed, s.stream, s.ka, s.kb, s.kc, d0 + 1);
+            double ua = philoxU01(S.g.seed, stream, ka, kb, kc, d0), ur = philoxU01(S.g.seed, stream, ka, kb, kc, d0 + 1);
             D3 tmp = norm3(rotAboutAxis(d3(L.tangent[0], L.tangent[1], L.tangent[2]), orient, urange(ua, 0, DRT_TWO_PI_F)));
             return add3(scale3(tmp, urange(ur, 0, L.radius)), lo);
           };
-          D3 target = (L.type == LT_DISK) ? diskPos(dim) : lo;
-          D3 lightNorm = norm3(sub3(xfPoint(LX.m, target), hitLoc));
+          // world position of the sample on the light: per ray for a disk, else the light's transformed origin (S.lightPos, formed once per upload)
+          const D3 target = (type == LT_DISK) ? xfPoint(S.xforms[L.xform].m, diskPos(dim)) : ldgD3(S.lightPos + 3 * li);
+          D3 lightNorm = norm3(sub3(target, hitLoc));
           Ray shadowRay = makeRay(hitLoc, lightNorm);
           // light.intersectCheck: distance to the light's (re-sampled, untransformed) origin, penumbra factor (SURVEY Q12)
-          D3 dOrg = (L.type == LT_DISK) ? diskPos(dim + 2) : lo;
+          D3 dOrg = (type == LT_DISK) ? diskPos(dim + 2) : lo;
           double t = sqrt(((hitLoc.x - dOrg.x) * (hitLoc.x - dOrg.x)) + ((hitLoc.y - dOrg.y) * (hitLoc.y - dOrg.y)) + ((hitLoc.z - dOrg.z) * (hitLoc.z - dOrg.z)));
           double ltMult = 1;
-          if (L.type == LT_SPOT) { double angle = acos(-1 * dot3(lightNorm, orient)); ltMult = (angle < L.innerRad) ? 1 : (angle > L.outerRad) ? 0 : (L.outerRad - angle) / L.radDiff; }
+          if (type == LT_SPOT) { double angle = acos(-1 * dot3(lightNorm, orient)); ltMult = (angle < L.innerRad) ? 1 : (angle > L.outerRad) ? 0 : (L.outerRad - angle) / L.radDiff; }
           if (ltMult == 0) continue;
           ++nShadow;
-          double time = rayTime(S, s.stream, s.ka, s.kb, s.kc, dim + 4);
+          double time = rayTime(S, stream, ka, kb, kc, dim + 4);
           const int occluded = anyHitT<F>(S, shadowRay, time, t, COUNT ? &tc : nullptr);
           if (F != TF_ALL && occluded < 0) { defer = true; break; }
           if (!occluded) {
+            const D3 N = ldgD3(s->n), tex = ldgD3(s->tex), color = d3(L.color[0], L.color[1], L.color[2]);
             double ld = dot3(lightNorm, N) * ltMult;
-            if (ld > DRT_EPS) { r += s.tex[0] * L.color[0] * ld; g += s.tex[1] * L.color[1] * ld; b += s.tex[2] * L.color[2] * ld; }
-            if (sh.phong == 0) continue;
-            D3 hN = norm3(sub3(lightNorm, rawDir));
+            if (ld > DRT_EPS) { r += tex.x * color.x * ld; g += tex.y * color.y * ld; b += tex.z * color.z * ld; }
+            const double phong = sh.phong;
+            if (phong == 0) continue;
+            D3 hN = norm3(sub3(lightNorm, ldgD3(s->rawDir)));
             double hd = dot3(hN, N) * ltMult;
-            if (hd > DRT_EPS) { double ph = pow(hd * hd, sh.phong); r += sh.spec[0] * L.color[0] * ph; g += sh.spec[1] * L.color[1] * ph; b += sh.spec[2] * L.color[2] * ph; }
+            if (hd > DRT_EPS) { double ph = pow(hd * hd, phong); r += sh.spec[0] * color.x * ph; g += sh.spec[1] * color.y * ph; b += sh.spec[2] * color.z * ph; }
           }
         }
         if (!defer) { cShadow += nShadow; nodes[i].local[0] += r; nodes[i].local[1] += g; nodes[i].local[2] += b; }
@@ -360,6 +392,12 @@ k_light(const __grid_constant__ DScene S, Wave w, const SurfRec* __restrict__ su
   }
   warpAdd(&ctr->shadowS[blockIdx.x & 63], cShadow);
   if (COUNT) { warpAdd(&ctr->box, tc.box); warpAdd(&ctr->prim, tc.prim); }
+}
+// world position of every light's origin, xfPoint(CTM, origin): the target of every shadow ray toward a point or spot light
+__global__ void k_light_pos(const FXform* __restrict__ xforms, const FLight* __restrict__ lights, int n, double* __restrict__ out) {
+  const int li = blockIdx.x * blockDim.x + threadIdx.x; if (li >= n) return;
+  const FLight L = lights[li]; const D3 p = xfPoint(xforms[L.xform].m, d3(L.origin[0], L.origin[1], L.origin[2]));
+  out[3 * li] = p.x; out[3 * li + 1] = p.y; out[3 * li + 2] = p.z;
 }
 
 __device__ __forceinline__ D3 nodeTotal(const NodeRec& nd) {
@@ -464,7 +502,7 @@ struct SceneArena {
 
 struct Renderer::Impl {
   DScene ds; SceneArena arena; DBuf<FNode> lbvhNodeBuf; DBuf<FNode32> lbvhNode32Buf; DBuf<FTri> lbvhTriBuf; LbvhScratch lbvhScratch; RefBvhScratch refScratch;
-  DBuf<RayRec> rays[2]; DBuf<Hit> hits; DBuf<Hit> hits0; DBuf<SurfRec> surf; DBuf<NodeRec> nodes; Counters* ctr = nullptr; Counters* ctrHost = nullptr;
+  DBuf<RayRec> rays[2]; DBuf<Hit> hits; DBuf<Hit> hits0; DBuf<SurfRec> surf; DBuf<NodeRec> nodes; DBuf<double> lightPos; Counters* ctr = nullptr; Counters* ctrHost = nullptr;
   DBuf<uint32_t> deferT, deferL;                 // deferral lists of the lean trace / light kernels (ray indices of one level)
   std::vector<cudaEvent_t> evPool;               // stage timing of a whole frame without a host sync per level
   int shape = TF_ALL;                            // kernel variant the uploaded scene runs with (see chooseShape)
@@ -498,7 +536,7 @@ Renderer::Renderer(int device) : impl_(new Impl), device_(device) {
 Renderer::~Renderer() {
   cudaSetDevice(device_);
   impl_->arena.release(); impl_->lbvhNodeBuf.release(); impl_->lbvhNode32Buf.release(); impl_->lbvhTriBuf.release(); impl_->lbvhScratch.release(); impl_->refScratch.release();
-  impl_->rays[0].release(); impl_->rays[1].release(); impl_->hits.release(); impl_->hits0.release(); impl_->surf.release(); impl_->nodes.release();
+  impl_->rays[0].release(); impl_->rays[1].release(); impl_->hits.release(); impl_->hits0.release(); impl_->surf.release(); impl_->nodes.release(); impl_->lightPos.release();
   impl_->oArgb.release(); impl_->oPrim.release(); impl_->oInst.release(); impl_->oRgb.release(); impl_->oT.release();
   impl_->deferT.release(); impl_->deferL.release(); for (auto& e : impl_->evPool) cudaEventDestroy(e);
   impl_->photons.release(); impl_->xCnt.release(); impl_->xMine.release(); impl_->xAll.release();
@@ -548,6 +586,8 @@ void Renderer::upload(const HostScene& hs, bool sameScene) {
   d.lists = A.put(hs.lists); d.nodes = A.put(hs.nodes); d.fnodes32 = A.put(hs.nodes32); d.tris = A.put(hs.tris); d.bvhs = A.put(bv); d.lights = A.put(hs.lights); d.shaders = A.put(hs.shaders);
   d.textures = A.put(hs.textures); d.texColors = A.put(hs.texColors); d.images = A.put(hs.images); d.texels = A.put(hs.texels);
   A.flush(st); A.stagedScene = (const void*)&hs; A.stagedUsed = needBytes; A.fill = true;
+  { const int nl = (int)hs.lights.size(); impl_->lightPos.ensure(3 * (size_t)std::max(nl, 1), st); d.lightPos = impl_->lightPos.p;
+    if (nl) { k_light_pos<<<(unsigned)((nl + 127) / 128), 128, 0, st>>>(d.xforms, d.lights, nl, impl_->lightPos.p); ++g_kernelLaunches; CK(cudaGetLastError()); } }
   d.fnodes = d.nodes; impl_->lbvhMs = 0; impl_->lbvhTris = 0; impl_->lbvhNodes = 0; impl_->bvhsUploaded = bv;
   if (extra) {
     const size_t n0 = hs.nodes.size();
@@ -602,7 +642,7 @@ void Renderer::renderRange(long long pix0, long long pix1, const RenderOutputs& 
 // device error word says whether the speculation held (queue capacity, launched depth); if not, the frame is rendered again with safer settings.
 void Renderer::renderChunks(long long pix0, long long pix1, int world, int rank, int chunkRows, const RenderOutputs& out, RenderStats* stats) {
   CK(cudaSetDevice(device_)); cudaStream_t st = (cudaStream_t)stream_; Impl& I = *impl_;
-  PixMap pm; pm.totalPix = (long long)g_.cols * g_.rows; pm.world = world < 1 ? 1 : world; pm.rank = rank;
+  PixMap pm; pm.totalPix = (long long)g_.cols * g_.rows; pm.world = world < 1 ? 1 : world; pm.rank = rank; pm.narrow = 0;
   pm.chunkPix = (pm.world == 1) ? (pm.totalPix > 0 ? pm.totalPix : 1) : (long long)chunkRows * g_.cols;
   if (pm.world > 1) { long long nChunks = (g_.rows + chunkRows - 1) / chunkRows, mine = (nChunks - rank + world - 1) / world; pix0 = 0; pix1 = mine * pm.chunkPix; }
   if (!I.ds.prims) throw std::runtime_error("render called before a scene was uploaded");
@@ -622,6 +662,8 @@ void Renderer::renderChunks(long long pix0, long long pix1, int world, int rank,
     std::memset(&rs, 0, sizeof(rs)); rs.photonsStored = I.photons.count; rs.photonSeg = I.photons.segments;
     long long pixPerBatch = batchRays / spp; if (pixPerBatch < 1) pixPerBatch = 1;
     const long long maxN0 = std::min(pixPerBatch, std::max<long long>(pix1 - pix0, 1)) * spp;
+    // compact pixels are < pix1, so absolute pixels are < (pix1 / chunkPix + 1) * world * chunkPix
+    pm.narrow = (maxN0 <= INT32_MAX && (pix1 / pm.chunkPix + 1) * pm.world * pm.chunkPix <= INT32_MAX) ? 1 : 0;
     const long long rayCap = (levels > 1) ? std::max<long long>(64, (long long)(capFactor * (double)maxN0)) : 1;
     const long long nodeCap = (levels > 1) ? maxN0 + ((capFactor >= 64.0) ? 126 * maxN0 : std::max<long long>(64, (long long)(3.0 * capFactor * (double)maxN0))) : maxN0;
     I.hits0.ensure(maxN0, st); I.surf.ensure(std::max(maxN0, rayCap), st); I.nodes.ensure(nodeCap, st);
@@ -656,7 +698,9 @@ void Renderer::renderChunks(long long pix0, long long pix1, int world, int rank,
           rs.kernelLaunches += 2; dbg("k_trace fix-up", level);
         }
         CK(cudaEventRecord(I.pev(evN++), st));
-        k_shade<<<grid, 128, 0, st>>>(I.ds, w, pm, b0, rays, hitBuf, I.surf.p, I.nodes.p, nextRays, I.ctr); ++rs.kernelLaunches; dbg("k_shade", level);
+        if (level == 0) k_shade<true><<<grid, 128, 0, st>>>(I.ds, w, pm, b0, rays, hitBuf, I.surf.p, I.nodes.p, nextRays, I.ctr);
+        else k_shade<false><<<grid, 128, 0, st>>>(I.ds, w, pm, b0, rays, hitBuf, I.surf.p, I.nodes.p, nextRays, I.ctr);
+        ++rs.kernelLaunches; dbg("k_shade", level);
         if (I.ds.numPhotons > 0) { k_photon_gather_lane<<<grid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr); k_photon_gather_warp<<<grid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr); rs.kernelLaunches += 2; dbg("k_photon_gather", level); }
         CK(cudaEventRecord(I.pev(evN++), st));
         if (generic) {
@@ -852,7 +896,7 @@ long long Renderer::distRankPixels(int cols, int rows, int world, int rank, int 
   const long long nChunks = (rows + chunkRows - 1) / chunkRows; return ((nChunks - rank + world - 1) / world) * (long long)chunkRows * cols;
 }
 long long Renderer::distAbsPixel(int cols, int rows, int world, int rank, int chunkRows, long long compact) {
-  PixMap pm; pm.totalPix = (long long)cols * rows; pm.world = world; pm.rank = rank; pm.chunkPix = (world == 1) ? std::max<long long>(pm.totalPix, 1) : (long long)chunkRows * cols;
+  PixMap pm; pm.totalPix = (long long)cols * rows; pm.world = world; pm.rank = rank; pm.narrow = 0; pm.chunkPix = (world == 1) ? std::max<long long>(pm.totalPix, 1) : (long long)chunkRows * cols;
   const long long q = absPixel(pm, compact); return q < pm.totalPix ? q : -1;
 }
 void Renderer::distPhotonRange(long long nCast, int world, int rank, long long out2[2]) { out2[0] = nCast * rank / world; out2[1] = nCast * (rank + 1) / world; }

@@ -22,9 +22,9 @@ import argparse, csv, hashlib, io, json, os, re, subprocess, sys, tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-KERNELS = {"k_trace": r"_ZN3drt7k_traceILb0ELi0EEE", "k_light": r"_ZN3drt7k_lightILb0ELi0EEE", "k_shade": r"_ZN3drt7k_shadeE"}
-VARIANT = {"k_trace": "<(bool)0, (int)0>", "k_light": "<(bool)0, (int)0>", "k_shade": "k_shade"}      # launch name filter in the ncu report
-RAWNAME = {"k_trace": "<0, 0>", "k_light": "<0, 0>", "k_shade": "k_shade"}
+KERNELS = {"k_trace": r"_ZN3drt7k_traceILb0ELi0EEE", "k_light": r"_ZN3drt7k_lightILb0ELi0EEE", "k_shade": r"_ZN3drt7k_shadeILb1EEE"}   # k_shade<true>: level 0
+VARIANT = {"k_trace": "<(bool)0, (int)0>", "k_light": "<(bool)0, (int)0>", "k_shade": "k_shade<(bool)1>"}      # launch name filter in the ncu report
+RAWNAME = {"k_trace": "<0, 0>", "k_light": "<0, 0>", "k_shade": "k_shade<1>"}
 
 
 def marker_ranges():
