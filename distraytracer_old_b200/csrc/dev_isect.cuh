@@ -112,12 +112,6 @@ __device__ __forceinline__ int boxQuick(const double* __restrict__ mn, const dou
   if (gap > tol) return near_ > 0 ? 1 : 0;
   return (-gap > tol) ? 0 : -1;
 }
-// box accepted?  te = conservative LOWER bound of the entry t (exact when the quick path could not decide)
-__device__ __forceinline__ bool boxAcceptLB(const double* __restrict__ mn, const double* __restrict__ mx, const Ray& r, const D3& inv, double& te) {
-  const int q = boxQuick(mn, mx, r, inv, te);
-  if (q >= 0) { te *= 0.999999999999999; return q != 0; }
-  return boxTestFx(mn, mx, r, inv, te);
-}
 // box accepted AND (dist - entry) > eps, the shadow-ray form (myGeomBase.java:166-170,268-269,397-404)
 __device__ __forceinline__ bool boxAcceptShadow(const double* __restrict__ mn, const double* __restrict__ mx, const Ray& r, const D3& inv, double dist) {
   double te; const int q = boxQuick(mn, mx, r, inv, te);
@@ -292,37 +286,8 @@ __device__ __noinline__ bool primTest(const DScene& S, int primIdx, const Ray& r
 // ---------------------------------------------------------------------------------------------------------------
 // fast BVHs: packed triangles, both child boxes per node, near-first ordered descent with global pruning
 // ---------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void ldTri(const FTri* __restrict__ p, double (&w)[14], int32_t& prim) {
-  const double2* __restrict__ q = reinterpret_cast<const double2*>(p);
-#pragma unroll
-  for (int i = 0; i < 7; ++i) { const double2 a = __ldg(q + i); w[2 * i] = a.x; w[2 * i + 1] = a.y; }
-  prim = __ldg(reinterpret_cast<const int32_t*>(p) + 29);      // rank in the reference's visiting order (FTri::pad[0])
-}
-// myTriangle.intersectCheck on a packed record: the same operations, in the same order, as primTest's PT_TRI case
-__device__ __forceinline__ bool triTestPacked(const double (&w)[14], const Ray& r, double& tOut, int& stOut) {
-  D3 N = d3(w[9], w[10], w[11]); double D = w[12];
-  double planeRes = dot3(N, r.d);
-  if (!(fabs(planeRes) > 0)) return false;
-  int st = 0;
-  if (planeRes > 0) { st = 1; N = d3(-N.x, -N.y, -N.z); D = w[13]; planeRes = dot3(N, r.d); if (!(fabs(planeRes) > 0) || planeRes > 0) return false; }
-  const double t = -(dot3(N, r.o) + D) / planeRes;
-  if (!(t > DRT_EPS)) return false;
-  const D3 p = pointOnRay(r, t);
-  const D3 a = d3(w[0], w[1], w[2]), b = d3(w[3], w[4], w[5]), c = d3(w[6], w[7], w[8]);
-  const D3 V0 = st ? c : a, V2 = st ? a : c;                       // reversed winding: vertices (c, b, a)
-  { D3 ir = d3(p.x - V0.x, p.y - V0.y, p.z - V0.z), e = d3(V0.x - V2.x, V0.y - V2.y, V0.z - V2.z); if (dot3(cross3(ir, e), N) < -DRT_EPS) return false; }
-  { D3 ir = d3(p.x - b.x, p.y - b.y, p.z - b.z), e = d3(b.x - V0.x, b.y - V0.y, b.z - V0.z); if (dot3(cross3(ir, e), N) < -DRT_EPS) return false; }
-  { D3 ir = d3(p.x - V2.x, p.y - V2.y, p.z - V2.z), e = d3(V2.x - b.x, V2.y - b.y, V2.z - b.z); if (dot3(cross3(ir, e), N) < -DRT_EPS) return false; }
-  tOut = t; stOut = st; return true;
-}
-// both child boxes of a node with 128-bit loads
-__device__ __forceinline__ void ldNode(const FNode* __restrict__ p, double (&bx)[12], int32_t& left, int32_t& right, int32_t& triL, int32_t& triR) {
-  const double2* __restrict__ q = reinterpret_cast<const double2*>(p);
-#pragma unroll
-  for (int i = 0; i < 6; ++i) { const double2 a = __ldg(q + i); bx[2 * i] = a.x; bx[2 * i + 1] = a.y; }
-  const int4 l = __ldg(reinterpret_cast<const int4*>(p) + 6); left = l.x; right = l.y; triL = l.z; triR = l.w;
-}
-// conventional conservative slab test (LBVH mode only): a ray that starts inside the box enters it at t = 0
+// conventional conservative slab test (LBVH mode only): a ray that starts inside the box enters it at t = 0.  fmin / fmax pick the near and
+// far plane of each axis whatever the sign of the direction, and drop the NaN slab value of an axis-parallel ray whose origin lies on a plane
 __device__ __forceinline__ bool boxTestStd(const double* mn, const double* mx, const Ray& r, const D3& inv, double& tEntry) {
   double t0 = (mn[0] - r.o.x) * inv.x, t1 = (mx[0] - r.o.x) * inv.x; double tn = fmin(t0, t1), tf = fmax(t0, t1);
   t0 = (mn[1] - r.o.y) * inv.y; t1 = (mx[1] - r.o.y) * inv.y; tn = fmax(tn, fmin(t0, t1)); tf = fmin(tf, fmax(t0, t1));
@@ -330,153 +295,24 @@ __device__ __forceinline__ bool boxTestStd(const double* mn, const double* mx, c
   tEntry = fmax(tn, 0.0); return tf >= tEntry;
 }
 
-// Traversal stack of the fast paths: the first DRT_SSTACK levels live in shared memory ([level][thread], 8-byte entries, conflict-free),
-// deeper levels (only unbalanced LBVHs get there) in a small local array.  Keeping the stack out of local memory matters: with ~110 k
-// resident threads a per-thread local frame of a few KB is larger than L2 and turns every push/pop into DRAM traffic (profiles/r1b).
-// entry.x = child reference (>= 0 inner node, < 0: ~tri-leaf code), entry.y = bits of the box-entry t rounded DOWN to float.
-#ifndef DRT_LEAN
-#define DRT_LEAN 1
-#endif
 // The traversal bodies are force-inlined in the lean kernels so that ray and hit records stay in registers; -DDRT_LEAN_INLINE=__noinline__ builds the
 // outlined form, which passes the same equivalence tests (DESIGN.md section 3, `__noinline__` note).
 #ifndef DRT_LEAN_INLINE
 #define DRT_LEAN_INLINE __forceinline__
 #endif
-#define DRT_TB 128              // threads per block of every kernel that traces
-#ifndef DRT_SSTACK
-#define DRT_SSTACK 0            // levels kept in shared memory; measured on B200 (profiles/r1_tuning.md): shared levels cost more L1 capacity than they save
-#endif
-#define DRT_FSTACK 64
-#if DRT_SSTACK > 0
-__shared__ uint2 g_fstk[DRT_SSTACK * DRT_TB];
-#endif
-template <int CAP>
-struct FStackT {
-  uint2 ovf[CAP - DRT_SSTACK]; int sp = 0; bool overflow = false;
-  __device__ __forceinline__ void push(int32_t ref, float te) {
-    const uint2 e = make_uint2((uint32_t)ref, __float_as_uint(te));
-#if DRT_SSTACK > 0
-    if (sp < DRT_SSTACK) g_fstk[sp * DRT_TB + threadIdx.x] = e; else
-#endif
-    if (sp < CAP) ovf[sp - DRT_SSTACK] = e;
-    if (sp < CAP) ++sp; else overflow = true;
-  }
-  __device__ __forceinline__ uint2 pop() {
-    --sp;
-#if DRT_SSTACK > 0
-    if (sp < DRT_SSTACK) return g_fstk[sp * DRT_TB + threadIdx.x];
-#endif
-    return ovf[sp - DRT_SSTACK];
-  }
-};
-typedef FStackT<DRT_FSTACK> FStack;
+#define DRT_FSTACK 64            // traversal stack of the generic kernels
 // Compile-time feature set of a tracing kernel (see render.cu): the lean kernels carry only the code their scene shape needs -- a small
 // local frame and register budget -- and hand the rare ray they cannot serve (axis-parallel direction, mixed units through an instance,
 // traversal deeper than the short stack) to the generic kernel through a deferral list.  Every ray is traced start to finish by ONE variant,
 // and all variants implement the same rules, so results do not depend on which one served a ray.
 enum : int { TF_LITERAL1 = 1,     // literal (reference-order) BVH recursion at the top level, lists holding instanced accels
-             TF_LEVEL2 = 2,       // literal recursion / non-lean descent inside instanced accels
-             TF_NONLEAN = 4,      // near-first descent with the generic slab test (irregular directions) at the top level
-             TF_ALL = 7 };
-#ifndef DRT_LEAN32
-#define DRT_LEAN32 1             // lean kernels take box decisions in FP32 under an error bound (leanClosest32); 0 = FP64 lean descent everywhere
-#endif
-#ifndef DRT_TWOLEVEL
-#define DRT_TWOLEVEL 1           // lean light kernel walks instance trees with instTreeShadow (mesh searches side by side); 0 = the nested literal loop
-#endif
+             TF_LEVEL2 = 2,       // literal recursion inside instanced accels
+             TF_ALL = 7 };        // the generic variant: serves every ray, whatever its direction
 #ifndef DRT_LSTACK
 #define DRT_LSTACK 32            // short traversal stack of the lean kernels (a <=5-per-leaf median tree over 2^24 triangles is 23 deep)
 #endif
 __device__ __forceinline__ int32_t childRef(int32_t link, int32_t triCode) { return link >= 0 ? link : ~triCode; }
 
-// Closest hit inside one fast BVH (root box already accepted by the caller). `trans` is the ray the boxes are tested with,
-// `r` the ray the triangles are tested with (see SURVEY Q7 for why they can differ; ONE_RAY: they are bitwise the same ray, which is
-// the case for every mesh that is not reached through an instance -- half the live registers).  Result: the minimum-t hit over every
-// leaf whose chain of boxes is accepted -- the set the reference's left-first recursion searches; equal-t candidates resolve to the
-// lower reference rank, i.e. the reference's visiting order.  stdBox: LBVH mode's conventional slab test.
-template <bool ONE_RAY>
-__device__ DRT_LEAN_INLINE bool fastClosest(const DScene& S, const FBvh& B, const Ray& transIn, const Ray& rIn, D3 rawDir, Hit& out, TraceCounters* tc) {
-  Ray trans; trans.o = transIn.o; trans.a = transIn.a; trans.d = transIn.a; trans.norm = false;
-  Ray r; if (ONE_RAY) r = trans; else { r.o = rIn.o; r.d = rIn.d; r.a = rIn.d; r.norm = false; }
-  const bool stdBox = S.accelMode == 2;
-  const D3 inv = rayInv(trans);
-  FStack stk;
-  double bestT = DRT_DMAX; int bestTri = -1, bestRank = 0x7fffffff, bestSt = 0;
-  int32_t ref = B.fastRoot;
-  while (true) {
-    if (ref >= 0) {
-      double bx[12]; int32_t left, right, triL, triR; ldNode(S.fnodes + ref, bx, left, right, triL, triR);
-      double teL, teR; if (tc) tc->box += 2;
-      bool hl, hr;
-      if (stdBox) { hl = boxTestStd(bx, bx + 3, trans, inv, teL); hr = boxTestStd(bx + 6, bx + 9, trans, inv, teR); }
-      else { hl = boxAcceptLB(bx, bx + 3, trans, inv, teL); hr = boxAcceptLB(bx + 6, bx + 9, trans, inv, teR); }
-      hl = hl && teL < bestT; hr = hr && teR < bestT;
-      const int32_t cl = childRef(left, triL), cr = childRef(right, triR);
-      if (hl && hr) {
-        const bool rightFirst = teR < teL;
-        stk.push(rightFirst ? cl : cr, __double2float_rd(rightFirst ? teL : teR));
-        ref = rightFirst ? cr : cl; continue;
-      }
-      if (hl) { ref = cl; continue; }
-      if (hr) { ref = cr; continue; }
-    } else {
-      const int code = ~ref, cnt = code & 7, first = code >> 3;
-      for (int i = 0; i < cnt; ++i) {
-        double w[14]; int32_t rank; ldTri(S.tris + first + i, w, rank);
-        double t; int st; if (tc) ++tc->prim;
-        if (triTestPacked(w, r, t, st) && (t < bestT || (t == bestT && rank < bestRank))) { bestT = t; bestTri = first + i; bestRank = rank; bestSt = st; }
-      }
-    }
-    // pop
-    while (true) {
-      if (stk.sp == 0) {
-        if (stk.overflow) flagError(1u);
-        if (bestTri < 0) return false;
-        out.t = bestT; out.prim = S.tris[bestTri].prim; out.arg0 = 0; out.arg1 = 0; out.state = bestSt; out.hitXform = B.triHitXform; out.shaderOverride = -1; out.inst = -1;
-        out.loc = pointOnRay(r, bestT); out.rawDir = rawDir; return true;
-      }
-      const uint2 e = stk.pop();
-      if ((double)__uint_as_float(e.y) < bestT) { ref = (int32_t)e.x; break; }
-    }
-  }
-}
-// Any hit inside one fast BVH: (dist - t) > eps for a triangle, every box on the way accepted with (dist - entry) > eps
-template <bool ONE_RAY>
-__device__ DRT_LEAN_INLINE bool fastShadow(const DScene& S, const FBvh& B, const Ray& transIn, const Ray& rIn, double dist, TraceCounters* tc) {
-  Ray trans; trans.o = transIn.o; trans.a = transIn.a; trans.d = transIn.a; trans.norm = false;
-  Ray r; if (ONE_RAY) r = trans; else { r.o = rIn.o; r.d = rIn.d; r.a = rIn.d; r.norm = false; }
-  const bool stdBox = S.accelMode == 2;
-  const D3 inv = rayInv(trans);
-  FStack stk;
-  int32_t ref = B.fastRoot;
-  while (true) {
-    if (ref >= 0) {
-      double bx[12]; int32_t left, right, triL, triR; ldNode(S.fnodes + ref, bx, left, right, triL, triR);
-      double teL, teR; if (tc) tc->box += 2;
-      bool hl, hr;
-      if (stdBox) { hl = boxTestStd(bx, bx + 3, trans, inv, teL) && (dist - teL) > DRT_EPS; hr = boxTestStd(bx + 6, bx + 9, trans, inv, teR) && (dist - teR) > DRT_EPS; }
-      else { hl = boxAcceptShadow(bx, bx + 3, trans, inv, dist); hr = boxAcceptShadow(bx + 6, bx + 9, trans, inv, dist); }
-      const int32_t cl = childRef(left, triL), cr = childRef(right, triR);
-      if (hl && hr) { stk.push(cr, 0.f); ref = cl; continue; }
-      if (hl) { ref = cl; continue; }
-      if (hr) { ref = cr; continue; }
-    } else {
-      const int code = ~ref, cnt = code & 7, first = code >> 3;
-      for (int i = 0; i < cnt; ++i) {
-        double w[14]; int32_t rank; ldTri(S.tris + first + i, w, rank);
-        double t; int st; if (tc) ++tc->prim;
-        if (triTestPacked(w, r, t, st) && (dist - t) > DRT_EPS) return true;
-      }
-    }
-    if (stk.sp == 0) { if (stk.overflow) flagError(1u); return false; }
-    ref = (int32_t)stk.pop().x;
-  }
-}
-// ---- lean descent for "regular" rays (every direction component finite, non-zero and of sane magnitude: all but axis-parallel rays)
-// The per-axis ordering the reference derives from `v1 < v2` is the sign of the direction component (node boxes of fast BVHs have
-// min <= max, checked by the host), so the near/far slab planes are picked per RAY, and each box costs 6 subtractions, 6 products, two
-// 3-way max/min and the margin check of boxQuick().  Anything inside the margin goes to the exact test, out of line.
-struct LeanRay { double ox, oy, oz, ix, iy, iz; bool px, py, pz; };
 // exact (true-division) box test, out of line; returns the entry t (> 0 by the acceptance rule) or -1 when the box is rejected.  The value
 // travels in the return register: a `double&` result would force the callers' entry-t variables into local memory on EVERY node visit.
 __device__ __noinline__ double boxExactEntry(const double* __restrict__ box6, double ox, double oy, double oz, double ax, double ay, double az) {
@@ -484,34 +320,35 @@ __device__ __noinline__ double boxExactEntry(const double* __restrict__ box6, do
   double b[6]; for (int i = 0; i < 6; ++i) b[i] = __ldg(box6 + i);
   return boxTest(b, b + 3, r, te, face) ? te : -1.0;
 }
-// 1 accepted / 0 rejected / -1 undecided; nearOut = entry t to ~3e-16 relative
-__device__ __forceinline__ int leanBox(double mnx, double mny, double mnz, double mxx, double mxy, double mxz, const LeanRay& R, double& nearOut) {
-  const double nx = ((R.px ? mnx : mxx) - R.ox) * R.ix, fx = ((R.px ? mxx : mnx) - R.ox) * R.ix;
-  const double ny = ((R.py ? mny : mxy) - R.oy) * R.iy, fy = ((R.py ? mxy : mny) - R.oy) * R.iy;
-  const double nz = ((R.pz ? mnz : mxz) - R.oz) * R.iz, fz = ((R.pz ? mxz : mnz) - R.oz) * R.iz;
-  double near_ = nx > ny ? nx : ny; near_ = nz > near_ ? nz : near_;
-  double far_ = fx < fy ? fx : fy; far_ = fz < far_ ? fz : far_;
-  nearOut = near_;
-  if (!(fabs(near_) > 1e-290)) return -1;
-  const double tol = 1e-14 * (fabs(far_) + fabs(near_)), gap = far_ - near_;
-  if (gap > tol) return near_ > 0 ? 1 : 0;
-  return (-gap > tol) ? 0 : -1;
+// conventional slab test (LBVH mode) out of line: entry t (>= 0) or -1.  ANY_DIR (generic kernels): boxTestStd's fmin / fmax, right for every
+// direction.  Otherwise (lean kernels, regular directions only) the near and far plane of each axis are picked by the sign of the direction: the
+// same slab values and decisions.  The lean form is kept because the fmin / fmax body changes the lean kernels' register allocation, which
+// measured 1.9 % slower per frame on plnts3ColsBunnies 4K (B200).
+template <bool ANY_DIR>
+__device__ __noinline__ double boxStdEntry(const double* __restrict__ box6, double ox, double oy, double oz, double ax, double ay, double az) {
+  if constexpr (ANY_DIR) {
+    Ray r; r.o = d3(ox, oy, oz); r.a = d3(ax, ay, az); r.d = r.a; r.norm = false; double te;
+    double b[6]; for (int i = 0; i < 6; ++i) b[i] = __ldg(box6 + i);
+    return boxTestStd(b, b + 3, r, rayInv(r), te) ? te : -1.0;
+  } else {
+    const double ix = 1.0 / ax, iy = 1.0 / ay, iz = 1.0 / az; const bool px = ax > 0, py = ay > 0, pz = az > 0;
+    const double mnx = __ldg(box6), mny = __ldg(box6 + 1), mnz = __ldg(box6 + 2), mxx = __ldg(box6 + 3), mxy = __ldg(box6 + 4), mxz = __ldg(box6 + 5);
+    const double nx = ((px ? mnx : mxx) - ox) * ix, fx = ((px ? mxx : mnx) - ox) * ix;
+    const double ny = ((py ? mny : mxy) - oy) * iy, fy = ((py ? mxy : mny) - oy) * iy;
+    const double nz = ((pz ? mnz : mxz) - oz) * iz, fz = ((pz ? mxz : mnz) - oz) * iz;
+    double near_ = nx > ny ? nx : ny; near_ = nz > near_ ? nz : near_; near_ = near_ > 0.0 ? near_ : 0.0;
+    double far_ = fx < fy ? fx : fy; far_ = fz < far_ ? fz : far_;
+    return far_ >= near_ ? near_ : -1.0;
+  }
 }
-// conventional slab test on the same per-ray ordered planes (LBVH mode: boxes are padded outward, a ray that starts inside enters at t = 0)
-__device__ __forceinline__ int leanBoxStd(double mnx, double mny, double mnz, double mxx, double mxy, double mxz, const LeanRay& R, double& nearOut) {
-  const double nx = ((R.px ? mnx : mxx) - R.ox) * R.ix, fx = ((R.px ? mxx : mnx) - R.ox) * R.ix;
-  const double ny = ((R.py ? mny : mxy) - R.oy) * R.iy, fy = ((R.py ? mxy : mny) - R.oy) * R.iy;
-  const double nz = ((R.pz ? mnz : mxz) - R.oz) * R.iz, fz = ((R.pz ? mxz : mnz) - R.oz) * R.iz;
-  double near_ = nx > ny ? nx : ny; near_ = nz > near_ ? nz : near_; near_ = near_ > 0.0 ? near_ : 0.0;
-  double far_ = fx < fy ? fx : fy; far_ = fz < far_ ? fz : far_;
-  nearOut = near_; return far_ >= near_ ? 1 : 0;
-}
+// directions the lean kernels serve: every component finite, non-zero and of sane magnitude (all but axis-parallel rays)
 __device__ __forceinline__ bool regularDir(D3 a) {
   const double x = fabs(a.x), y = fabs(a.y), z = fabs(a.z);
   return x > 1e-100 && x < 1e100 && y > 1e-100 && y < 1e100 && z > 1e-100 && z < 1e100;
 }
-// triangle test of triTestPacked with one shortcut that cannot change the outcome: a plane hit farther than the best hit so far is
-// dropped before the inside test (the reference would compute it and then discard it in `t < closest`)
+// myTriangle.intersectCheck on a packed record: the same operations, in the same order, as primTest's PT_TRI case, with one shortcut that
+// cannot change the outcome: a plane hit farther than the best hit so far is dropped before the inside test (the reference would compute it
+// and then discard it in `t < closest`)
 __device__ __forceinline__ bool leanTri(const FTri* __restrict__ T, double ox, double oy, double oz, double dx, double dy, double dz, double bestT, double& tOut, int& stOut, int32_t& rank) {
   const double2* __restrict__ q = reinterpret_cast<const double2*>(T);
   const double2 q4 = __ldg(q + 4), q5 = __ldg(q + 5), q6 = __ldg(q + 6);                    // (v8, N.x) (N.y, N.z) (D, Drev)
@@ -538,119 +375,19 @@ __device__ __forceinline__ bool leanTri(const FTri* __restrict__ T, double ox, d
   rank = __ldg(reinterpret_cast<const int32_t*>(T) + 29);
   tOut = t; stOut = st; return true;
 }
-// returns 1 hit / 0 miss / -1 the CAP-entry stack overflowed (the caller defers the ray to the generic kernel or flags a device error)
-// Loop shape ("while-while"): every lane first descends inner nodes until it HOLDS A LEAF (or is finished), then the warp tests triangles
-// together -- the triangle test is the expensive, divergence-prone part (measured: 11.6 of 32 lanes active in the one-loop form).  The visiting
-// order changes nothing: the result is the minimum over all accepted leaves, ties resolved by reference rank.
-template <bool ONE_RAY, int CAP>
-__device__ DRT_LEAN_INLINE int leanClosest(const DScene& S, const FBvh& B, const D3 bo, const D3 ba, const D3 to, const D3 td, const D3 rawDir, Hit& out, TraceCounters* tc) {
-  LeanRay R; R.ox = bo.x; R.oy = bo.y; R.oz = bo.z;
-  const double ax = ba.x, ay = ba.y, az = ba.z;
-  R.ix = 1.0 / ax; R.iy = 1.0 / ay; R.iz = 1.0 / az; R.px = ax > 0; R.py = ay > 0; R.pz = az > 0;
-  const double tox = ONE_RAY ? R.ox : to.x, toy = ONE_RAY ? R.oy : to.y, toz = ONE_RAY ? R.oz : to.z;
-  const double tdx = ONE_RAY ? ax : td.x, tdy = ONE_RAY ? ay : td.y, tdz = ONE_RAY ? az : td.z;
-  // (stack array and its scalar state are separate variables: a struct holding a dynamically indexed array lives in local memory as a whole,
-  //  and `sp` would be re-loaded and re-stored on every push and pop)
-  uint2 stkE[CAP]; int sp = 0; bool overflow = false; const bool stdBox = S.accelMode == 2;
-  double bestT = DRT_DMAX; int bestTri = -1, bestRank = 0x7fffffff, bestSt = 0;
-  int32_t ref = B.fastRoot; bool alive = true;
-  auto popNext = [&]() { alive = false; while (sp > 0) { const uint2 e = stkE[--sp]; if ((double)__uint_as_float(e.y) < bestT) { ref = (int32_t)e.x; alive = true; break; } } };
-  while (true) {
-    while (alive && ref >= 0) {
-      const double2* q = reinterpret_cast<const double2*>(S.fnodes + ref);
-      const double2 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2), q3 = __ldg(q + 3), q4 = __ldg(q + 4), q5 = __ldg(q + 5);
-      const int4 lk = __ldg(reinterpret_cast<const int4*>(q) + 6);
-      if (tc) tc->box += 2;
-      double teL, teR;
-      const int ql = stdBox ? leanBoxStd(q0.x, q0.y, q1.x, q1.y, q2.x, q2.y, R, teL) : leanBox(q0.x, q0.y, q1.x, q1.y, q2.x, q2.y, R, teL);
-      const int qr = stdBox ? leanBoxStd(q3.x, q3.y, q4.x, q4.y, q5.x, q5.y, R, teR) : leanBox(q3.x, q3.y, q4.x, q4.y, q5.x, q5.y, R, teR);
-      bool hl = ql > 0, hr = qr > 0;
-      if (ql >= 0) teL *= 0.999999999999999; else { teL = boxExactEntry(reinterpret_cast<const double*>(q), R.ox, R.oy, R.oz, ax, ay, az); hl = teL > 0; }
-      if (qr >= 0) teR *= 0.999999999999999; else { teR = boxExactEntry(reinterpret_cast<const double*>(q) + 6, R.ox, R.oy, R.oz, ax, ay, az); hr = teR > 0; }
-      hl = hl && teL < bestT; hr = hr && teR < bestT;
-      const int32_t cl = childRef(lk.x, lk.z), cr = childRef(lk.y, lk.w);
-      if (hl && hr) {
-        const bool rightFirst = teR < teL;
-        if (sp < CAP) stkE[sp++] = make_uint2((uint32_t)(rightFirst ? cl : cr), __float_as_uint(__double2float_rd(rightFirst ? teL : teR))); else overflow = true;
-        ref = rightFirst ? cr : cl;
-      } else if (hl) ref = cl;
-      else if (hr) ref = cr;
-      else popNext();
-    }
-    if (!alive) break;
-    {
-      const int code = ~ref, cnt = code & 7, first = code >> 3;
-      for (int i = 0; i < cnt; ++i) {
-        double t; int st; int32_t rank; if (tc) ++tc->prim;
-        if (leanTri(S.tris + first + i, tox, toy, toz, tdx, tdy, tdz, bestT, t, st, rank) && (t < bestT || rank < bestRank)) { bestT = t; bestTri = first + i; bestRank = rank; bestSt = st; }
-      }
-    }
-    popNext();
-  }
-  if (overflow) return -1;
-  if (bestTri < 0) return 0;
-  out.t = bestT; out.prim = S.tris[bestTri].prim; out.arg0 = 0; out.arg1 = 0; out.state = bestSt; out.hitXform = B.triHitXform; out.shaderOverride = -1; out.inst = -1;
-  out.loc = d3((tdx * bestT) + tox, (tdy * bestT) + toy, (tdz * bestT) + toz); out.rawDir = rawDir; return 1;
-}
-template <bool ONE_RAY, int CAP>
-__device__ DRT_LEAN_INLINE int leanShadow(const DScene& S, const FBvh& B, const D3 bo, const D3 ba, const D3 to, const D3 td, double dist, TraceCounters* tc) {
-  LeanRay R; R.ox = bo.x; R.oy = bo.y; R.oz = bo.z;
-  const double ax = ba.x, ay = ba.y, az = ba.z;
-  R.ix = 1.0 / ax; R.iy = 1.0 / ay; R.iz = 1.0 / az; R.px = ax > 0; R.py = ay > 0; R.pz = az > 0;
-  const double tox = ONE_RAY ? R.ox : to.x, toy = ONE_RAY ? R.oy : to.y, toz = ONE_RAY ? R.oz : to.z;
-  const double tdx = ONE_RAY ? ax : td.x, tdy = ONE_RAY ? ay : td.y, tdz = ONE_RAY ? az : td.z;
-  int32_t stkE[CAP]; int sp = 0; bool overflow = false; const bool stdBox = S.accelMode == 2;
-  int32_t ref = B.fastRoot; bool alive = true, found = false;
-  auto accept = [&](int q, double te, const double* box6) {       // (dist - entry) > eps, with the exact entry t only when it is too close to call
-    if (q == 0) return false;
-    if (stdBox) return (dist - te) > DRT_EPS;
-    if (q > 0) { const double diff = dist - te, m = 1e-13 * (fabs(dist) + fabs(te)); if (diff > DRT_EPS + m) return true; if (diff < DRT_EPS - m) return false; }
-    const double tx = boxExactEntry(box6, R.ox, R.oy, R.oz, ax, ay, az); return tx > 0 && (dist - tx) > DRT_EPS;
-  };
-  while (true) {
-    while (alive && ref >= 0) {
-      const double2* q = reinterpret_cast<const double2*>(S.fnodes + ref);
-      const double2 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2), q3 = __ldg(q + 3), q4 = __ldg(q + 4), q5 = __ldg(q + 5);
-      const int4 lk = __ldg(reinterpret_cast<const int4*>(q) + 6);
-      if (tc) tc->box += 2;
-      double teL, teR;
-      const int ql = stdBox ? leanBoxStd(q0.x, q0.y, q1.x, q1.y, q2.x, q2.y, R, teL) : leanBox(q0.x, q0.y, q1.x, q1.y, q2.x, q2.y, R, teL);
-      const int qr = stdBox ? leanBoxStd(q3.x, q3.y, q4.x, q4.y, q5.x, q5.y, R, teR) : leanBox(q3.x, q3.y, q4.x, q4.y, q5.x, q5.y, R, teR);
-      const bool hl = accept(ql, teL, reinterpret_cast<const double*>(q)), hr = accept(qr, teR, reinterpret_cast<const double*>(q) + 6);
-      const int32_t cl = childRef(lk.x, lk.z), cr = childRef(lk.y, lk.w);
-      if (hl && hr) { if (sp < CAP) stkE[sp++] = cr; else overflow = true; ref = cl; }
-      else if (hl) ref = cl;
-      else if (hr) ref = cr;
-      else if (sp > 0) ref = stkE[--sp];
-      else alive = false;
-    }
-    if (!alive) break;
-    {
-      const int code = ~ref, cnt = code & 7, first = code >> 3;
-      for (int i = 0; i < cnt; ++i) {
-        double t; int st; int32_t rank; if (tc) ++tc->prim;
-        if (leanTri(S.tris + first + i, tox, toy, toz, tdx, tdy, tdz, DRT_DMAX, t, st, rank) && (dist - t) > DRT_EPS) { found = true; break; }
-      }
-    }
-    if (found) break;
-    if (sp > 0) ref = stkE[--sp]; else alive = false;
-  }
-  if (found) return 1;
-  return overflow ? -1 : 0;
-}
 // ---------------------------------------------------------------------------------------------------------------
-// FP32 pre-test descent of the lean kernels.
-// A node visit of the FP64 descent above costs ~160 instructions, 46 of them on the half-rate FP64 pipe.  Almost every box decision is far
-// from its boundary, so it is taken in FP32 on a 64-byte mirror of the node (FNode32: 4 loads instead of 7) under a rigorous error bound, and
-// only an undecidable box goes to the reference's own FP64 test (true divisions, out of line).  Bound: with u = 2^-24, b32 = fl(b),
-// inv32 = fl(1/a), oi32 = fl(o/a) and t32 = fma(b32, inv32, -oi32) (one rounding),
+// The one descent through a fast BVH (FP32 pre-test), closest hit and any hit.
+// Almost every box decision is far from its boundary, so it is taken in FP32 on a 64-byte mirror of the node (FNode32: 4 loads instead of 7)
+// under a rigorous error bound, and only an undecidable box goes to the reference's own FP64 test (true divisions, out of line).  Bound: with
+// u = 2^-24, b32 = fl(b), inv32 = fl(1/a), oi32 = fl(o/a) and t32 = fma(b32, inv32, -oi32) (one rounding),
 //     |t32 - (b - o)/a| <= u (3 |b/a| + 2 |o/a|) (1 + O(u)),        |b| <= absMax (per BVH, per axis),
 // and the reference's FP64 quotient is within 2.3e-16 (|b/a| + |o/a|) of the same real number.  M = 1.1 u max_axis (3 absMax + 2 |o|) |1/a|
 // (+ a denormal floor) therefore bounds the error of every slab value of the ray; min / max are 1-Lipschitz, so near32 / far32 are within M of
 // the reference's biggestMin / min(tMax).  A box is ACCEPTED when far32 - near32 > 2M and near32 > M (=> far > near and near > 0 in the
 // reference's arithmetic), REJECTED when far32 - near32 < -2M or near32 < -M, otherwise undecided.  Rays whose reciprocals or products leave the
-// comfortable float range get M = +inf: every comparison fails and every box takes the exact test.  Entry times only order and prune
-// (conservative lower bound near32 - M), exactly as in the FP64 descent; triangles are always tested in FP64.
+// comfortable float range get M = +inf: every comparison fails and every box takes the exact test -- this is how the generic kernels serve an
+// axis-parallel ray (a reciprocal of +-inf).  Entry times only order and prune (conservative lower bound near32 - M); triangles are always
+// tested in FP64.
 struct Lean32 { float ix, iy, iz, ox, oy, oz, M, M2; };
 __device__ __forceinline__ Lean32 makeLean32(const FBvh& B, double ox, double oy, double oz, const D3& inv) {      // inv = rayInv() of the ray the boxes are tested with
   const double ix = inv.x, iy = inv.y, iz = inv.z; Lean32 L;
@@ -673,17 +410,23 @@ __device__ __forceinline__ int leanBox32(float mnx, float mny, float mnz, float 
   if (gap < -L.M2 || near_ < -L.M) return 0;
   return -1;
 }
-// conventional slab test (LBVH mode) out of line, the arithmetic of leanBoxStd(): entry t (>= 0) or -1
-__device__ __noinline__ double boxStdEntry(const double* __restrict__ box6, double ox, double oy, double oz, double ax, double ay, double az) {
-  LeanRay R; R.ox = ox; R.oy = oy; R.oz = oz; R.ix = 1.0 / ax; R.iy = 1.0 / ay; R.iz = 1.0 / az; R.px = ax > 0; R.py = ay > 0; R.pz = az > 0;
-  double te; return leanBoxStd(__ldg(box6), __ldg(box6 + 1), __ldg(box6 + 2), __ldg(box6 + 3), __ldg(box6 + 4), __ldg(box6 + 5), R, te) > 0 ? te : -1.0;
-}
 // tScale (<= 1): lower bound of |ba| when the triangles see the NORMALISED direction of a ray whose box-space direction ba is shorter than unit
 // length (an instance that enlarges its mesh, SURVEY Q7): a box entered at te (box units) is entered at te |ba| in triangle units, so a subtree
 // may be skipped against the best hit only if te * tScale >= bestT.  1 when |ba| >= 1 (te itself is then the conservative bound).
 __device__ __forceinline__ float leanScale(double len2) { return len2 >= 1.0 ? 1.0f : __double2float_rd(sqrt(len2)) * 0.999999f; }
-template <int CAP>
-__device__ DRT_LEAN_INLINE int leanClosest32(const DScene& S, const FBvh& B, const D3 bo, const D3 ba, const D3 binv, const D3 to, const D3 td, const D3 rawDir, Hit& out, const double bound, const float tScale = 1.0f) {
+// Closest hit inside one fast BVH (root box already accepted by the caller).  (bo, ba, binv) is the ray the boxes are tested with, (to, td) the
+// ray the triangles are tested with (see SURVEY Q7 for why they can differ).  Result: the minimum-t hit over every leaf whose chain of boxes is
+// accepted -- the set the reference's left-first recursion searches; equal-t candidates resolve to the lower reference rank, i.e. the reference's
+// visiting order.  It is written to `out` only when strictly closer than `bound`.  Returns 1 hit / 0 miss / -1 the CAP-entry stack overflowed
+// (the caller defers the ray to the generic kernel or flags a device error).  tc (counter builds): node visits (two boxes each), triangle tests.
+// Loop shape ("while-while"): every lane first descends inner nodes until it HOLDS A LEAF (or is finished), then the warp tests triangles
+// together -- the triangle test is the expensive, divergence-prone part (measured: 11.6 of 32 lanes active in the one-loop form).
+// Stack entry: x = child reference (>= 0 inner node, < 0: ~tri-leaf code), y = bits of the lower bound of its box-entry t.  (The stack array and
+// its scalar state are separate variables: a struct holding a dynamically indexed array lives in local memory as a whole, and `sp` would be
+// re-loaded and re-stored on every push and pop.)
+template <int CAP, bool ANY_DIR = false>
+__device__ DRT_LEAN_INLINE int leanClosest32(const DScene& S, const FBvh& B, const D3 bo, const D3 ba, const D3 binv, const D3 to, const D3 td, const D3 rawDir, Hit& out, const double bound,
+                                             const float tScale = 1.0f, TraceCounters* tc = nullptr) {
   const Lean32 L = makeLean32(B, bo.x, bo.y, bo.z, binv);
   const bool stdBox = S.accelMode == 2;
   uint2 stkE[CAP]; int sp = 0; bool overflow = false;
@@ -694,7 +437,7 @@ __device__ DRT_LEAN_INLINE int leanClosest32(const DScene& S, const FBvh& B, con
   auto popNext = [&]() { alive = false; while (sp > 0) { const uint2 e = stkE[--sp]; if (__uint_as_float(e.y) < bestTf) { ref = (int32_t)e.x; alive = true; break; } } };
   auto exact = [&](const FNode* nd, int side) -> float {     // undecided box: the reference's own test; returns a lower bound of the entry t, or -1 (rejected)
     const double* b6 = reinterpret_cast<const double*>(nd) + 6 * side;
-    const double te = stdBox ? boxStdEntry(b6, bo.x, bo.y, bo.z, ba.x, ba.y, ba.z) : boxExactEntry(b6, bo.x, bo.y, bo.z, ba.x, ba.y, ba.z);
+    const double te = stdBox ? boxStdEntry<ANY_DIR>(b6, bo.x, bo.y, bo.z, ba.x, ba.y, ba.z) : boxExactEntry(b6, bo.x, bo.y, bo.z, ba.x, ba.y, ba.z);
     return (stdBox ? te >= 0 : te > 0) ? __double2float_rd(te) : -1.0f;
   };
   while (true) {
@@ -702,6 +445,7 @@ __device__ DRT_LEAN_INLINE int leanClosest32(const DScene& S, const FBvh& B, con
     while (alive && ref >= 0) {
       const float4* q = reinterpret_cast<const float4*>(S.fnodes32 + ref);
       const float4 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2); const int4 lk = __ldg(reinterpret_cast<const int4*>(q) + 3);
+      if (tc) tc->box += 2;
       float teL, teR;
       const int ql = leanBox32(q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, L, stdBox, teL), qr = leanBox32(q1.z, q1.w, q2.x, q2.y, q2.z, q2.w, L, stdBox, teR);
       bool hl = ql > 0, hr = qr > 0;
@@ -723,7 +467,7 @@ __device__ DRT_LEAN_INLINE int leanClosest32(const DScene& S, const FBvh& B, con
     {
       const int code = ~ref, cnt = code & 7, first = code >> 3;
       for (int i = 0; i < cnt; ++i) {
-        double t; int st; int32_t rank;
+        double t; int st; int32_t rank; if (tc) ++tc->prim;
         if (leanTri(S.tris + first + i, to.x, to.y, to.z, td.x, td.y, td.z, bestT, t, st, rank) && (t < bestT || rank < bestRank)) { bestT = t; bestTf = __fdiv_ru(__double2float_ru(t), tScale); bestTri = first + i; bestRank = rank; bestSt = st; }
       }
     }
@@ -735,8 +479,9 @@ __device__ DRT_LEAN_INLINE int leanClosest32(const DScene& S, const FBvh& B, con
   out.t = bestT; out.prim = S.tris[bestTri].prim; out.arg0 = 0; out.arg1 = 0; out.state = bestSt; out.hitXform = B.triHitXform; out.shaderOverride = -1; out.inst = -1; out.pad0 = 0;
   out.loc = d3((td.x * bestT) + to.x, (td.y * bestT) + to.y, (td.z * bestT) + to.z); out.rawDir = rawDir; return 1;
 }
-template <int CAP>
-__device__ DRT_LEAN_INLINE int leanShadow32(const DScene& S, const FBvh& B, const D3 bo, const D3 ba, const D3 binv, const D3 to, const D3 td, double dist) {
+// Any hit inside one fast BVH: (dist - t) > eps for a triangle, every box on the way accepted with (dist - entry) > eps.  Rays and results as leanClosest32.
+template <int CAP, bool ANY_DIR = false>
+__device__ DRT_LEAN_INLINE int leanShadow32(const DScene& S, const FBvh& B, const D3 bo, const D3 ba, const D3 binv, const D3 to, const D3 td, double dist, TraceCounters* tc = nullptr) {
   const Lean32 L = makeLean32(B, bo.x, bo.y, bo.z, binv);
   const bool stdBox = S.accelMode == 2;
   // (dist - entry) > eps decided on near32 when it clears the bound: entry < dist - eps - M  /  entry > dist - eps + M
@@ -747,7 +492,7 @@ __device__ DRT_LEAN_INLINE int leanShadow32(const DScene& S, const FBvh& B, cons
     if (q == 0) return false;
     if (q > 0) { if (te < accBelow) return true; if (te > rejAbove) return false; }
     const double* b6 = reinterpret_cast<const double*>(nd) + 6 * side;
-    const double tx = stdBox ? boxStdEntry(b6, bo.x, bo.y, bo.z, ba.x, ba.y, ba.z) : boxExactEntry(b6, bo.x, bo.y, bo.z, ba.x, ba.y, ba.z);
+    const double tx = stdBox ? boxStdEntry<ANY_DIR>(b6, bo.x, bo.y, bo.z, ba.x, ba.y, ba.z) : boxExactEntry(b6, bo.x, bo.y, bo.z, ba.x, ba.y, ba.z);
     return (stdBox ? tx >= 0 : tx > 0) && (dist - tx) > DRT_EPS;
   };
   while (true) {
@@ -755,6 +500,7 @@ __device__ DRT_LEAN_INLINE int leanShadow32(const DScene& S, const FBvh& B, cons
     while (alive && ref >= 0) {
       const float4* q = reinterpret_cast<const float4*>(S.fnodes32 + ref);
       const float4 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2); const int4 lk = __ldg(reinterpret_cast<const int4*>(q) + 3);
+      if (tc) tc->box += 2;
       float teL, teR;
       const int ql = leanBox32(q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, L, stdBox, teL), qr = leanBox32(q1.z, q1.w, q2.x, q2.y, q2.z, q2.w, L, stdBox, teR);
       const bool hl = accept(ql, teL, S.fnodes + ref, 0), hr = accept(qr, teR, S.fnodes + ref, 1);
@@ -771,7 +517,7 @@ __device__ DRT_LEAN_INLINE int leanShadow32(const DScene& S, const FBvh& B, cons
     {
       const int code = ~ref, cnt = code & 7, first = code >> 3;
       for (int i = 0; i < cnt; ++i) {
-        double t; int st; int32_t rank;
+        double t; int st; int32_t rank; if (tc) ++tc->prim;
         if (leanTri(S.tris + first + i, to.x, to.y, to.z, td.x, td.y, td.z, DRT_DMAX, t, st, rank) && (dist - t) > DRT_EPS) { found = true; break; }
       }
     }
@@ -783,10 +529,6 @@ __device__ DRT_LEAN_INLINE int leanShadow32(const DScene& S, const FBvh& B, cons
   return overflow ? -1 : 0;
 }
 __device__ __forceinline__ bool sameRay(const Ray& trans, const Ray& r) { return trans.o.x == r.o.x && trans.o.y == r.o.y && trans.o.z == r.o.z && trans.a.x == r.d.x && trans.a.y == r.d.y && trans.a.z == r.d.z; }
-// may this BVH be searched out of the reference's order for this pair of rays?  (SURVEY Q7: through an instance the triangles see a
-// re-normalised direction, so hit t and box-entry t are in different units; pruning stays conservative only if the local direction
-// was at least unit length)
-__device__ __forceinline__ bool fastUsable(const DScene& S, const FBvh& B, double localDirLen2) { return S.accelMode != 0 && B.fast != 0 && localDirLen2 >= 1.0; }
 
 #define DRT_STACK 48
 struct Frame { int32_t node; double tL; };     // node >= 0: "after left" of that node; node == -1: "after right", tL saved
@@ -853,7 +595,6 @@ __device__ __forceinline__ double leafClosest(const DScene& S, int listIdx, Ray&
 template <int F, int LVL>
 __device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int idx, Ray& _ray, const Ray& trans, int transXf, double time, Hit& out, TraceCounters* tc, double bound) {
   constexpr bool LITERAL = (LVL == 1) ? ((F & TF_LITERAL1) != 0) : ((F & TF_LEVEL2) != 0);      // literal recursion compiled in at this level?
-  constexpr bool NONLEAN = (LVL == 1) ? ((F & TF_NONLEAN) != 0) : ((F & TF_LEVEL2) != 0);
   const D3 inv = rayInv(trans);
   if (kind == OK_LIST) {
     const FList& L = S.lists[idx];
@@ -868,35 +609,27 @@ __device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int i
   if (tc) ++tc->box;
   if (!boxHit(B.bmin, B.bmax, trans, inv)) return 0;
   if (S.accelMode != 0 && B.fast != 0) {
-    const double len2 = _ray.norm ? 1.0 : dot3(_ray.d, _ray.d);
-    constexpr bool SCALED = DRT_LEAN && DRT_LEAN32 && F != TF_ALL;          // the FP32 lean search prunes with a scaled bound when the local direction is shorter than 1
-    if (fastUsable(S, B, len2) || (SCALED && len2 > 1e-200)) {
+    const double len2 = _ray.norm ? 1.0 : dot3(_ray.d, _ray.d);      // < 1 through an instance that enlarges its mesh: the search scales its bound (leanScale)
+    if (len2 > 1e-200) {
       // what every leaf child of this mesh would be tested with.  getTransformedRay is a pure function of (ray, CTM) once the source direction is
       // unit length, so when `trans` was formed from this very ray with the triangles' own CTM the two rays are the same bits: nothing to recompute
       const bool sameXf = _ray.norm && transXf == B.triXform;
       const Ray r = sameXf ? trans : xfRay(_ray, S.xforms[B.triXform].inv);
-      const bool one = sameXf || sameRay(trans, r);
-#if DRT_LEAN
-      if (regularDir(trans.a)) {
-        // one instantiation per lean kernel (one traversal stack in its frame): flat scenes test boxes and triangles with the same ray, scenes
-        // with instanced meshes need the two-ray form (which gives the same bits when both rays coincide); a flat-scene kernel defers the rest
-        if constexpr (F == TF_ALL) {
-          const int got = one ? leanClosest<true, DRT_FSTACK>(S, B, trans.o, trans.a, r.o, r.d, _ray.d, out, tc) : leanClosest<false, DRT_FSTACK>(S, B, trans.o, trans.a, r.o, r.d, _ray.d, out, tc);
-          if (got < 0) { flagError(1u); return 0; }
-          return got;
-        } else {
-#if DRT_LEAN32
+      if constexpr (F == TF_ALL) {
+        const int got = leanClosest32<DRT_FSTACK, true>(S, B, trans.o, trans.a, inv, r.o, r.d, _ray.d, out, bound, leanScale(len2), tc);
+        if (got < 0) { flagError(1u); return 0; }
+        return got;
+      } else {
+        // the lean kernels defer axis-parallel rays.  One instantiation per lean kernel (one traversal stack in its frame): scenes with instanced
+        // meshes need the two-ray form (which gives the same bits when both rays coincide), flat scenes test boxes and triangles with the same ray
+        // and defer the rest
+        const bool one = sameXf || sameRay(trans, r);
+        if (regularDir(trans.a)) {
           if constexpr ((F & TF_LITERAL1) != 0) return leanClosest32<DRT_LSTACK>(S, B, trans.o, trans.a, inv, r.o, r.d, _ray.d, out, bound, leanScale(len2));
           else { if (!one) return -1; return leanClosest32<DRT_LSTACK>(S, B, trans.o, trans.a, inv, trans.o, trans.a, _ray.d, out, bound); }      // flat scenes: one ray, one register set
-#else
-          if constexpr ((F & TF_LITERAL1) != 0) return leanClosest<false, DRT_LSTACK>(S, B, trans.o, trans.a, r.o, r.d, _ray.d, out, tc);
-          else { if (!one) return -1; return leanClosest<true, DRT_LSTACK>(S, B, trans.o, trans.a, r.o, r.d, _ray.d, out, tc); }
-#endif
         }
       }
-#endif
-      if constexpr (!NONLEAN) return -1;
-      else return (one ? fastClosest<true>(S, B, trans, r, _ray.d, out, tc) : fastClosest<false>(S, B, trans, r, _ray.d, out, tc)) ? 1 : 0;
+      return -1;
     }
   }
   if constexpr (!LITERAL) return -1;
@@ -943,14 +676,14 @@ __device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int i
 
 // myScene.findClosestRayHit: linear scan of the top-level list, first-inserted wins among equal t.
 // The accel searches take `bound`: they write their winner to the record they are given only if it is strictly closer than bound -- the same
-// decision as "h.t < best.t" on a separate record.  The flat lean variants (no literal recursion, no generic descent: every search they reach
-// honours bound) pass `best` itself, so a single Hit lives across the BVH walk instead of two, and they carry only the winner's key across
-// it: which top-level object (wTop) and, in best.pad0, which list child produced it.  Its hit point and recorded direction are formed once,
-// after the loop, from the same transformed ray the winning test used: getTransformedRay is a pure function of (unit-length ray, CTM), so the
-// recomputed ray has the bits the loop had.
+// decision as "h.t < best.t" on a separate record.  The flat lean variants (no literal recursion: every search they reach honours bound) pass
+// `best` itself, so a single Hit lives across the BVH walk instead of two, and they carry only the winner's key across it: which top-level
+// object (wTop) and, in best.pad0, which list child produced it.  Its hit point and recorded direction are formed once, after the loop, from
+// the same transformed ray the winning test used: getTransformedRay is a pure function of (unit-length ray, CTM), so the recomputed ray has
+// the bits the loop had.
 template <int F>
 __device__ __forceinline__ int closestHitT(const DScene& S, Ray& ray, double time, Hit& best, TraceCounters* tc) {
-  constexpr bool IN_PLACE = DRT_LEAN && DRT_LEAN32 && (F & (TF_LITERAL1 | TF_NONLEAN)) == 0;
+  constexpr bool IN_PLACE = (F & TF_LITERAL1) == 0;
   hitReset(best);
   Hit h; if constexpr (!IN_PLACE) hitReset(h);
   Ray tr; int trXf = -1;        // consecutive top-level objects often share one CTM (a polygon soup read under one transform): the transformed
@@ -1115,7 +848,6 @@ __device__ __forceinline__ int instTreeShadow(const DScene& S, const FBvh& B, Ra
 template <int F, int LVL>
 __device__ __forceinline__ int accelShadowImpl(const DScene& S, int kind, int idx, Ray& _ray, const Ray& trans, int transXf, double time, double dist, TraceCounters* tc) {
   constexpr bool LITERAL = (LVL == 1) ? ((F & TF_LITERAL1) != 0) : ((F & TF_LEVEL2) != 0);
-  constexpr bool NONLEAN = (LVL == 1) ? ((F & TF_NONLEAN) != 0) : ((F & TF_LEVEL2) != 0);
   const D3 inv = rayInv(trans);
   XfCache xc; xc.xf = -1;
   if (kind == OK_LIST) return listShadow<F, LVL>(S, idx, _ray, trans, inv, time, dist, tc, xc);
@@ -1123,29 +855,21 @@ __device__ __forceinline__ int accelShadowImpl(const DScene& S, int kind, int id
   if (S.accelMode != 0 && B.fast != 0) {                              // any-hit does not depend on the visiting order
     const bool sameXf = _ray.norm && transXf == B.triXform;          // see accelClosestImpl
     const Ray r = sameXf ? trans : xfRay(_ray, S.xforms[B.triXform].inv);
-    const bool one = sameXf || sameRay(trans, r);
-#if DRT_LEAN
-    if (regularDir(trans.a)) {
-      if constexpr (F == TF_ALL) {
-        const int got = one ? leanShadow<true, DRT_FSTACK>(S, B, trans.o, trans.a, r.o, r.d, dist, tc) : leanShadow<false, DRT_FSTACK>(S, B, trans.o, trans.a, r.o, r.d, dist, tc);
-        if (got < 0) { flagError(1u); return 0; }
-        return got;
-      } else {
-#if DRT_LEAN32
+    if constexpr (F == TF_ALL) {
+      const int got = leanShadow32<DRT_FSTACK, true>(S, B, trans.o, trans.a, inv, r.o, r.d, dist, tc);
+      if (got < 0) { flagError(1u); return 0; }
+      return got;
+    } else {
+      const bool one = sameXf || sameRay(trans, r);
+      if (regularDir(trans.a)) {
         if constexpr ((F & TF_LITERAL1) != 0) return leanShadow32<DRT_LSTACK>(S, B, trans.o, trans.a, inv, r.o, r.d, dist);
         else { if (!one) return -1; return leanShadow32<DRT_LSTACK>(S, B, trans.o, trans.a, inv, trans.o, trans.a, dist); }
-#else
-        if constexpr ((F & TF_LITERAL1) != 0) return leanShadow<false, DRT_LSTACK>(S, B, trans.o, trans.a, r.o, r.d, dist, tc);
-        else { if (!one) return -1; return leanShadow<true, DRT_LSTACK>(S, B, trans.o, trans.a, r.o, r.d, dist, tc); }
-#endif
       }
     }
-#endif
-    if constexpr (!NONLEAN) return -1;
-    else return (one ? fastShadow<true>(S, B, trans, r, dist, tc) : fastShadow<false>(S, B, trans, r, dist, tc)) ? 1 : 0;
+    return -1;
   }
   if constexpr (!LITERAL) return -1;
-  else if constexpr (F != TF_ALL && LVL == 1 && DRT_TWOLEVEL) return instTreeShadow<F>(S, B, _ray, trans, inv, time, dist);
+  else if constexpr (F != TF_ALL && LVL == 1) return instTreeShadow<F>(S, B, _ray, trans, inv, time, dist);
   else {
   int32_t stack[DRT_STACK]; int sp = 0; int32_t node = B.root;
   while (true) {

@@ -50,12 +50,19 @@ def test_fast_mode_counters_do_less_work(drt, gpu_ctx_factory):
 
 
 def test_fast_mode_explicit_rays_from_everywhere(drt, gpu_ctx_factory):
-    """Rays starting inside / on / outside the meshes' boxes: closest-hit IDs and t must be identical in both modes."""
+    """Rays starting inside / on / outside the meshes' boxes, a share of them (almost) axis-parallel: closest-hit IDs and t must be identical
+    in both modes."""
     rng = np.random.default_rng(3)
     for name in ("p3_t09", "p3_t10", "p3_t11_sierp"):
         n = 200000
         org = rng.uniform(-3, 3, size=(n, 3)); org[:, 2] -= 3
         d = rng.normal(size=(n, 3))
+        # rows [0, 2k): exactly axis-parallel (one component +0.0 or -0.0, two in the first k); rows [2k, 3k): one component around 1e-17
+        k = n // 8; rows = np.arange(2 * k)
+        zero = np.where(rng.random(size=(2 * k, 3)) < 0.5, 0.0, -0.0); ax = rng.integers(0, 3, size=2 * k)
+        d[rows, ax] = zero[rows, ax]
+        d[rows[:k], (ax[:k] + 1) % 3] = zero[rows[:k], (ax[:k] + 1) % 3]
+        d[np.arange(2 * k, 3 * k), rng.integers(0, 3, size=k)] = rng.choice([-1e-17, 1e-17], size=k) * rng.uniform(0.5, 2.0, size=k)
         res = []
         for accel in (drt.ACCEL_REFERENCE, drt.ACCEL_REFERENCE_FAST):
             ctx = gpu_ctx_factory()
@@ -64,7 +71,7 @@ def test_fast_mode_explicit_rays_from_everywhere(drt, gpu_ctx_factory):
             ctx.close()
         assert np.array_equal(res[0][0], res[1][0]), name
         assert np.array_equal(res[0][1], res[1][1]), name
-        assert (res[0][0][:, 0] >= 0).sum() > 1000
+        assert (res[0][0][:, 0] >= 0).sum() > 1000 and (res[0][0][:2 * k, 0] >= 0).sum() > 1000
 
 
 # ---- kernel variants and the sync-free wavefront loop (round 2) ------------------------------------------------------------------------

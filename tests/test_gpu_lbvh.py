@@ -39,14 +39,21 @@ def test_lbvh_explicit_rays_from_outside(drt, gpu_ctx_factory):
     u = rng.normal(size=(n, 3)); u /= np.linalg.norm(u, axis=1, keepdims=True)
     org = 9.0 * u + np.array([0, 0, -3.0])                      # outside every mesh box of the scenes below
     tgt = rng.uniform(-1.2, 1.2, size=(n, 3)) + np.array([0, 0, -3.0])
+    # axis-parallel rays aimed at targets of the same region: one direction component +-1, the others +0.0 or -0.0
+    m = 100000
+    d2 = np.where(rng.random(size=(m, 3)) < 0.5, 0.0, -0.0)
+    d2[np.arange(m), rng.integers(0, 3, size=m)] = rng.choice([-1.0, 1.0], size=m)
+    tgt2 = rng.uniform(-1.2, 1.2, size=(m, 3)) + np.array([0, 0, -3.0])
+    dirs = np.concatenate([tgt - org, d2])
+    org = np.concatenate([org, tgt2 - 9.0 * d2])
     for name in ("p3_t09", "p3_t08"):
         res = []
         for accel in (drt.ACCEL_REFERENCE, drt.ACCEL_LBVH):
             ctx = gpu_ctx_factory()
             s = drt.Scene.from_cli(ctx, name + ".cli", accel=accel)
-            res.append(s.trace_rays(org, tgt - org))
+            res.append(s.trace_rays(org, dirs))
             ctx.close()
-        assert (res[0][0][:, 0] >= 0).sum() > 10000
+        assert (res[0][0][:n, 0] >= 0).sum() > 10000 and (res[0][0][n:, 0] >= 0).sum() > 1000
         assert np.array_equal(res[0][0], res[1][0]) and np.array_equal(res[0][1], res[1][1]), name
 
 
