@@ -171,14 +171,19 @@ __global__ void k_photon_bounds(const PhotonRec* __restrict__ rec, long long n, 
     blockMinMax[blockIdx.x * 6 + threadIdx.x] = a; blockMinMax[blockIdx.x * 6 + 3 + threadIdx.x] = b; }
 }
 __device__ __forceinline__ int phCellCoord(double v, double gmin, double cell, int dim) { int c = (int)floor((v - gmin) / cell); return c < 0 ? 0 : (c >= dim ? dim - 1 : c); }
+// Two-level key of fine cell (fx, fy, fz) in a grid of dx x dy x . coarse cells: the coarse cell (side = search radius, x fastest) shifted left
+// by 6, OR the 4x4x4 fine sub-cell.  Consecutive keys therefore cover a row of coarse cells along x and a run of fine cells along x inside one
+// coarse cell (phRowRange): each is one contiguous photon range of cellStart.
+__device__ __forceinline__ uint32_t phKey(uint32_t dx, uint32_t dy, uint32_t fx, uint32_t fy, uint32_t fz) {
+  return ((((fz >> 2) * dy + (fy >> 2)) * dx + (fx >> 2)) << 6) | ((fz & 3u) << 4) | ((fy & 3u) << 2) | (fx & 3u);
+}
 __global__ void k_photon_cellkeys(const PhotonRec* __restrict__ rec, long long n, PhGrid G, uint32_t* __restrict__ keys, uint32_t* __restrict__ cellCount) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; if (i >= n) return;
   const PhotonRec r = rec[i];
-  // two-level key: coarse cell (side = search radius, x fastest: a run of coarse cells along x is one contiguous photon range) and, inside it,
-  // a 4x4x4 fine sub-cell index.  Every coordinate derives from the FINE one, so both levels are consistent with each other.
+  // every coordinate derives from the FINE one, so both levels of the key are consistent with each other
   const double cf = G.cell * 0.25;
   const uint32_t fx = phCellCoord(r.x, G.gmin[0], cf, 4 * G.dim[0]), fy = phCellCoord(r.y, G.gmin[1], cf, 4 * G.dim[1]), fz = phCellCoord(r.z, G.gmin[2], cf, 4 * G.dim[2]);
-  const uint32_t key = ((((fz >> 2) * G.dim[1] + (fy >> 2)) * G.dim[0] + (fx >> 2)) << 6) | ((fz & 3u) << 4) | ((fy & 3u) << 2) | (fx & 3u);
+  const uint32_t key = phKey(G.dim[0], G.dim[1], fx, fy, fz);
   keys[i] = key; atomicAdd(&cellCount[key], 1u);
 }
 // sorted order -> the two 32-byte-per-photon arrays the gather reads with 128-bit loads
@@ -191,24 +196,24 @@ __global__ void k_photon_reorder(const PhotonRec* __restrict__ rec, const uint32
 // ---------------------------------------------------------------------------------------------------------------
 // gather
 // ---------------------------------------------------------------------------------------------------------------
-#ifndef DRT_PH_LANE_MAX
 #define DRT_PH_LANE_MAX 1024u     // candidate count up to which a lane serves its own query
-#endif
 #define DRT_PH_BINS 256
-#ifndef DRT_PH_TIGHT
-#define DRT_PH_TIGHT 1           // search plans shrink their radius to the expected k-th neighbour distance (phMakePlan)
-#endif
-#ifndef DRT_PH_FP32
-#define DRT_PH_FP32 1            // warp tier: FP32 pre-test selection first (phWarpGather32), FP64 radix select as the fallback
-#endif
 #define DRT_PH_LIST 128
-#define DRT_PH_MAXRANGES 160      // candidate ranges of one query: <= 7 x 7 fine rows x 3 runs (fine cube of half-width 3), <= 3 x 3 coarse rows
+// Candidate ranges of one warp query.  Coarse rows: the cell is >= r, so the bounding cube of a sphere of radius r (1 + 1e-7) touches at most
+// 4 cells per axis: <= 4 x 4 rows.  Fine runs: a plan's block is at most 7 fine cells per axis (s <= 3), and 7 consecutive fine cells touch at
+// most 3 coarse cells along x: <= 3 x 7 x 7 = 147 runs.
+#define DRT_PH_MAXRANGES 160
 struct PhWarpShared { uint32_t hist[DRT_PH_BINS]; double listD2[DRT_PH_LIST]; uint32_t listIdx[DRT_PH_LIST]; uint32_t listN; uint32_t pad[3];
                       uint32_t rA[DRT_PH_MAXRANGES + 33], rOff[DRT_PH_MAXRANGES + 33]; };     // non-empty candidate ranges: first photon, exclusive prefix of the lengths (+ sentinels)
 
-// Sum of the powers of the k nearest photons with d^2 < r^2 around p, and the largest of their d^2 -- computed by one warp.
-// Selection = radix select on a 32-bit quantisation of d^2 (monotone in d^2), 8 bits per level over the candidate rows of the grid,
-// finished exactly (double d^2, index tie-break) on the short list of the boundary bin.
+// photon range [a, b) of the cells x0..x1 of one row: the coarse cells of coarse row (y, z), or (fine) the fine cells of fine row (y, z), which
+// must lie inside one coarse cell (x1 <= x0 | 3)
+__device__ __forceinline__ void phRowRange(const DScene& S, bool fine, int y, int z, int x0, int x1, uint32_t& a, uint32_t& b) {
+  const uint32_t c = fine ? 1u : 4u;                                        // fine cells per cell of the row
+  a = S.cellStart[phKey(S.gridDim[0], S.gridDim[1], c * x0, c * y, c * z)];
+  b = S.cellStart[phKey(S.gridDim[0], S.gridDim[1], c * x1, c * y, c * z) + (fine ? 1u : 64u)];     // the key after cell x1
+}
+
 // cells the bounding cube of the search sphere overlaps (radius inflated by 1e-7 so that no photon with d^2 < r^2 can sit in a cell outside
 // the range whatever the rounding of its own cell index); false when the cube misses the grid
 __device__ __forceinline__ bool phCellRange(const DScene& S, D3 p, double radius2, int lo[3], int hi[3]) {
@@ -221,68 +226,125 @@ __device__ __forceinline__ bool phCellRange(const DScene& S, D3 p, double radius
   }
   return ok;
 }
-// r2: search threshold (the scene's r^2, or a smaller guess -- then `needAll`: return false without a result if fewer than k photons are inside it)
-__device__ inline bool phWarpGather(const DScene& S, D3 p, double r2, bool needAll, bool atMostK, int fineHalf, const int lo[3], const int hi[3], PhWarpShared& sh, double sum[3], double& dmax2, unsigned long long* visited) {
-  const unsigned lane = threadIdx.x & 31; const int K = S.g.kNhood;
-  sum[0] = sum[1] = sum[2] = 0; dmax2 = 0;
-  if (S.numPhotons == 0 || K <= 0) return true;
+
+// ---- warp-cooperative tier: the k nearest photons with d^2 < r^2 around p, their summed power and the largest of their d^2, computed by one
+// warp.  The candidates of a query are a list of photon ranges (phWarpRanges); two selections read it, and both end in the same exact
+// resolution of a short boundary list by (double d^2, index) (phRankList).
+
+// The candidate ranges -- coarse rows lo..hi, or the runs of fine cells lo..hi (fine) -- enumerated lane-parallel and compacted (empty ones
+// dropped) into shared memory with the running offset of each.  Range order = z, then y, then x, so photon order within the list is fixed.
+struct PhRanges { uint32_t n, total; };
+__device__ inline PhRanges phWarpRanges(const DScene& S, bool fine, const int lo[3], const int hi[3], PhWarpShared& sh) {
+  const unsigned lane = threadIdx.x & 31;
+  const int x0 = lo[0], x1 = hi[0], y0 = lo[1], z0 = lo[2], nx = fine ? (x1 >> 2) - (x0 >> 2) + 1 : 1, ny = hi[1] - y0 + 1, nz = hi[2] - z0 + 1;
+  int slots = nx * ny * nz;
+  if (slots > DRT_PH_MAXRANGES) { flagError(1u); slots = 0; }      // excluded by the bound above; the host reports an incomplete result
+  uint32_t nRanges = 0, total = 0;
+  for (int s0 = 0; s0 < slots; s0 += 32) {
+    const int slot = s0 + (int)lane; uint32_t a = 0, b = 0;
+    if (slot < slots) {
+      const int ir = slot % nx, fy = y0 + (slot / nx) % ny, fz = z0 + slot / (nx * ny);
+      const int fx = ir == 0 ? x0 : (((x0 >> 2) + ir) << 2);
+      phRowRange(S, fine, fy, fz, fx, fine ? min(x1, fx | 3) : x1, a, b);
+    }
+    const uint32_t len = b - a; const unsigned ne = __ballot_sync(0xffffffffu, len > 0);
+    uint32_t incl = len;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= (unsigned)o) incl += t; }
+    if (len > 0) { const uint32_t at = nRanges + __popc(ne & ((1u << lane) - 1u)); sh.rA[at] = a; sh.rOff[at] = total + incl - len; }
+    nRanges += __popc(ne); total += __shfl_sync(0xffffffffu, incl, 31);
+  }
+  for (uint32_t i = nRanges + lane; i < nRanges + 33; i += 32) { sh.rA[i] = 0; sh.rOff[i] = total; }       // sentinels: empty ranges at the end
+  __syncwarp();
+  return {nRanges, total};
+}
+// f(j, valid) warp-wide for every candidate: range by range, 32 consecutive photons of a range per step
+template <class F> __device__ __forceinline__ void phEachRange(const PhWarpShared& sh, PhRanges R, F&& f) {
+  const unsigned lane = threadIdx.x & 31;
+  for (uint32_t r = 0; r < R.n; ++r) {
+    const uint32_t a = sh.rA[r], b = a + (sh.rOff[r + 1] - sh.rOff[r]);
+    for (uint32_t j0 = a; j0 < b; j0 += 32) f(j0 + lane, j0 + lane < b);
+  }
+}
+// f(j, valid) warp-wide for every candidate, 32 consecutive FLAT indices per step: a fine row run holds ~10-30 photons, so the per-range walk
+// leaves two thirds of the lanes idle and spends 40 % of the instructions on warp-uniform range bookkeeping (profiles/r2d_ncu_gather.md).
+// base = range holding flat index t0; the ranges that start inside (t0, t0 + 32) are among the next 32 (every range is non-empty), each lane
+// looks at one of them: OR of their start bits -> owner of every lane.
+template <class F> __device__ __forceinline__ void phEachFlat(const PhWarpShared& sh, PhRanges R, F&& f) {
+  if (R.total >= 64u * R.n) { phEachRange(sh, R, f); return; }      // long ranges (coarse rows of a sparse map): the per-range walk wastes nothing
+  const unsigned lane = threadIdx.x & 31; uint32_t base = 0;
+  for (uint32_t t0 = 0; t0 < R.total; t0 += 32) {
+    const uint32_t rel = sh.rOff[base + 1 + lane] - t0;                      // >= 1
+    const unsigned mask = __reduce_or_sync(0xffffffffu, rel < 32u ? (1u << rel) : 0u);
+    const uint32_t owner = base + __popc(mask & ((2u << lane) - 1u)), t = t0 + lane;
+    f(sh.rA[owner] + (t - sh.rOff[owner]), t < R.total);
+    base += __popc(__ballot_sync(0xffffffffu, rel <= 32u));
+  }
+}
+// the histogram bin where the running count reaches `target` (1 <= target <= the histogram's total): its index, the count of the bins below it
+// and its own count
+__device__ __forceinline__ void phFindBin(const PhWarpShared& sh, uint32_t target, uint32_t& bin, uint32_t& before, uint32_t& inBin) {
+  const unsigned lane = threadIdx.x & 31;
+  uint32_t loc[8], s = 0;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) { loc[i] = sh.hist[lane * 8 + i]; s += loc[i]; }
+  uint32_t incl = s;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= (unsigned)o) incl += t; }
+  const unsigned reach = __ballot_sync(0xffffffffu, incl >= target); const int L = __ffs(reach) - 1;
+  bin = 0; before = 0; inBin = 0;
+  if ((int)lane == L) { uint32_t c = incl - s; for (int i = 0; i < 8; ++i) { if (c + loc[i] >= target) { bin = lane * 8 + i; before = c; inBin = loc[i]; break; } c += loc[i]; } }
+  bin = __shfl_sync(0xffffffffu, bin, L); before = __shfl_sync(0xffffffffu, before, L); inBin = __shfl_sync(0xffffffffu, inBin, L);
+}
+// exact end of both selections: the `need` smallest (d^2, index) of the boundary list sh.listD2 / listIdx go into the lane's sums
+__device__ __forceinline__ void phRankList(const PhWarpShared& sh, int need, const double4* __restrict__ W, double& s0, double& s1, double& s2, double& mx) {
+  __syncwarp();
+  const int n = (int)min(sh.listN, (uint32_t)DRT_PH_LIST);
+  for (int i = threadIdx.x & 31; i < n; i += 32) {
+    const double di = sh.listD2[i]; const uint32_t ji = sh.listIdx[i]; int rank = 0;
+    for (int t = 0; t < n; ++t) { const double dt = sh.listD2[t]; rank += (dt < di || (dt == di && sh.listIdx[t] < ji)) ? 1 : 0; }
+    if (rank < need) { const double4 w = W[ji]; s0 += w.x; s1 += w.y; s2 += w.z; mx = fmax(mx, di); }
+  }
+}
+__device__ __forceinline__ void phWarpSum(double s0, double s1, double s2, double mx, double sum[3], double& dmax2) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) { s0 += __shfl_xor_sync(0xffffffffu, s0, o); s1 += __shfl_xor_sync(0xffffffffu, s1, o); s2 += __shfl_xor_sync(0xffffffffu, s2, o); mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o)); }
+  sum[0] = s0; sum[1] = s1; sum[2] = s2; dmax2 = mx;
+}
+
+// FP64 selection: radix select on a 32-bit quantisation of d^2 (monotone in d^2), 8 bits per level, each level one walk over the candidates,
+// finished exactly on the boundary bin once it holds <= DRT_PH_LIST photons.  r2: search threshold (the scene's r^2, or a smaller guess --
+// then `needAll`: return false without a result if fewer than k photons are inside it).
+__device__ inline bool phWarpGather64(const DScene& S, D3 p, double r2, bool needAll, PhRanges R, PhWarpShared& sh, double sum[3], double& dmax2) {
+  const unsigned lane = threadIdx.x & 31;
   const double qscale = 4294967295.0 / r2;          // quantised key: monotone non-decreasing in d^2, < 2^32 for d^2 < r^2
   const double4* __restrict__ P = reinterpret_cast<const double4*>(S.phPos); const double4* __restrict__ W = reinterpret_cast<const double4*>(S.phPwr);
-  // visit every candidate; F(j, d2, q, ok) is called warp-wide, ok = d2 < r2.  Two shapes of candidate set:
-  //   coarse (fineHalf < 0): the <= 3x3 rows of coarse cells lo..hi the r-sphere's bounding cube overlaps, one contiguous photon range per row
-  //   fine   (fineHalf >= 0): the block of fine sub-cells lo..hi the plan's search sphere overlaps (see phMakePlan)
-  auto scan = [&](uint32_t a, uint32_t b, auto&& F) {
-    for (uint32_t j0 = a; j0 < b; j0 += 32) {
-      const uint32_t j = j0 + lane; bool ok = j < b; double d2 = 0;
-      if (ok) { const double4 q = P[j]; const double dx = p.x - q.x, dy2 = p.y - q.y, dz2 = p.z - q.z; d2 = dx * dx + dy2 * dy2 + dz2 * dz2; ok = d2 < r2; }
+  // F(j, d2, q, ok) warp-wide for every candidate, ok = d2 < r2.  The per-range walk gives each lane the same photons in the same order on
+  // every level and in the final pass.
+  auto each = [&](auto&& F) {
+    phEachRange(sh, R, [&](uint32_t j, bool ok) {
+      double d2 = 0;
+      if (ok) { const double4 q = P[j]; const double dx = p.x - q.x, dy = p.y - q.y, dz = p.z - q.z; d2 = dx * dx + dy * dy + dz * dz; ok = d2 < r2; }
       F(j, d2, ok ? (uint32_t)(d2 * qscale) : 0u, ok);
-    }
-  };
-  auto forEach = [&](auto&& F) {
-    if (fineHalf < 0) {
-      for (int cz = lo[2]; cz <= hi[2]; ++cz) for (int cy = lo[1]; cy <= hi[1]; ++cy) {
-        const uint32_t row = ((uint32_t)cz * S.gridDim[1] + (uint32_t)cy) * S.gridDim[0];
-        scan(S.cellStart[(size_t)(row + lo[0]) << 6], S.cellStart[(size_t)(row + hi[0] + 1) << 6], F);
-      }
-    } else {
-      const int z0 = lo[2], z1 = hi[2], y0 = lo[1], y1 = hi[1], x0 = lo[0], x1 = hi[0];          // fine-cell bounds of the plan (inclusive, inside the grid)
-      for (int fz = z0; fz <= z1; ++fz) for (int fy = y0; fy <= y1; ++fy) {
-        const uint32_t crow = ((uint32_t)(fz >> 2) * S.gridDim[1] + (uint32_t)(fy >> 2)) * S.gridDim[0], sub = ((uint32_t)(fz & 3) << 4) | ((uint32_t)(fy & 3) << 2);
-        for (int fx = x0; fx <= x1; ) {          // fine cells of one coarse cell that share (fy, fz) are consecutive keys: one range per run
-          const int runEnd = min(x1, fx | 3); const size_t k0 = ((size_t)(crow + (uint32_t)(fx >> 2)) << 6) | sub | (uint32_t)(fx & 3);
-          scan(S.cellStart[k0], S.cellStart[k0 + (size_t)(runEnd - fx) + 1], F);
-          fx = runEnd + 1;
-        }
-      }
-    }
+    });
   };
   // level loop: keys with (q >> shift) < prefix are already known to be inside; those == prefix are undecided
-  uint32_t prefix = 0; int shift = 32; int need = K; bool takeAllUndecided = atMostK, haveList = false;     // atMostK: the candidate cells hold <= k photons, nothing to select
-  while (!atMostK) {
+  uint32_t prefix = 0; int shift = 32; int need = S.g.kNhood; bool takeAllUndecided = false, haveList = false;
+  while (true) {
     const int nshift = shift - 8;
+    __syncwarp();
     for (int i = lane; i < DRT_PH_BINS; i += 32) sh.hist[i] = 0;
     __syncwarp();
-    unsigned m = 0, vis = 0;
-    forEach([&](uint32_t, double, uint32_t q, bool ok) {
+    unsigned m = 0;
+    each([&](uint32_t, double, uint32_t q, bool ok) {
       const bool und = ok && (shift == 32 || (q >> shift) == prefix);
       if (und) atomicAdd(&sh.hist[(q >> nshift) & 255u], 1u);
-      m += __popc(__ballot_sync(0xffffffffu, und)); vis += 32;
+      m += __popc(__ballot_sync(0xffffffffu, und));
     });
-    if (visited && shift == 32 && lane == 0) *visited += vis;
     __syncwarp();
     if (needAll && shift == 32 && (int)m < need) return false;              // the guessed radius holds fewer than k photons: caller retries with the full one
     if ((int)m <= need) { takeAllUndecided = true; break; }                 // fewer undecided candidates than still needed: all of them are in
-    // find the bin where the running count reaches `need`
-    uint32_t loc[8], s = 0;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) { loc[i] = sh.hist[lane * 8 + i]; s += loc[i]; }
-    uint32_t incl = s;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) { uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= (unsigned)o) incl += t; }
-    const unsigned reach = __ballot_sync(0xffffffffu, incl >= (uint32_t)need); const int L = __ffs(reach) - 1;
-    uint32_t binSel = 0, before = 0, inBin = 0;
-    if ((int)lane == L) { uint32_t c = incl - s; for (int i = 0; i < 8; ++i) { if (c + loc[i] >= (uint32_t)need) { binSel = lane * 8 + i; before = c; inBin = loc[i]; break; } c += loc[i]; } }
-    binSel = __shfl_sync(0xffffffffu, binSel, L); before = __shfl_sync(0xffffffffu, before, L); inBin = __shfl_sync(0xffffffffu, inBin, L);
+    uint32_t binSel, before, inBin; phFindBin(sh, (uint32_t)need, binSel, before, inBin);
     need -= (int)before; prefix = (shift == 32) ? binSel : ((prefix << 8) | binSel); shift = nshift;
     if (inBin <= DRT_PH_LIST) { haveList = true; break; }
     if (shift == 0) break;                                                    // > DRT_PH_LIST photons with identical 32-bit distance keys: take by index order below
@@ -291,7 +353,7 @@ __device__ inline bool phWarpGather(const DScene& S, D3 p, double r2, bool needA
   if (lane == 0) sh.listN = 0;
   __syncwarp();
   double s0 = 0, s1 = 0, s2 = 0, mx = 0; int tieTaken = 0;
-  forEach([&](uint32_t j, double d2, uint32_t q, bool ok) {
+  each([&](uint32_t j, double d2, uint32_t q, bool ok) {
     bool in = false, bnd = false;
     if (ok) {
       if (takeAllUndecided) in = (shift == 32) || ((q >> shift) <= prefix);
@@ -309,36 +371,24 @@ __device__ inline bool phWarpGather(const DScene& S, D3 p, double r2, bool needA
     }
     if (in) { const double4 w = W[j]; s0 += w.x; s1 += w.y; s2 += w.z; mx = fmax(mx, d2); }
   });
-  if (haveList) {   // exact selection of the `need` smallest (d2, index) of the boundary list
-    __syncwarp();
-    const int n = (int)min(sh.listN, (uint32_t)DRT_PH_LIST);
-    for (int i = lane; i < n; i += 32) {
-      const double di = sh.listD2[i]; const uint32_t ji = sh.listIdx[i]; int rank = 0;
-      for (int t = 0; t < n; ++t) { const double dt = sh.listD2[t]; rank += (dt < di || (dt == di && sh.listIdx[t] < ji)) ? 1 : 0; }
-      if (rank < need) { const double4 w = W[ji]; s0 += w.x; s1 += w.y; s2 += w.z; mx = fmax(mx, di); }
-    }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) { s0 += __shfl_xor_sync(0xffffffffu, s0, o); s1 += __shfl_xor_sync(0xffffffffu, s1, o); s2 += __shfl_xor_sync(0xffffffffu, s2, o); mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o)); }
-  sum[0] = s0; sum[1] = s1; sum[2] = s2; dmax2 = mx;
+  if (haveList) phRankList(sh, need, W, s0, s1, s2, mx);
+  phWarpSum(s0, s1, s2, mx, sum, dmax2);
   return true;
 }
 
-// FP32 pre-test form of phWarpGather: the same exact result from ONE histogram pass and one collection pass, both in FP32.
-// The FP64 selection above re-reads every candidate's 32-byte position and re-forms d^2 in FP64 for every radix level (2-3 scans of ~11 FP64-pipe
+// FP32 pre-test selection: the same exact result from ONE histogram pass and one collection pass, both in FP32.
+// The FP64 selection re-reads every candidate's 32-byte position and re-forms d^2 in FP64 for every radix level (2-3 walks of ~11 FP64-pipe
 // operations per candidate: the half-rate FP64 pipe is what bounds dense maps).  Here d^2 is formed in FP32 from a float4 mirror of the positions;
 // with u = 2^-24, A = largest |coordinate| of a photon and rho = sqrt(r2),
 //     |d2_32 - d2| <= delta = 2 sqrt(3) rho e + 3 e^2 + 4 u r2,     e = u (|p|_inf + A + rho)        (coordinate rounding + one rounding per operation)
 // for every candidate with d2 <= r2.  256 bins of width w = r2/256 over the FP32 values; the method is used only if 4 delta < w.  Then, with b the
 // bin where the running count reaches k: every candidate binned <= b-2 is among the k nearest (the k-th true distance is >= edge(b) - delta),
 // every candidate binned >= b+2 is not, and the <= 128 candidates of bins b-1..b+1 are resolved exactly -- FP64 d^2 from the FP64 positions,
-// (d^2, index) order -- exactly as the boundary list of phWarpGather.  The k-th neighbour itself is always in that list, so the d^2 that leaves the
-// function is the FP64 value.  Candidates within delta of the radius are classified by their FP64 d^2.  Returns 1 (done), 0 (needAll and fewer
-// than k photons inside r2) or -1 (margin too wide, or a boundary list longer than 128: the caller runs phWarpGather).
-__device__ inline int phWarpGather32(const DScene& S, D3 p, double r2, bool needAll, int fineHalf, const int lo[3], const int hi[3], PhWarpShared& sh, double sum[3], double& dmax2) {
+// (d^2, index) order -- by the same boundary-list ranking as the FP64 selection.  The k-th neighbour itself is always in that list, so the d^2
+// that leaves the function is the FP64 value.  Candidates within delta of the radius are classified by their FP64 d^2.  Returns 1 (done), 0
+// (needAll and fewer than k photons inside r2) or -1 (margin too wide, or a boundary list longer than 128: the FP64 selection decides).
+__device__ inline int phWarpGather32(const DScene& S, D3 p, double r2, bool needAll, PhRanges R, PhWarpShared& sh, double sum[3], double& dmax2) {
   const unsigned lane = threadIdx.x & 31; const int K = S.g.kNhood;
-  sum[0] = sum[1] = sum[2] = 0; dmax2 = 0;
-  if (S.numPhotons == 0 || K <= 0) return 1;
   const float u = 5.9604644775390625e-8f, rho = __double2float_ru(sqrt(r2)), r2f = __double2float_ru(r2);
   const float pm = fmaxf(fmaxf(fabsf(__double2float_ru(fabs(p.x))), fabsf(__double2float_ru(fabs(p.y)))), fabsf(__double2float_ru(fabs(p.z))));
   const float e = 1.01f * u * (pm + S.phAbsMax + rho), delta = 1.05f * (3.4641016f * rho * e + 3.0f * e * e + 4.0f * u * r2f);
@@ -357,80 +407,20 @@ __device__ inline int phWarpGather32(const DScene& S, D3 p, double r2, bool need
   for (int i = lane; i < DRT_PH_BINS; i += 32) sh.hist[i] = 0;
   if (lane == 0) sh.listN = 0;
   __syncwarp();
-  // ---- the candidate ranges, enumerated lane-parallel and compacted (empty ones dropped) into shared memory with the running offset of each:
-  // a fine row run holds ~10-30 photons, so looping "per range, 32 lanes over its photons" left two thirds of the lanes idle and spent 40 % of
-  // the instructions on warp-uniform range bookkeeping (profiles/r2d_ncu_gather.md).  The two passes below walk the FLAT candidate index instead.
-  uint32_t nRanges = 0, total = 0;
-  {
-    const int x0 = lo[0], x1 = hi[0], y0 = lo[1], y1 = hi[1], z0 = lo[2], z1 = hi[2], nx = fineHalf < 0 ? 1 : (x1 >> 2) - (x0 >> 2) + 1;     // coarse rows, or runs of fine cells
-    const int ny = y1 - y0 + 1, nz = z1 - z0 + 1, slots = nx * ny * nz;
-    if (slots > DRT_PH_MAXRANGES || slots <= 0) return -1;
-    for (int s0 = 0; s0 < slots; s0 += 32) {
-      const int slot = s0 + (int)lane; uint32_t a = 0, len = 0;
-      if (slot < slots) {
-        const int ir = slot % nx, iy = (slot / nx) % ny, iz = slot / (nx * ny); const int fy = y0 + iy, fz = z0 + iz;
-        if (fineHalf < 0) { const uint32_t row = ((uint32_t)fz * S.gridDim[1] + (uint32_t)fy) * S.gridDim[0]; a = S.cellStart[(size_t)(row + x0) << 6]; len = S.cellStart[(size_t)(row + x1 + 1) << 6] - a; }
-        else {
-          const int fx = ir == 0 ? x0 : (((x0 >> 2) + ir) << 2), runEnd = min(x1, fx | 3);
-          const uint32_t crow = ((uint32_t)(fz >> 2) * S.gridDim[1] + (uint32_t)(fy >> 2)) * S.gridDim[0], sub = ((uint32_t)(fz & 3) << 4) | ((uint32_t)(fy & 3) << 2);
-          const size_t k0 = ((size_t)(crow + (uint32_t)(fx >> 2)) << 6) | sub | (uint32_t)(fx & 3);
-          a = S.cellStart[k0]; len = S.cellStart[k0 + (size_t)(runEnd - fx) + 1] - a;
-        }
-      }
-      const unsigned ne = __ballot_sync(0xffffffffu, len > 0);
-      uint32_t incl = len;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= (unsigned)o) incl += t; }
-      if (len > 0) { const uint32_t at = nRanges + __popc(ne & ((1u << lane) - 1u)); sh.rA[at] = a; sh.rOff[at] = total + incl - len; }
-      nRanges += __popc(ne); total += __shfl_sync(0xffffffffu, incl, 31);
-    }
-    for (uint32_t i = nRanges + lane; i < nRanges + 33; i += 32) { sh.rA[i] = 0; sh.rOff[i] = 0xFFFFFFFFu; }       // sentinels: "starts beyond everything"
-  }
-  __syncwarp();
-  // F(j, valid) for every candidate, 32 consecutive flat indices per step.  base = range holding flat index t0; the ranges that start inside
-  // (t0, t0 + 32) are among the next 32 (every range is non-empty), each lane looks at one of them: OR of their start bits -> owner of every lane.
-  auto flat = [&](auto&& F) {
-    if (total >= 64u * nRanges) {            // long ranges (coarse rows of a sparse map): the plain per-range loop wastes nothing and needs no search
-      for (uint32_t r = 0; r < nRanges; ++r) { const uint32_t a = sh.rA[r], b = a + (sh.rOff[r + 1] == 0xFFFFFFFFu ? total - sh.rOff[r] : sh.rOff[r + 1] - sh.rOff[r]);
-        for (uint32_t j0 = a; j0 < b; j0 += 32) F(j0 + lane, j0 + lane < b); }
-      return;
-    }
-    uint32_t base = 0;
-    for (uint32_t t0 = 0; t0 < total; t0 += 32) {
-      const uint32_t rel = sh.rOff[base + 1 + lane] - t0;                      // >= 1
-      const unsigned mask = __reduce_or_sync(0xffffffffu, rel < 32u ? (1u << rel) : 0u);
-      const uint32_t owner = base + __popc(mask & ((2u << lane) - 1u)), t = t0 + lane;
-      F(sh.rA[owner] + (t - sh.rOff[owner]), t < total);
-      base += __popc(__ballot_sync(0xffffffffu, rel <= 32u));
-    }
-  };
   unsigned m = 0;
-  flat([&](uint32_t j, bool valid) { const int bin = valid ? binOf(j) : -1; if (bin >= 0) atomicAdd(&sh.hist[bin], 1u); m += __popc(__ballot_sync(0xffffffffu, bin >= 0)); });
+  phEachFlat(sh, R, [&](uint32_t j, bool valid) { const int bin = valid ? binOf(j) : -1; if (bin >= 0) atomicAdd(&sh.hist[bin], 1u); m += __popc(__ballot_sync(0xffffffffu, bin >= 0)); });
   __syncwarp();
   if (needAll && (int)m < K) return 0;
   if (m == 0) return 1;
   // boundary bin b: running count reaches k (m > k), or the highest non-empty bin (m <= k: every photon inside r2 is taken)
-  uint32_t loc[8], s = 0;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) { loc[i] = sh.hist[lane * 8 + i]; s += loc[i]; }
-  uint32_t incl = s;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) { const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= (unsigned)o) incl += t; }
   const uint32_t target = (int)m > K ? (uint32_t)K : m;
-  const unsigned reach = __ballot_sync(0xffffffffu, incl >= target); const int L = __ffs(reach) - 1;
-  int bSel = 0;
-  if ((int)lane == L) { uint32_t c = incl - s; for (int i = 0; i < 8; ++i) { if (c + loc[i] >= target) { bSel = (int)lane * 8 + i; break; } c += loc[i]; } }
-  bSel = __shfl_sync(0xffffffffu, bSel, L);
-  const int bLo = bSel - 1, bHi = bSel + 1;                  // exact zone; bins < bLo are in, bins > bHi are out
-  uint32_t below = 0, zone = 0;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) { const int bin = (int)lane * 8 + i; if (bin < bLo) below += loc[i]; else if (bin <= bHi) zone += loc[i]; }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) { below += __shfl_xor_sync(0xffffffffu, below, o); zone += __shfl_xor_sync(0xffffffffu, zone, o); }
-  if (zone > DRT_PH_LIST) return -1;
-  const int need = (int)target - (int)below;                 // >= 1: the running count through bin b-1 is below the target
+  uint32_t bSel, before, inBin; phFindBin(sh, target, bSel, before, inBin);
+  const uint32_t prev = bSel > 0 ? sh.hist[bSel - 1] : 0u, next = bSel < DRT_PH_BINS - 1 ? sh.hist[bSel + 1] : 0u;
+  if (prev + inBin + next > DRT_PH_LIST) return -1;
+  const int bLo = (int)bSel - 1, bHi = (int)bSel + 1;        // exact zone; bins < bLo are in, bins > bHi are out
+  const int need = (int)target - (int)(before - prev);       // >= 1: the running count through bin b-1 is below the target
   double s0 = 0, s1 = 0, s2 = 0, mx = 0;
-  flat([&](uint32_t j, bool valid) {
+  phEachFlat(sh, R, [&](uint32_t j, bool valid) {
     const int bin = valid ? binOf(j) : -1;
     if (bin >= 0 && bin < bLo) { const double4 w = W[j]; s0 += w.x; s1 += w.y; s2 += w.z; }
     const bool bnd = bin >= bLo && bin <= bHi; const unsigned bm = __ballot_sync(0xffffffffu, bnd);
@@ -441,26 +431,25 @@ __device__ inline int phWarpGather32(const DScene& S, D3 p, double r2, bool need
       __syncwarp();
     }
   });
-  __syncwarp();
-  const int n = (int)sh.listN;
-  for (int i = lane; i < n; i += 32) {
-    const double di = sh.listD2[i]; const uint32_t ji = sh.listIdx[i]; int rank = 0;
-    for (int t = 0; t < n; ++t) { const double dt = sh.listD2[t]; rank += (dt < di || (dt == di && sh.listIdx[t] < ji)) ? 1 : 0; }
-    if (rank < need) { const double4 w = W[ji]; s0 += w.x; s1 += w.y; s2 += w.z; mx = fmax(mx, di); }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) { s0 += __shfl_xor_sync(0xffffffffu, s0, o); s1 += __shfl_xor_sync(0xffffffffu, s1, o); s2 += __shfl_xor_sync(0xffffffffu, s2, o); mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o)); }
-  __syncwarp();
-  sum[0] = s0; sum[1] = s1; sum[2] = s2; dmax2 = mx;
+  phRankList(sh, need, W, s0, s1, s2, mx);
+  phWarpSum(s0, s1, s2, mx, sum, dmax2);
   return 1;
+}
+
+// One search of the warp tier over the cells lo..hi (coarse rows, or the fine cells of a plan): one candidate list, the FP32 selection, and
+// the FP64 one when the FP32 one cannot decide.  False when `needAll` and fewer than k photons lie inside r2.
+__device__ inline bool phWarpGather(const DScene& S, D3 p, double r2, bool needAll, bool fine, const int lo[3], const int hi[3], PhWarpShared& sh, double sum[3], double& dmax2) {
+  sum[0] = sum[1] = sum[2] = 0; dmax2 = 0;
+  const PhRanges R = phWarpRanges(S, fine, lo, hi, sh);
+  const int g = phWarpGather32(S, p, r2, needAll, R, sh, sum, dmax2);
+  return g < 0 ? phWarpGather64(S, p, r2, needAll, R, sh, sum, dmax2) : g > 0;
 }
 
 // cheap per-lane test: does any cell the search sphere's bounding cube overlaps hold a photon at all?  (sparse caustic maps: most queries do not)
 __device__ inline uint32_t phCountCandidates(const DScene& S, const int lo[3], const int hi[3]) {
   uint32_t c = 0;
   for (int cz = lo[2]; cz <= hi[2]; ++cz) for (int cy = lo[1]; cy <= hi[1]; ++cy) {
-    const uint32_t row = ((uint32_t)cz * S.gridDim[1] + (uint32_t)cy) * S.gridDim[0];
-    c += S.cellStart[(size_t)(row + hi[0] + 1) << 6] - S.cellStart[(size_t)(row + lo[0]) << 6];
+    uint32_t a, b; phRowRange(S, false, cy, cz, lo[0], hi[0], a, b); c += b - a;
   }
   return c;
 }
@@ -474,11 +463,8 @@ __device__ __forceinline__ uint32_t phCountFineCube(const DScene& S, const int f
   const int fdx = 4 * (int)S.gridDim[0], fdy = 4 * (int)S.gridDim[1], fdz = 4 * (int)S.gridDim[2];
   const int z0 = max(f[2] - s, 0), z1 = min(f[2] + s, fdz - 1), y0 = max(f[1] - s, 0), y1 = min(f[1] + s, fdy - 1), x0 = max(f[0] - s, 0), x1 = min(f[0] + s, fdx - 1);
   uint32_t c = 0;
-  for (int fz = z0; fz <= z1; ++fz) for (int fy = y0; fy <= y1; ++fy) {
-    const uint32_t crow = ((uint32_t)(fz >> 2) * S.gridDim[1] + (uint32_t)(fy >> 2)) * S.gridDim[0], sub = ((uint32_t)(fz & 3) << 4) | ((uint32_t)(fy & 3) << 2);
-    for (int fx = x0; fx <= x1; ) { const int runEnd = min(x1, fx | 3); const size_t k0 = ((size_t)(crow + (uint32_t)(fx >> 2)) << 6) | sub | (uint32_t)(fx & 3);
-      c += S.cellStart[k0 + (size_t)(runEnd - fx) + 1] - S.cellStart[k0]; fx = runEnd + 1; }
-  }
+  for (int fz = z0; fz <= z1; ++fz) for (int fy = y0; fy <= y1; ++fy)
+    for (int fx = x0; fx <= x1; ) { const int runEnd = min(x1, fx | 3); uint32_t a, b; phRowRange(S, true, fy, fz, fx, runEnd, a, b); c += b - a; fx = runEnd + 1; }
   return c;
 }
 // The plan: a search radius rho <= s fine cells (s = 1, 2, 3) and the block of fine cells its sphere's bounding cube overlaps.  s = the first
@@ -502,9 +488,6 @@ __device__ __forceinline__ void phMakePlan(const DScene& S, D3 p, uint32_t coars
     const double inSphere = (double)phCountFineCube(S, f, s) * frac[s];
     if (inSphere >= 1.25 * K) {
       double rad = radMax * sqrt(1.5 * K / inSphere); if (!(rad < radMax)) rad = radMax;
-#if !DRT_PH_TIGHT
-      rad = radMax;
-#endif
       const double reach = rad * (1.0 + 1e-6) + 1e-9 * cf;                     // cells the sphere can touch, with room for the rounding of a photon's own cell index
       pl.fineHalf = s; pl.r2 = rad * rad; pl.r2max = radMax * radMax; pl.shrunk = rad < radMax;
       for (int k = 0; k < 3; ++k) { const int fd = 4 * (int)S.gridDim[k]; const int a = (int)floor((pp[k] - reach - S.gridMin[k]) / cf), b = (int)floor((pp[k] + reach - S.gridMin[k]) / cf);
@@ -520,11 +503,6 @@ __device__ __forceinline__ void phMakePlan(const DScene& S, D3 p, uint32_t coars
 // Results per lane: sum of the k nearest powers and d^2 of the farthest (0 = no photon in range). `path` (optional) reports the tier taken.
 struct PhLaneShared { uint16_t laneHist[128 * 128]; };      // lane-private 128-bin histograms laid out [bin][thread]
 struct PhWarpTierShared { PhWarpShared warp[4]; };
-
-__device__ __forceinline__ void phLaneRows(const DScene& S, const int lo[3], const int hi[3], int cz, int cy, uint32_t& a, uint32_t& b) {
-  const uint32_t row = ((uint32_t)cz * S.gridDim[1] + (uint32_t)cy) * S.gridDim[0];
-  a = S.cellStart[(size_t)(row + lo[0]) << 6]; b = S.cellStart[(size_t)(row + hi[0] + 1) << 6];
-}
 // tiers 1 and 2; returns true when the query is left for the warp-cooperative tier
 __device__ inline bool phLaneTiers(const DScene& S, bool needs, D3 loc, PhLaneShared& sm, double sum[3], double& dmax2, int* path) {
   const double r2 = S.g.phMaxDist2; const int K = S.g.kNhood;
@@ -537,7 +515,7 @@ __device__ inline bool phLaneTiers(const DScene& S, bool needs, D3 loc, PhLaneSh
     if (needs && few) {                                                    // tier 1. Sum order = photon order in the sorted array
       double s0 = 0, s1 = 0, s2 = 0, mx = 0;
       for (int cz = lo[2]; cz <= hi[2]; ++cz) for (int cy = lo[1]; cy <= hi[1]; ++cy) {
-        uint32_t a, b; phLaneRows(S, lo, hi, cz, cy, a, b);
+        uint32_t a, b; phRowRange(S, false, cy, cz, lo[0], hi[0], a, b);
         for (uint32_t j = a; j < b; ++j) { const double4 q = P[j]; const double dx = loc.x - q.x, dy = loc.y - q.y, dz = loc.z - q.z, d2 = dx * dx + dy * dy + dz * dz;
           if (d2 < r2) { const double4 w = W[j]; s0 += w.x; s1 += w.y; s2 += w.z; mx = fmax(mx, d2); } }
       }
@@ -551,7 +529,7 @@ __device__ inline bool phLaneTiers(const DScene& S, bool needs, D3 loc, PhLaneSh
       for (int b = 0; b < 128; ++b) h[b * 128] = 0;
       int m = 0;
       for (int cz = lo[2]; cz <= hi[2]; ++cz) for (int cy = lo[1]; cy <= hi[1]; ++cy) {
-        uint32_t a, b; phLaneRows(S, lo, hi, cz, cy, a, b);
+        uint32_t a, b; phRowRange(S, false, cy, cz, lo[0], hi[0], a, b);
         for (uint32_t j = a; j < b; ++j) { const double4 q = P[j]; const double dx = loc.x - q.x, dy = loc.y - q.y, dz = loc.z - q.z, d2 = dx * dx + dy * dy + dz * dz;
           if (d2 < r2) { ++m; ++h[(int)(d2 * bscale) * 128]; } }
       }
@@ -562,7 +540,7 @@ __device__ inline bool phLaneTiers(const DScene& S, bool needs, D3 loc, PhLaneSh
         const int need = K - below;                                       // photons to take from the boundary bin (m > K only)
         double s0 = 0, s1 = 0, s2 = 0, mx = 0, ld[8]; uint32_t lj[8]; int ln = 0; bool overflow = false;
         for (int cz = lo[2]; cz <= hi[2]; ++cz) for (int cy = lo[1]; cy <= hi[1]; ++cy) {
-          uint32_t a, b; phLaneRows(S, lo, hi, cz, cy, a, b);
+          uint32_t a, b; phRowRange(S, false, cy, cz, lo[0], hi[0], a, b);
           for (uint32_t j = a; j < b; ++j) { const double4 q = P[j]; const double dx = loc.x - q.x, dy = loc.y - q.y, dz = loc.z - q.z, d2 = dx * dx + dy * dy + dz * dz;
             if (d2 < r2) { const int bin = (int)(d2 * bscale);
               if (bin < bsel) { const double4 w = W[j]; s0 += w.x; s1 += w.y; s2 += w.z; mx = fmax(mx, d2); }
@@ -582,9 +560,10 @@ __device__ inline bool phLaneTiers(const DScene& S, bool needs, D3 loc, PhLaneSh
 // tier 3 / 4: the warp serves its pending queries one at a time
 __device__ inline void phWarpTier(const DScene& S, bool pending, D3 loc, PhWarpTierShared& sm, double sum[3], double& dmax2, int* path) {
   const unsigned lane = threadIdx.x & 31; const double r2 = S.g.phMaxDist2; const int K = S.g.kNhood;
-  bool few = false; int lo[3] = {0, 0, 0}, hi[3] = {0, 0, 0}; PhPlan pl; pl.fineHalf = -1; pl.r2 = r2; pl.r2max = r2; pl.shrunk = false; for (int k = 0; k < 3; ++k) pl.c[k] = pl.h[k] = pl.f[k] = 0;
+  int lo[3] = {0, 0, 0}, hi[3] = {0, 0, 0}; PhPlan pl; pl.fineHalf = -1; pl.r2 = r2; pl.r2max = r2; pl.shrunk = false; for (int k = 0; k < 3; ++k) pl.c[k] = pl.h[k] = pl.f[k] = 0;
   bool needs = pending && S.numPhotons > 0 && K > 0;
-  if (needs) { needs = phCellRange(S, loc, r2, lo, hi); const uint32_t cnt = needs ? phCountCandidates(S, lo, hi) : 0u; needs = cnt > 0; few = cnt <= (uint32_t)K; if (needs) phMakePlan(S, loc, cnt, lo, hi, pl); }
+  if (needs) { needs = phCellRange(S, loc, r2, lo, hi); const uint32_t cnt = needs ? phCountCandidates(S, lo, hi) : 0u; needs = cnt > 0; if (needs) phMakePlan(S, loc, cnt, lo, hi, pl); }
+  PhWarpShared& sh = sm.warp[threadIdx.x >> 5];
   unsigned mask = __ballot_sync(0xffffffffu, needs);
   while (mask) {
     const int src = __ffs(mask) - 1; mask &= mask - 1;
@@ -595,21 +574,18 @@ __device__ inline void phWarpTier(const DScene& S, bool pending, D3 loc, PhWarpT
       const double pr2 = __shfl_sync(0xffffffffu, pl.r2, src);
 #pragma unroll
       for (int k = 0; k < 3; ++k) { qlo[k] = __shfl_sync(0xffffffffu, pl.c[k], src); qhi[k] = __shfl_sync(0xffffffffu, pl.h[k], src); }
-      const int g32 = DRT_PH_FP32 ? phWarpGather32(S, p, pr2, true, fineHalf, qlo, qhi, sm.warp[threadIdx.x >> 5], qs, qd) : -1;
-      done = g32 > 0 || (g32 < 0 && phWarpGather(S, p, pr2, true, false, fineHalf, qlo, qhi, sm.warp[threadIdx.x >> 5], qs, qd, nullptr));
+      done = phWarpGather(S, p, pr2, true, true, qlo, qhi, sh, qs, qd);
       if (!done && __shfl_sync(0xffffffffu, (int)pl.shrunk, src) != 0) {      // fewer than k photons inside the shrunk radius: the plan's full radius over its whole cube, before the coarse rows
         const double pr2m = __shfl_sync(0xffffffffu, pl.r2max, src);
 #pragma unroll
         for (int k = 0; k < 3; ++k) { const int fk = __shfl_sync(0xffffffffu, pl.f[k], src); qlo[k] = max(fk - fineHalf, 0); qhi[k] = min(fk + fineHalf, 4 * (int)S.gridDim[k] - 1); }
-        const int g2 = DRT_PH_FP32 ? phWarpGather32(S, p, pr2m, true, fineHalf, qlo, qhi, sm.warp[threadIdx.x >> 5], qs, qd) : -1;
-        done = g2 > 0 || (g2 < 0 && phWarpGather(S, p, pr2m, true, false, fineHalf, qlo, qhi, sm.warp[threadIdx.x >> 5], qs, qd, nullptr));
+        done = phWarpGather(S, p, pr2m, true, true, qlo, qhi, sh, qs, qd);
       }
     }
     if (!done) {
 #pragma unroll
       for (int k = 0; k < 3; ++k) { qlo[k] = __shfl_sync(0xffffffffu, lo[k], src); qhi[k] = __shfl_sync(0xffffffffu, hi[k], src); }
-      const int g32 = DRT_PH_FP32 ? phWarpGather32(S, p, r2, false, -1, qlo, qhi, sm.warp[threadIdx.x >> 5], qs, qd) : -1;
-      if (g32 < 0) phWarpGather(S, p, r2, false, __shfl_sync(0xffffffffu, (int)few, src) != 0, -1, qlo, qhi, sm.warp[threadIdx.x >> 5], qs, qd, nullptr);
+      phWarpGather(S, p, r2, false, false, qlo, qhi, sh, qs, qd);
     }
     if ((int)lane == src) { sum[0] = qs[0]; sum[1] = qs[1]; sum[2] = qs[2]; dmax2 = qd; if (path) *path = done ? 4 : 3; }
     __syncwarp();
@@ -617,7 +593,7 @@ __device__ inline void phWarpTier(const DScene& S, bool pending, D3 loc, PhWarpT
 }
 
 // Run between k_shade (local = ambient) and k_light (local += direct), which is the reference's accumulation order (myObjShader.java:413-425).
-// Two kernels so that the warp-cooperative tier keeps its occupancy (64 registers, 10 KB shared) and the lane tiers their histogram space:
+// Two kernels so that the warp-cooperative tier keeps its occupancy (96 registers, 16 KB shared) and the lane tiers their histogram space:
 // k_photon_gather_lane resolves tiers 1-2 and marks what is left in SurfRec::pad, k_photon_gather_warp serves the marked queries.
 __device__ __forceinline__ void phApply(const DScene& S, int shIdx, const double sum[3], double dmax2, double* l) {
   if (!(dmax2 > 0)) return;

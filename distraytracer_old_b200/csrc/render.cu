@@ -21,9 +21,10 @@ namespace drt {
 #define CK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e_) + " at " #x); } while (0)
 
 static void devErrorReset(cudaStream_t st) { const unsigned int z = 0; CK(cudaMemcpyToSymbolAsync(g_devError, &z, sizeof(z), 0, cudaMemcpyHostToDevice, st)); }
+static const char* const kDevIncomplete = "device search beyond its capacity (traversal stack overflow, or a photon query with more candidate ranges than the gather holds): the result would be incomplete";
 static void devErrorCheck(cudaStream_t st) {
   unsigned int e = 0; CK(cudaMemcpyFromSymbolAsync(&e, g_devError, sizeof(e), 0, cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st));
-  if (e & 1u) throw std::runtime_error("traversal stack overflow on the device (acceleration structure deeper than the kernels support): the result would be incomplete");
+  if (e & 1u) throw std::runtime_error(kDevIncomplete);
 }
 
 struct alignas(16) RayRec { double o[3], d[3]; double kt0, kt1; uint32_t ka, kb, kc, stream; int32_t gen, valid; int32_t pad[2]; };
@@ -726,7 +727,7 @@ void Renderer::renderChunks(long long pix0, long long pix1, int world, int rank,
     CK(cudaMemcpyAsync(I.ctrHost, I.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, st));
     unsigned int devErr = 0; CK(cudaMemcpyFromSymbolAsync(&devErr, g_devError, sizeof(devErr), 0, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st)); CK(cudaGetLastError()); ++rs.hostSyncs;
-    if (devErr & 1u) throw std::runtime_error("traversal stack overflow on the device (acceleration structure deeper than the kernels support): the result would be incomplete");
+    if (devErr & 1u) throw std::runtime_error(kDevIncomplete);
     if (devErr & 4u) { if (levels >= fullDepth) throw std::runtime_error("internal error: bounce depth beyond numRays"); levels = fullDepth; ++retries; continue; }
     if (devErr & 2u) { if (capFactor >= 64.0) throw std::runtime_error("internal error: secondary-ray queues overflow at their upper bound"); capFactor = std::min(64.0, capFactor * 2); if (capFactor > 2.0) batchRays = std::max<long long>(65536, batchRays / 2); ++retries; continue; }
     float msT = 0, msS = 0, msL = 0, tot = 0;
@@ -797,12 +798,13 @@ void Renderer::buildPhotonsFromDevice(const double* src6Dev, long long n, Render
 }
 void Renderer::probePhotons(long long n, const double* ptsHost, double* out5Host) {
   CK(cudaSetDevice(device_)); Impl& I = *impl_; cudaStream_t st = (cudaStream_t)stream_;
+  devErrorReset(st);
   if (g_.photonKind != 0 && !I.photons.built) I.photons.emitAndBuild(I.ds, I.ctr, I.ctrHost, st);
   double *a, *b; CK(cudaMalloc(&a, n * 24)); CK(cudaMalloc(&b, n * 40));
   CK(cudaMemcpyAsync(a, ptsHost, n * 24, cudaMemcpyHostToDevice, st)); CK(cudaMemsetAsync(b, 0, n * 40, st));
   if (I.ds.numPhotons > 0) k_photon_probe<<<gridFor(n, 128), 128, 0, st>>>(I.ds, n, a, b);
   CK(cudaMemcpyAsync(out5Host, b, n * 40, cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st)); CK(cudaGetLastError());
-  cudaFree(a); cudaFree(b);
+  cudaFree(a); cudaFree(b); devErrorCheck(st);
 }
 // parity probe: the resident packed triangles of fast BVH `fastIndex` and, in DRT_ACCEL_LBVH mode, its GPU-built nodes
 long long Renderer::probeFastBvh(int fastIndex, std::vector<FTri>& tris, std::vector<FNode>& nodes, int32_t info[4]) {
