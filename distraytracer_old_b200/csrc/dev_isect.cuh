@@ -38,8 +38,12 @@ __device__ __forceinline__ void hitReset(Hit& h) { h.t = DRT_DMAX; h.prim = -1; 
 
 struct TraceCounters { unsigned long long box, prim; };
 
-// device-side error word, checked by the host after every render / trace / photon call (bit 0: a traversal stack overflowed -- the result
-// would silently miss geometry, so the call fails instead)
+// device-side error word, reset and checked by the host around every render / probe / photon call:
+//   DEV_ERR_INCOMPLETE  a search ran beyond its capacity (traversal stack, photon candidate ranges): the result would silently miss
+//                       something, so the call fails instead
+//   DEV_ERR_QUEUE       a bounce level overflowed its queue or the node pool: the host renders the frame again with smaller batches
+//   DEV_ERR_DEPTH       rays reached a level the call did not launch: the host renders the frame again with full depth
+constexpr unsigned int DEV_ERR_INCOMPLETE = 1u, DEV_ERR_QUEUE = 2u, DEV_ERR_DEPTH = 4u;
 __device__ unsigned int g_devError;
 __device__ __forceinline__ void flagError(unsigned int bit) { if (!(g_devError & bit)) atomicOr(&g_devError, bit); }
 
@@ -617,7 +621,7 @@ __device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int i
       const Ray r = sameXf ? trans : xfRay(_ray, S.xforms[B.triXform].inv);
       if constexpr (F == TF_ALL) {
         const int got = leanClosest32<DRT_FSTACK, true>(S, B, trans.o, trans.a, inv, r.o, r.d, _ray.d, out, bound, leanScale(len2), tc);
-        if (got < 0) { flagError(1u); return 0; }
+        if (got < 0) { flagError(DEV_ERR_INCOMPLETE); return 0; }
         return got;
       } else {
         // the lean kernels defer axis-parallel rays.  One instantiation per lean kernel (one traversal stack in its frame): scenes with instanced
@@ -651,7 +655,7 @@ __device__ __forceinline__ int accelClosestImpl(const DScene& S, int kind, int i
     } else {
       const FNode& N = S.nodes[node];
       if (tc) ++tc->box;
-      if (sp >= DRT_STACK) flagError(1u);
+      if (sp >= DRT_STACK) flagError(DEV_ERR_INCOMPLETE);
       if (boxHit(N.lmin, N.lmax, trans, inv) && sp < DRT_STACK) { stack[sp].node = node; stack[sp].tL = 0; ++sp; node = N.left; tCur = DRT_DMAX; continue; }
       tCur = DRT_DMAX; afterLeftOf = node;
     }
@@ -805,7 +809,7 @@ __device__ __forceinline__ int instTreeShadow(const DScene& S, const FBvh& B, Ra
         } else {
           const FNode& N = S.nodes[node];
           const bool hl = boxAcceptShadow(N.lmin, N.lmax, trans, inv, dist), hr = boxAcceptShadow(N.rmin, N.rmax, trans, inv, dist);
-          if (hl) { if (hr) { if (sp < DRT_STACK) stack[sp++] = N.right; else flagError(1u); } node = N.left; }
+          if (hl) { if (hr) { if (sp < DRT_STACK) stack[sp++] = N.right; else flagError(DEV_ERR_INCOMPLETE); } node = N.left; }
           else if (hr) node = N.right;
           else mode = M_POP;
         }
@@ -857,7 +861,7 @@ __device__ __forceinline__ int accelShadowImpl(const DScene& S, int kind, int id
     const Ray r = sameXf ? trans : xfRay(_ray, S.xforms[B.triXform].inv);
     if constexpr (F == TF_ALL) {
       const int got = leanShadow32<DRT_FSTACK, true>(S, B, trans.o, trans.a, inv, r.o, r.d, dist, tc);
-      if (got < 0) { flagError(1u); return 0; }
+      if (got < 0) { flagError(DEV_ERR_INCOMPLETE); return 0; }
       return got;
     } else {
       const bool one = sameXf || sameRay(trans, r);
@@ -879,7 +883,7 @@ __device__ __forceinline__ int accelShadowImpl(const DScene& S, int kind, int id
       if (tc) tc->box += 2;
       bool hl = boxAcceptShadow(N.lmin, N.lmax, trans, inv, dist);
       bool hr = boxAcceptShadow(N.rmin, N.rmax, trans, inv, dist);
-      if (hl) { if (hr) { if (sp < DRT_STACK) stack[sp++] = N.right; else flagError(1u); } node = N.left; continue; }
+      if (hl) { if (hr) { if (sp < DRT_STACK) stack[sp++] = N.right; else flagError(DEV_ERR_INCOMPLETE); } node = N.left; continue; }
       if (hr) { node = N.right; continue; }
     }
     if (sp == 0) return 0;

@@ -8,15 +8,10 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdexcept>
-#include <string>
 
 namespace drt {
 
 static thread_local unsigned long long g_kernelLaunches = 0;   // every launch of the build-side kernels (sort, scan, photon map, LBVH) bumps this; the renderer folds it into its stats
-
-#ifndef CK
-#define CK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e_) + " at " #x); } while (0)
-#endif
 
 // ---------------------------------------------------------------------------------------------------------------
 // exclusive scan, u32, any n: 256 threads x 8 items per block, block sums scanned recursively

@@ -74,10 +74,10 @@ int drt_scene_load_cli(drt_ctx* ctx, const char* file, const char* data_dir) {
 int drt_scene_override(drt_ctx* ctx, int32_t spp, int64_t photons) { GUARD(ctx, { ctx->spp = spp; ctx->photons = photons; }, DRT_ERR_SCENE) }
 int drt_scene_finalize(drt_ctx* ctx, int32_t accel_mode) {
   GUARD(ctx, {
-    if ((accel_mode & 3) == 3 || (accel_mode & ~(3 | 256 | 512)) != 0) throw std::runtime_error("unknown acceleration mode (use DRT_ACCEL_REFERENCE, DRT_ACCEL_REFERENCE_FAST or DRT_ACCEL_LBVH)");
+    if (accel_mode < 0 || accel_mode > 2) throw std::runtime_error("unknown acceleration mode (use DRT_ACCEL_REFERENCE, DRT_ACCEL_REFERENCE_FAST or DRT_ACCEL_LBVH)");
     ctx->scene->overrideSpp(ctx->spp); ctx->scene->overridePhotons(ctx->photons);
     ctx->scene->finalize();
-    if (ctx->renderer) { ctx->renderer->setTraceMode(accel_mode); const double t0 = wallMs(); ctx->renderer->upload(*ctx->scene); ctx->msUpload = wallMs() - t0; ctx->finalized = true; } }, DRT_ERR_SCENE)
+    if (ctx->renderer) { ctx->renderer->setAccelMode(accel_mode); const double t0 = wallMs(); ctx->renderer->upload(*ctx->scene); ctx->msUpload = wallMs() - t0; ctx->finalized = true; } }, DRT_ERR_SCENE)
 }
 int drt_scene_reupload(drt_ctx* ctx) { NEED_DEV(ctx) GUARD(ctx, { if (!ctx->finalized) throw std::runtime_error("scene not finalized"); ctx->renderer->upload(*ctx->scene, true); }, DRT_ERR_STATE) }
 int drt_accel_info(drt_ctx* ctx, double* out4) { NEED_DEV(ctx) GUARD(ctx, { if (!ctx->finalized || !out4) throw std::runtime_error("scene not finalized"); ctx->renderer->accelInfo(out4); }, DRT_ERR_STATE) }

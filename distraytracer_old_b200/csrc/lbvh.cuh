@@ -7,6 +7,7 @@
 // reference tree holds (its dropped object, SURVEY Q2, is already absent from the packed records), the root-box gate stays the
 // reference's (SURVEY Q1a), so primary-ray hit IDs are unchanged; see DESIGN.md for what cannot match (Q1b).
 #pragma once
+#include "dbuf.h"
 #include "dev_sort.cuh"
 
 namespace drt {
@@ -89,36 +90,28 @@ __global__ void k_lbvh_refit(int nLeaves, int nTris, int triBase, int nodeBase, 
 // host driver: rebuilds one BVH. `trisAll` is the device copy of the packed-triangle array (the BVH's range is re-ordered in place),
 // nodesOut receives nLeaves-1 nodes whose child links are absolute (nodeBase + i). Returns the number of nodes written (0 = not rebuilt).
 struct LbvhScratch {
-  uint32_t *keys[2] = {nullptr, nullptr}, *vals[2] = {nullptr, nullptr}, *hist = nullptr, *scan = nullptr, *leafCode = nullptr; unsigned int* flags = nullptr;
-  FTri* tmp = nullptr; LbvhBox *leafBox = nullptr, *nodeBox = nullptr; int2* child = nullptr; int *parentI = nullptr, *parentL = nullptr; size_t cap = 0;
-  void ensure(size_t n) {
-    if (n <= cap) return; release(); cap = n + n / 4 + 1024;
-    for (int k = 0; k < 2; ++k) { CK(cudaMalloc(&keys[k], cap * 4)); CK(cudaMalloc(&vals[k], cap * 4)); }
-    const long long nb = radixBlocks((long long)cap);
-    CK(cudaMalloc(&hist, (size_t)256 * nb * 4)); CK(cudaMalloc(&scan, (size_t)scanScratchWords(256 * nb) * 4));
-    CK(cudaMalloc(&leafCode, cap * 4)); CK(cudaMalloc(&flags, cap * 4)); CK(cudaMalloc(&tmp, cap * sizeof(FTri)));
-    CK(cudaMalloc(&leafBox, cap * sizeof(LbvhBox))); CK(cudaMalloc(&nodeBox, cap * sizeof(LbvhBox))); CK(cudaMalloc(&child, cap * sizeof(int2)));
-    CK(cudaMalloc(&parentI, cap * 4)); CK(cudaMalloc(&parentL, cap * 4));
-  }
-  void release() {
-    for (int k = 0; k < 2; ++k) { cudaFree(keys[k]); cudaFree(vals[k]); keys[k] = vals[k] = nullptr; }
-    cudaFree(hist); cudaFree(scan); cudaFree(leafCode); cudaFree(flags); cudaFree(tmp); cudaFree(leafBox); cudaFree(nodeBox); cudaFree(child); cudaFree(parentI); cudaFree(parentL);
-    hist = scan = leafCode = nullptr; flags = nullptr; tmp = nullptr; leafBox = nodeBox = nullptr; child = nullptr; parentI = parentL = nullptr; cap = 0;
+  DBuf<uint32_t> keys[2], vals[2], hist, scan, leafCode; DBuf<unsigned int> flags; DBuf<FTri> tmp; DBuf<LbvhBox> leafBox, nodeBox; DBuf<int2> child; DBuf<int> parentI, parentL;
+  void ensure(size_t n, cudaStream_t st) {
+    for (int k = 0; k < 2; ++k) { keys[k].ensure(n, st); vals[k].ensure(n, st); }
+    const long long nb = radixBlocks((long long)n);
+    hist.ensure((size_t)256 * nb, st); scan.ensure((size_t)scanScratchWords(256 * nb), st);
+    leafCode.ensure(n, st); flags.ensure(n, st); tmp.ensure(n, st); leafBox.ensure(n, st); nodeBox.ensure(n, st); child.ensure(n, st); parentI.ensure(n, st); parentL.ensure(n, st);
   }
 };
 static inline int lbvhBuild(FTri* trisAll, int triStart, int nTris, const double bmin[3], const double bmax[3], FNode* nodesOut, int nodeBase, LbvhScratch& sc, cudaStream_t st) {
   const int nLeaves = (nTris + 3) / 4; if (nLeaves < 2) return 0;
-  sc.ensure((size_t)nTris);
+  sc.ensure((size_t)nTris, st);
   LbvhBox root; for (int k = 0; k < 3; ++k) { root.mn[k] = bmin[k]; root.mx[k] = bmax[k]; }
   FTri* range = trisAll + triStart;
-  k_lbvh_morton<<<(nTris + 255) / 256, 256, 0, st>>>(range, nTris, root, sc.keys[0]); ++g_kernelLaunches;
-  const int cur = radixSortPairs(sc.keys, sc.vals, nTris, 30, true, sc.hist, sc.scan, st);
-  k_lbvh_gather<<<(unsigned)(((long long)nTris * 8 + 255) / 256), 256, 0, st>>>(range, sc.vals[cur], nTris, sc.tmp); ++g_kernelLaunches;
-  CK(cudaMemcpyAsync(range, sc.tmp, (size_t)nTris * sizeof(FTri), cudaMemcpyDeviceToDevice, st));
-  k_lbvh_leaves<<<(nLeaves + 255) / 256, 256, 0, st>>>(range, sc.keys[cur], nTris, nLeaves, sc.leafBox, sc.leafCode); ++g_kernelLaunches;
-  k_lbvh_hierarchy<<<(nLeaves - 1 + 255) / 256, 256, 0, st>>>(sc.leafCode, nLeaves, sc.child, sc.parentI, sc.parentL); ++g_kernelLaunches;
-  CK(cudaMemsetAsync(sc.flags, 0, (size_t)nLeaves * 4, st));
-  k_lbvh_refit<<<(nLeaves + 255) / 256, 256, 0, st>>>(nLeaves, nTris, triStart, nodeBase, sc.child, sc.parentI, sc.parentL, sc.leafBox, sc.nodeBox, sc.flags, nodesOut); ++g_kernelLaunches;
+  uint32_t* keys[2] = {sc.keys[0].p, sc.keys[1].p}; uint32_t* vals[2] = {sc.vals[0].p, sc.vals[1].p};
+  k_lbvh_morton<<<(nTris + 255) / 256, 256, 0, st>>>(range, nTris, root, keys[0]); ++g_kernelLaunches;
+  const int cur = radixSortPairs(keys, vals, nTris, 30, true, sc.hist.p, sc.scan.p, st);
+  k_lbvh_gather<<<(unsigned)(((long long)nTris * 8 + 255) / 256), 256, 0, st>>>(range, vals[cur], nTris, sc.tmp.p); ++g_kernelLaunches;
+  CK(cudaMemcpyAsync(range, sc.tmp.p, (size_t)nTris * sizeof(FTri), cudaMemcpyDeviceToDevice, st));
+  k_lbvh_leaves<<<(nLeaves + 255) / 256, 256, 0, st>>>(range, keys[cur], nTris, nLeaves, sc.leafBox.p, sc.leafCode.p); ++g_kernelLaunches;
+  k_lbvh_hierarchy<<<(nLeaves - 1 + 255) / 256, 256, 0, st>>>(sc.leafCode.p, nLeaves, sc.child.p, sc.parentI.p, sc.parentL.p); ++g_kernelLaunches;
+  CK(cudaMemsetAsync(sc.flags.p, 0, (size_t)nLeaves * 4, st));
+  k_lbvh_refit<<<(nLeaves + 255) / 256, 256, 0, st>>>(nLeaves, nTris, triStart, nodeBase, sc.child.p, sc.parentI.p, sc.parentL.p, sc.leafBox.p, sc.nodeBox.p, sc.flags.p, nodesOut); ++g_kernelLaunches;
   return nLeaves - 1;
 }
 

@@ -14,6 +14,7 @@
 // Photon order is canonical: record order = (photon index, light index, store index), independent of launch geometry and of how
 // photon indices are split across GPUs; the per-cell order after the stable sort inherits it, so sums are reproducible.
 #pragma once
+#include "dbuf.h"
 #include "dev_sort.cuh"
 #include <algorithm>
 #include <vector>
@@ -238,7 +239,7 @@ __device__ inline PhRanges phWarpRanges(const DScene& S, bool fine, const int lo
   const unsigned lane = threadIdx.x & 31;
   const int x0 = lo[0], x1 = hi[0], y0 = lo[1], z0 = lo[2], nx = fine ? (x1 >> 2) - (x0 >> 2) + 1 : 1, ny = hi[1] - y0 + 1, nz = hi[2] - z0 + 1;
   int slots = nx * ny * nz;
-  if (slots > DRT_PH_MAXRANGES) { flagError(1u); slots = 0; }      // excluded by the bound above; the host reports an incomplete result
+  if (slots > DRT_PH_MAXRANGES) { flagError(DEV_ERR_INCOMPLETE); slots = 0; }      // excluded by the bound above; the host reports an incomplete result
   uint32_t nRanges = 0, total = 0;
   for (int s0 = 0; s0 < slots; s0 += 32) {
     const int slot = s0 + (int)lane; uint32_t a = 0, b = 0;
@@ -644,25 +645,12 @@ __global__ void __launch_bounds__(128) k_photon_probe(const __grid_constant__ DS
 // ---------------------------------------------------------------------------------------------------------------
 struct PhotonMap {
   bool built = false, emitted = false; unsigned long long count = 0, segments = 0;
-  PhotonRec* rec = nullptr; size_t recCap = 0;                  // canonical-order records (emission output / grid input)
-  double4 *pos = nullptr, *pwr = nullptr; float4* pos32 = nullptr; uint32_t* cellStart = nullptr; size_t sortedCap = 0, cellCap = 0;
+  DBuf<PhotonRec> rec;                                          // canonical-order records (emission output / grid input)
+  DBuf<double4> pos, pwr; DBuf<float4> pos32; DBuf<uint32_t> cellStart;      // the sorted map
   PhGrid grid{}; float msEmit = 0, msBuild = 0;
-  // grow-only scratch (no cudaMalloc / cudaFree on the per-frame path: they cost tens to hundreds of ms when they hit the driver's slow path)
-  struct Scratch { void* p = nullptr; size_t cap = 0; template <class T> T* get(size_t n) { const size_t b = n * sizeof(T); if (b > cap) { cudaFree(p); p = nullptr; cap = b + b / 4 + 4096; CK(cudaMalloc(&p, cap)); } return reinterpret_cast<T*>(p); }
-                   void release() { cudaFree(p); p = nullptr; cap = 0; } };
-  Scratch sSlots, sCnt, sOff, sScan, sKeys[2], sVals[2], sHist, sBounds; cudaEvent_t evA = nullptr, evB = nullptr;
-  void events() { if (!evA) { CK(cudaEventCreate(&evA)); CK(cudaEventCreate(&evB)); } }
+  DBuf<PhotonRec> sSlots; DBuf<uint32_t> sCnt, sOff, sScan, sKeys[2], sVals[2], sHist; DBuf<double> sBounds; DEvent evA, evB;
 
   void reset() { built = false; emitted = false; count = 0; segments = 0; }
-  void release() { cudaFree(rec); cudaFree(pos); cudaFree(pwr); cudaFree(pos32); cudaFree(cellStart); rec = nullptr; pos = pwr = nullptr; pos32 = nullptr; cellStart = nullptr; recCap = sortedCap = cellCap = 0; reset();
-    sSlots.release(); sCnt.release(); sOff.release(); sScan.release(); sHist.release(); sBounds.release(); for (int k = 0; k < 2; ++k) { sKeys[k].release(); sVals[k].release(); }
-    if (evA) { cudaEventDestroy(evA); cudaEventDestroy(evB); evA = evB = nullptr; } }
-  void ensureRec(size_t n, cudaStream_t st) {
-    if (n <= recCap) return;
-    size_t nc = n + n / 2 + 4096; PhotonRec* q = nullptr; CK(cudaMalloc(&q, nc * sizeof(PhotonRec)));
-    if (rec && count) CK(cudaMemcpyAsync(q, rec, count * sizeof(PhotonRec), cudaMemcpyDeviceToDevice, st));
-    CK(cudaStreamSynchronize(st)); cudaFree(rec); rec = q; recCap = nc;
-  }
 
   // photons [i0, i1) of every light -> appended to `rec` in canonical order. Chunked so the slot buffer stays bounded.
   void emitRange(const DScene& ds, long long i0, long long i1, Counters* ctr, Counters* ctrHost, cudaStream_t st) {
@@ -671,9 +659,9 @@ struct PhotonMap {
     const int maxStore = ds.g.photonKind == 1 ? 1 : (ds.g.numPhotonRays + 1);
     const long long chunkPhotons = std::max<long long>(1, (1ll << 21) / nl);
     const long long maxThreads = std::min(chunkPhotons, i1 - i0) * nl;
-    PhotonRec* slots = sSlots.get<PhotonRec>((size_t)maxThreads * maxStore); uint32_t* cnt = sCnt.get<uint32_t>((size_t)maxThreads + 1); uint32_t* off = sOff.get<uint32_t>((size_t)maxThreads + 1);
-    uint32_t* scratch = sScan.get<uint32_t>((size_t)scanScratchWords(maxThreads + 1));
-    events(); cudaEvent_t e0 = evA, e1 = evB; CK(cudaEventRecord(e0, st));
+    PhotonRec* slots = sSlots.ensure((size_t)maxThreads * maxStore, st); uint32_t* cnt = sCnt.ensure((size_t)maxThreads + 1, st); uint32_t* off = sOff.ensure((size_t)maxThreads + 1, st);
+    uint32_t* scratch = sScan.ensure((size_t)scanScratchWords(maxThreads + 1), st);
+    CK(cudaEventRecord(evA, st));
     CK(cudaMemsetAsync(&ctr->pad, 0, sizeof(unsigned long long), st));
     for (long long c0 = i0; c0 < i1; c0 += chunkPhotons) {
       const long long np = std::min(chunkPhotons, i1 - c0), nt = np * nl;
@@ -681,18 +669,18 @@ struct PhotonMap {
       k_photon_emit<<<(unsigned)((nt + 127) / 128), 128, 0, st>>>(ds, c0, nt, maxStore, slots, cnt, ctr); ++g_kernelLaunches;
       scanExclusiveU32(cnt, off, nt + 1, scratch, st);
       uint32_t total = 0; CK(cudaMemcpyAsync(&total, off + nt, 4, cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st));
-      ensureRec(count + total, st);
-      if (total) { k_photon_compact<<<(unsigned)((nt + 255) / 256), 256, 0, st>>>(nt, maxStore, slots, cnt, off, rec + count); ++g_kernelLaunches; }
+      rec.ensure(count + total, st, true);
+      if (total) { k_photon_compact<<<(unsigned)((nt + 255) / 256), 256, 0, st>>>(nt, maxStore, slots, cnt, off, rec.p + count); ++g_kernelLaunches; }
       count += total;
     }
     CK(cudaMemcpyAsync(ctrHost, ctr, sizeof(Counters), cudaMemcpyDeviceToHost, st));
-    CK(cudaEventRecord(e1, st)); CK(cudaStreamSynchronize(st)); CK(cudaGetLastError());
-    segments = ctrHost->pad; CK(cudaEventElapsedTime(&msEmit, e0, e1));
+    CK(cudaEventRecord(evB, st)); CK(cudaStreamSynchronize(st)); CK(cudaGetLastError());
+    segments = ctrHost->pad; CK(cudaEventElapsedTime(&msEmit, evA, evB));
   }
   // replace the record store with `n` records that already live on the device (multi-GPU: the all-gathered set)
   void setRecords(const PhotonRec* srcDev, unsigned long long n, cudaStream_t st) {
-    built = false; emitted = true; count = 0; ensureRec((size_t)n, st);
-    if (n) CK(cudaMemcpyAsync(rec, srcDev, n * sizeof(PhotonRec), cudaMemcpyDeviceToDevice, st));
+    built = false; emitted = true; count = 0; rec.ensure((size_t)n, st);
+    if (n) CK(cudaMemcpyAsync(rec.p, srcDev, n * sizeof(PhotonRec), cudaMemcpyDeviceToDevice, st));
     count = n; CK(cudaStreamSynchronize(st));
   }
 
@@ -700,11 +688,11 @@ struct PhotonMap {
     ds.numPhotons = 0; ds.phPos = nullptr; ds.phPwr = nullptr; ds.cellStart = nullptr; ds.phPos32 = nullptr; ds.phAbsMax = 0; ds.padP = 0; built = true; msBuild = 0;
     if (count == 0) return;
     if (count >= 0xFFFFFFF0ull) throw std::runtime_error("photon map larger than 2^32 records");
-    events(); cudaEvent_t e0 = evA, e1 = evB; CK(cudaEventRecord(e0, st));
+    CK(cudaEventRecord(evA, st));
     const long long n = (long long)count;
     // bounds
-    const int nbB = 592; double* bmm = sBounds.get<double>((size_t)nbB * 6);
-    k_photon_bounds<<<nbB, 256, 0, st>>>(rec, n, bmm); ++g_kernelLaunches;
+    const int nbB = 592; double* bmm = sBounds.ensure((size_t)nbB * 6, st);
+    k_photon_bounds<<<nbB, 256, 0, st>>>(rec.p, n, bmm); ++g_kernelLaunches;
     std::vector<double> hb(nbB * 6); CK(cudaMemcpyAsync(hb.data(), bmm, hb.size() * 8, cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st));
     double mn[3] = {DRT_DMAX, DRT_DMAX, DRT_DMAX}, mx[3] = {-DRT_DMAX, -DRT_DMAX, -DRT_DMAX};
     for (int b = 0; b < nbB; ++b) for (int k = 0; k < 3; ++k) { mn[k] = std::min(mn[k], hb[b * 6 + k]); mx[k] = std::max(mx[k], hb[b * 6 + 3 + k]); }
@@ -717,20 +705,19 @@ struct PhotonMap {
     }
     G.cell = cell; for (int k = 0; k < 3; ++k) G.gmin[k] = mn[k]; G.nCells = G.dim[0] * G.dim[1] * G.dim[2] * 64u; grid = G;     // nCells counts FINE cells
     // keys + per-cell counts, cellStart = exclusive scan (nCells + 1 entries: cellStart[nCells] = n)
-    if ((size_t)G.nCells + 1 > cellCap) { cudaFree(cellStart); cellCap = (size_t)G.nCells + 1 + (size_t)G.nCells / 4; CK(cudaMalloc(&cellStart, cellCap * 4)); }
-    if ((size_t)n > sortedCap) { cudaFree(pos); cudaFree(pwr); cudaFree(pos32); sortedCap = (size_t)n + (size_t)n / 8 + 1024; CK(cudaMalloc(&pos, sortedCap * sizeof(double4))); CK(cudaMalloc(&pwr, sortedCap * sizeof(double4))); CK(cudaMalloc(&pos32, sortedCap * sizeof(float4))); }
+    uint32_t* cells = cellStart.ensure((size_t)G.nCells + 1, st); pos.ensure((size_t)n, st); pwr.ensure((size_t)n, st); pos32.ensure((size_t)n, st);
     uint32_t *keys[2], *vals[2]; const long long nb = radixBlocks(n);
-    for (int k = 0; k < 2; ++k) { keys[k] = sKeys[k].get<uint32_t>((size_t)n); vals[k] = sVals[k].get<uint32_t>((size_t)n); }
+    for (int k = 0; k < 2; ++k) { keys[k] = sKeys[k].ensure((size_t)n, st); vals[k] = sVals[k].ensure((size_t)n, st); }
     const long long scanWords = std::max(scanScratchWords(256 * nb), scanScratchWords((long long)G.nCells + 1));
-    uint32_t* hist = sHist.get<uint32_t>((size_t)256 * nb); uint32_t* scratch = sScan.get<uint32_t>((size_t)scanWords);
-    CK(cudaMemsetAsync(cellStart, 0, ((size_t)G.nCells + 1) * 4, st));
-    k_photon_cellkeys<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(rec, n, G, keys[0], cellStart); ++g_kernelLaunches;
-    scanExclusiveU32(cellStart, cellStart, (long long)G.nCells + 1, scratch, st);
+    uint32_t* hist = sHist.ensure((size_t)256 * nb, st); uint32_t* scratch = sScan.ensure((size_t)scanWords, st);
+    CK(cudaMemsetAsync(cells, 0, ((size_t)G.nCells + 1) * 4, st));
+    k_photon_cellkeys<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(rec.p, n, G, keys[0], cells); ++g_kernelLaunches;
+    scanExclusiveU32(cells, cells, (long long)G.nCells + 1, scratch, st);
     int bits = 1; while ((1ull << bits) < (unsigned long long)G.nCells) ++bits;
     const int cur = radixSortPairs(keys, vals, n, bits, true, hist, scratch, st);
-    k_photon_reorder<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(rec, vals[cur], n, pos, pwr, pos32); ++g_kernelLaunches;
-    CK(cudaEventRecord(e1, st)); CK(cudaStreamSynchronize(st)); CK(cudaGetLastError()); CK(cudaEventElapsedTime(&msBuild, e0, e1));
-    ds.numPhotons = (uint32_t)n; ds.phPos = reinterpret_cast<const double*>(pos); ds.phPwr = reinterpret_cast<const double*>(pwr); ds.cellStart = cellStart; ds.phPos32 = reinterpret_cast<const float*>(pos32);
+    k_photon_reorder<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(rec.p, vals[cur], n, pos.p, pwr.p, pos32.p); ++g_kernelLaunches;
+    CK(cudaEventRecord(evB, st)); CK(cudaStreamSynchronize(st)); CK(cudaGetLastError()); CK(cudaEventElapsedTime(&msBuild, evA, evB));
+    ds.numPhotons = (uint32_t)n; ds.phPos = reinterpret_cast<const double*>(pos.p); ds.phPwr = reinterpret_cast<const double*>(pwr.p); ds.cellStart = cells; ds.phPos32 = reinterpret_cast<const float*>(pos32.p);
     { double a = 0; for (int k = 0; k < 3; ++k) a = std::max(a, std::max(std::fabs(mn[k]), std::fabs(mx[k]))); const float f = (float)a; ds.phAbsMax = f >= a ? f : std::nextafter(f, INFINITY); ds.padP = 0; }
     for (int k = 0; k < 3; ++k) { ds.gridDim[k] = G.dim[k]; ds.gridMin[k] = G.gmin[k]; } ds.cellSize = G.cell;
   }
@@ -739,7 +726,7 @@ struct PhotonMap {
 
   long long download(double* out6, long long cap, cudaStream_t st) {
     long long n = std::min<long long>((long long)count, cap); if (n <= 0 || !out6) return (long long)count;
-    CK(cudaMemcpyAsync(out6, rec, (size_t)n * sizeof(PhotonRec), cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st)); return n;
+    CK(cudaMemcpyAsync(out6, rec.p, (size_t)n * sizeof(PhotonRec), cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st)); return n;
   }
 };
 

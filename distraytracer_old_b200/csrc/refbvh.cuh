@@ -14,6 +14,7 @@
 // All sorts are the LSD radix sort of dev_sort.cuh (HBM-bound: per pass 3 x 4 B read + 2 x 4 B written per object).
 // Result: the same ord[] array as the host recursion, bit for bit (tests/test_gpu_refbvh.py compares the BVH dumps).
 #pragma once
+#include "dbuf.h"
 #include "dev_sort.cuh"
 #include <algorithm>
 #include <vector>
@@ -83,32 +84,16 @@ __global__ void k_rb_keys(const uint32_t* __restrict__ ord, const uint32_t* __re
 __global__ void k_rb_gather(const uint32_t* __restrict__ src, const uint32_t* __restrict__ idx, int n, uint32_t* __restrict__ dst) { const int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) dst[i] = src[idx[i]]; }
 
 struct RefBvhScratch {
-  double *key[3] = {nullptr, nullptr, nullptr}, *keyOfRank[3] = {nullptr, nullptr, nullptr};
-  uint32_t *rank[3] = {nullptr, nullptr, nullptr}, *keys[2] = {nullptr, nullptr}, *vals[2] = {nullptr, nullptr}, *ord[2] = {nullptr, nullptr}, *runOfPos = nullptr, *flag = nullptr, *hist = nullptr, *scan = nullptr, *mn = nullptr, *mx = nullptr;
-  int32_t *runStart = nullptr, *runKind = nullptr, *axis = nullptr; unsigned int* err = nullptr; size_t cap = 0, runCap = 0;
-  void ensure(size_t n, size_t runsTotal, size_t runsMax) {
-    if (n > cap) {
-      releaseN(); cap = n + n / 8 + 1024;
-      for (int a = 0; a < 3; ++a) { CK(cudaMalloc(&key[a], cap * 8)); CK(cudaMalloc(&keyOfRank[a], cap * 8)); CK(cudaMalloc(&rank[a], cap * 4)); }
-      for (int k = 0; k < 2; ++k) { CK(cudaMalloc(&keys[k], cap * 4)); CK(cudaMalloc(&vals[k], cap * 4)); CK(cudaMalloc(&ord[k], cap * 4)); }
-      CK(cudaMalloc(&runOfPos, cap * 4)); CK(cudaMalloc(&flag, cap * 4));
-      const long long nb = radixBlocks((long long)cap);
-      CK(cudaMalloc(&hist, (size_t)256 * nb * 4)); CK(cudaMalloc(&scan, (size_t)(scanScratchWords(256 * nb) + scanScratchWords((long long)cap)) * 4));
-      CK(cudaMalloc(&err, 4));
-    }
-    if (runsTotal > runCap) {
-      releaseRuns(); runCap = runsTotal + runsTotal / 8 + 64;
-      CK(cudaMalloc(&runStart, runCap * 4)); CK(cudaMalloc(&runKind, runCap * 4)); CK(cudaMalloc(&axis, runCap * 4)); CK(cudaMalloc(&mn, runCap * 12)); CK(cudaMalloc(&mx, runCap * 12));
-    }
-    (void)runsMax;
+  DBuf<double> key[3], keyOfRank[3]; DBuf<uint32_t> rank[3], keys[2], vals[2], ord[2], runOfPos, flag, hist, sortScan, rankScan, mn, mx;
+  DBuf<int32_t> runStart, runKind, axis; DBuf<unsigned int> err; DEvent ev[2];
+  void ensure(size_t n, size_t runs, cudaStream_t st) {
+    for (int a = 0; a < 3; ++a) { key[a].ensure(n, st); keyOfRank[a].ensure(n, st); rank[a].ensure(n, st); }
+    for (int k = 0; k < 2; ++k) { keys[k].ensure(n, st); vals[k].ensure(n, st); ord[k].ensure(n, st); }
+    runOfPos.ensure(n, st); flag.ensure(n, st);
+    const long long nb = radixBlocks((long long)n);
+    hist.ensure((size_t)256 * nb, st); sortScan.ensure((size_t)scanScratchWords(256 * nb), st); rankScan.ensure((size_t)scanScratchWords((long long)n), st); err.ensure(1, st);
+    runStart.ensure(runs, st); runKind.ensure(runs, st); axis.ensure(runs, st); mn.ensure(3 * runs, st); mx.ensure(3 * runs, st);
   }
-  void releaseN() {
-    for (int a = 0; a < 3; ++a) { cudaFree(key[a]); cudaFree(keyOfRank[a]); cudaFree(rank[a]); key[a] = keyOfRank[a] = nullptr; rank[a] = nullptr; }
-    for (int k = 0; k < 2; ++k) { cudaFree(keys[k]); cudaFree(vals[k]); cudaFree(ord[k]); keys[k] = vals[k] = ord[k] = nullptr; }
-    cudaFree(runOfPos); cudaFree(flag); cudaFree(hist); cudaFree(scan); cudaFree(err); runOfPos = flag = hist = scan = nullptr; err = nullptr; cap = 0;
-  }
-  void releaseRuns() { cudaFree(runStart); cudaFree(runKind); cudaFree(axis); cudaFree(mn); cudaFree(mx); runStart = runKind = axis = nullptr; mn = mx = nullptr; runCap = 0; }
-  void release() { releaseN(); releaseRuns(); }
 };
 
 // keysHost = [3][n]; ordHost[n] receives the order.  Returns false when the device cannot decide (NaN / infinite spans): the host recursion then
@@ -129,57 +114,57 @@ static inline bool refOrderDevice(int n, const double* keysHost, int32_t* ordHos
       for (const Seg& g : cur) if (g.count > 5) { const int split = (int)(.5 * g.count); next.push_back({g.s, split, split}); next.push_back({g.s + split, g.count - split, g.count - split}); }
       cur.swap(next);
     } }
-  int runsMax = 0; for (int r : lvlRuns) runsMax = std::max(runsMax, r);
-  sc.ensure((size_t)n, runStart.size(), (size_t)runsMax);
-  cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1)); CK(cudaEventRecord(e0, st));
-  for (int a = 0; a < 3; ++a) CK(cudaMemcpyAsync(sc.key[a], keysHost + (size_t)a * n, (size_t)n * 8, cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(sc.runStart, runStart.data(), runStart.size() * 4, cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(sc.runKind, runKind.data(), runKind.size() * 4, cudaMemcpyHostToDevice, st));
-  CK(cudaMemsetAsync(sc.err, 0, 4, st));
+  sc.ensure((size_t)n, runStart.size(), st);
+  CK(cudaEventRecord(sc.ev[0], st));
+  for (int a = 0; a < 3; ++a) CK(cudaMemcpyAsync(sc.key[a].p, keysHost + (size_t)a * n, (size_t)n * 8, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(sc.runStart.p, runStart.data(), runStart.size() * 4, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(sc.runKind.p, runKind.data(), runKind.size() * 4, cudaMemcpyHostToDevice, st));
+  CK(cudaMemsetAsync(sc.err.p, 0, 4, st));
   const unsigned gN = (unsigned)((n + 255) / 256);
   int rankBits = 1; while ((1ll << rankBits) < (long long)n) ++rankBits;
-  uint32_t* scanScratch2 = sc.scan + scanScratchWords(256 * radixBlocks((long long)sc.cap));
+  uint32_t* keys[2] = {sc.keys[0].p, sc.keys[1].p}; uint32_t* vals[2] = {sc.vals[0].p, sc.vals[1].p};
+  const uint32_t* rank[3] = {sc.rank[0].p, sc.rank[1].p, sc.rank[2].p}; const double* keyOfRank[3] = {sc.keyOfRank[0].p, sc.keyOfRank[1].p, sc.keyOfRank[2].p};
+  uint32_t* ord[2] = {sc.ord[0].p, sc.ord[1].p};
   // ---- dense ranks per axis
   for (int a = 0; a < 3; ++a) {
-    k_rb_lowkeys<<<gN, 256, 0, st>>>(sc.key[a], n, sc.keys[0]); ++g_kernelLaunches;
-    int cur = radixSortPairs(sc.keys, sc.vals, n, 32, true, sc.hist, sc.scan, st);
-    uint32_t* k2[2] = {sc.keys[cur ^ 1], sc.keys[cur]}; uint32_t* v2[2] = {sc.vals[cur], sc.vals[cur ^ 1]};
-    k_rb_highkeys<<<gN, 256, 0, st>>>(sc.key[a], v2[0], n, k2[0]); ++g_kernelLaunches;
-    const int c2 = radixSortPairs(k2, v2, n, 32, false, sc.hist, sc.scan, st);
+    k_rb_lowkeys<<<gN, 256, 0, st>>>(sc.key[a].p, n, keys[0]); ++g_kernelLaunches;
+    int cur = radixSortPairs(keys, vals, n, 32, true, sc.hist.p, sc.sortScan.p, st);
+    uint32_t* k2[2] = {keys[cur ^ 1], keys[cur]}; uint32_t* v2[2] = {vals[cur], vals[cur ^ 1]};
+    k_rb_highkeys<<<gN, 256, 0, st>>>(sc.key[a].p, v2[0], n, k2[0]); ++g_kernelLaunches;
+    const int c2 = radixSortPairs(k2, v2, n, 32, false, sc.hist.p, sc.sortScan.p, st);
     const uint32_t* order = v2[c2];
-    k_rb_flags<<<gN, 256, 0, st>>>(sc.key[a], order, n, sc.flag); ++g_kernelLaunches;
-    scanExclusiveU32(sc.flag, sc.runOfPos, n, scanScratch2, st);
-    k_rb_ranks<<<gN, 256, 0, st>>>(sc.key[a], order, sc.runOfPos, sc.flag, n, sc.rank[a], sc.keyOfRank[a]); ++g_kernelLaunches;
+    k_rb_flags<<<gN, 256, 0, st>>>(sc.key[a].p, order, n, sc.flag.p); ++g_kernelLaunches;
+    scanExclusiveU32(sc.flag.p, sc.runOfPos.p, n, sc.rankScan.p, st);
+    k_rb_ranks<<<gN, 256, 0, st>>>(sc.key[a].p, order, sc.runOfPos.p, sc.flag.p, n, sc.rank[a].p, sc.keyOfRank[a].p); ++g_kernelLaunches;
   }
   // ---- levels
-  int oc = 0; k_rb_iota<<<gN, 256, 0, st>>>(n, sc.ord[0]); ++g_kernelLaunches;
+  int oc = 0; k_rb_iota<<<gN, 256, 0, st>>>(n, ord[0]); ++g_kernelLaunches;
   for (size_t L = 0; L < lvlOff.size(); ++L) {
-    const int nRuns = lvlRuns[L]; const int32_t* rs = sc.runStart + lvlOff[L]; const int32_t* rk = sc.runKind + lvlOff[L]; int32_t* ax = sc.axis + lvlOff[L];
+    const int nRuns = lvlRuns[L]; const int32_t* rs = sc.runStart.p + lvlOff[L]; const int32_t* rk = sc.runKind.p + lvlOff[L]; int32_t* ax = sc.axis.p + lvlOff[L];
     const unsigned gR = (unsigned)((3 * nRuns + 255) / 256);
-    k_rb_assign<<<gN, 256, 0, st>>>(rs, nRuns, n, sc.runOfPos);
-    k_rb_init_minmax<<<gR, 256, 0, st>>>(nRuns, sc.mn, sc.mx);
-    k_rb_minmax<<<gN, 256, 0, st>>>(sc.ord[oc], sc.runOfPos, rk, sc.rank[0], sc.rank[1], sc.rank[2], n, nRuns, sc.mn, sc.mx);
-    k_rb_axis<<<(unsigned)((nRuns + 255) / 256), 256, 0, st>>>(nRuns, rk, sc.mn, sc.mx, sc.keyOfRank[0], sc.keyOfRank[1], sc.keyOfRank[2], ax, sc.err);
+    k_rb_assign<<<gN, 256, 0, st>>>(rs, nRuns, n, sc.runOfPos.p);
+    k_rb_init_minmax<<<gR, 256, 0, st>>>(nRuns, sc.mn.p, sc.mx.p);
+    k_rb_minmax<<<gN, 256, 0, st>>>(ord[oc], sc.runOfPos.p, rk, rank[0], rank[1], rank[2], n, nRuns, sc.mn.p, sc.mx.p);
+    k_rb_axis<<<(unsigned)((nRuns + 255) / 256), 256, 0, st>>>(nRuns, rk, sc.mn.p, sc.mx.p, keyOfRank[0], keyOfRank[1], keyOfRank[2], ax, sc.err.p);
     int runBits = 1; while ((1ll << runBits) < (long long)nRuns) ++runBits;
     const int composite = (runBits + rankBits <= 32) ? 1 : 0;
-    k_rb_keys<<<gN, 256, 0, st>>>(sc.ord[oc], sc.runOfPos, ax, sc.rank[0], sc.rank[1], sc.rank[2], n, rankBits, composite, sc.keys[0]);
+    k_rb_keys<<<gN, 256, 0, st>>>(ord[oc], sc.runOfPos.p, ax, rank[0], rank[1], rank[2], n, rankBits, composite, keys[0]);
     g_kernelLaunches += 5;
     const uint32_t* perm;
-    if (composite) { const int c = radixSortPairs(sc.keys, sc.vals, n, nRuns > 1 ? runBits + rankBits : rankBits, true, sc.hist, sc.scan, st); perm = sc.vals[c]; }
+    if (composite) { const int c = radixSortPairs(keys, vals, n, nRuns > 1 ? runBits + rankBits : rankBits, true, sc.hist.p, sc.sortScan.p, st); perm = vals[c]; }
     else {
-      const int c = radixSortPairs(sc.keys, sc.vals, n, rankBits, true, sc.hist, sc.scan, st);
-      uint32_t* k2[2] = {sc.keys[c ^ 1], sc.keys[c]}; uint32_t* v2[2] = {sc.vals[c], sc.vals[c ^ 1]};
-      k_rb_gather<<<gN, 256, 0, st>>>(sc.runOfPos, v2[0], n, k2[0]); ++g_kernelLaunches;
-      const int c2 = radixSortPairs(k2, v2, n, runBits, false, sc.hist, sc.scan, st); perm = v2[c2];
+      const int c = radixSortPairs(keys, vals, n, rankBits, true, sc.hist.p, sc.sortScan.p, st);
+      uint32_t* k2[2] = {keys[c ^ 1], keys[c]}; uint32_t* v2[2] = {vals[c], vals[c ^ 1]};
+      k_rb_gather<<<gN, 256, 0, st>>>(sc.runOfPos.p, v2[0], n, k2[0]); ++g_kernelLaunches;
+      const int c2 = radixSortPairs(k2, v2, n, runBits, false, sc.hist.p, sc.sortScan.p, st); perm = v2[c2];
     }
-    k_rb_gather<<<gN, 256, 0, st>>>(sc.ord[oc], perm, n, sc.ord[oc ^ 1]); ++g_kernelLaunches; oc ^= 1;
+    k_rb_gather<<<gN, 256, 0, st>>>(ord[oc], perm, n, ord[oc ^ 1]); ++g_kernelLaunches; oc ^= 1;
   }
   unsigned int err = 0;
-  CK(cudaMemcpyAsync(ordHost, sc.ord[oc], (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-  CK(cudaMemcpyAsync(&err, sc.err, 4, cudaMemcpyDeviceToHost, st));
-  CK(cudaEventRecord(e1, st)); CK(cudaStreamSynchronize(st));
-  float ms = 0; CK(cudaEventElapsedTime(&ms, e0, e1)); if (msOut) *msOut = ms;
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
+  CK(cudaMemcpyAsync(ordHost, ord[oc], (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(&err, sc.err.p, 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaEventRecord(sc.ev[1], st)); CK(cudaStreamSynchronize(st));
+  float ms = 0; CK(cudaEventElapsedTime(&ms, sc.ev[0], sc.ev[1])); if (msOut) *msOut = ms;
   return err == 0;
 }
 

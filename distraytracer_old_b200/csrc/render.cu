@@ -11,21 +11,22 @@
 //   k_resolve  the return path of the recursion: per-bounce clamp (myObjShader.java:661) then weighting (SURVEY Q14)
 //   k_finish   mean of clamped samples, clamp, (int)(c*255) pack (myScene.java:1460, myObjShader.java:671)
 #include "renderer.h"
+#include "dbuf.h"
 #include "dev_shade.cuh"
 #include <cstdio>
+#include <initializer_list>
 #include <stdexcept>
 #include <vector>
 
 namespace drt {
 
-#define CK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) throw std::runtime_error(std::string("CUDA error: ") + cudaGetErrorString(e_) + " at " #x); } while (0)
-
+// the device error word (dev_isect.cuh): devErrorFetch queues its copy to *e, which holds it after the next sync of `st`
 static void devErrorReset(cudaStream_t st) { const unsigned int z = 0; CK(cudaMemcpyToSymbolAsync(g_devError, &z, sizeof(z), 0, cudaMemcpyHostToDevice, st)); }
-static const char* const kDevIncomplete = "device search beyond its capacity (traversal stack overflow, or a photon query with more candidate ranges than the gather holds): the result would be incomplete";
-static void devErrorCheck(cudaStream_t st) {
-  unsigned int e = 0; CK(cudaMemcpyFromSymbolAsync(&e, g_devError, sizeof(e), 0, cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st));
-  if (e & 1u) throw std::runtime_error(kDevIncomplete);
+static void devErrorFetch(unsigned int* e, cudaStream_t st) { CK(cudaMemcpyFromSymbolAsync(e, g_devError, sizeof(*e), 0, cudaMemcpyDeviceToHost, st)); }
+static void throwIfIncomplete(unsigned int e) {
+  if (e & DEV_ERR_INCOMPLETE) throw std::runtime_error("device search beyond its capacity (traversal stack overflow, or a photon query with more candidate ranges than the gather holds): the result would be incomplete");
 }
+static void devErrorCheck(cudaStream_t st) { unsigned int e = 0; devErrorFetch(&e, st); CK(cudaStreamSynchronize(st)); throwIfIncomplete(e); }
 
 struct alignas(16) RayRec { double o[3], d[3]; double kt0, kt1; uint32_t ka, kb, kc, stream; int32_t gen, valid; int32_t pad[2]; };
 struct alignas(16) SurfRec { double loc[3], n[3], rawDir[3], tex[3]; int32_t shader, valid; uint32_t ka, kb, kc, stream; int32_t gen, pad; };
@@ -304,8 +305,8 @@ __global__ void __launch_bounds__(128, DRT_SHADE_MINBLOCKS) k_shade(const __grid
   if (total > 0) {
     if (lane == 31) { qbase = atomicAdd(&ctr->levelCount[w.level + 1], (unsigned long long)total);
       if (ctr->maxLevel < (unsigned long long)(w.level + 1)) atomicMax(&ctr->maxLevel, (unsigned long long)(w.level + 1));
-      if (w.level + 1 >= w.launchedLevels) flagError(4u);                               // deeper than the levels this call launched: the host re-renders with full depth
-      if ((long long)(qbase + total) > nextCap) flagError(2u); }                          // queue / node pool exhausted: the host re-renders with smaller batches
+      if (w.level + 1 >= w.launchedLevels) flagError(DEV_ERR_DEPTH);                    // deeper than the levels this call launched: the host re-renders with full depth
+      if ((long long)(qbase + total) > nextCap) flagError(DEV_ERR_QUEUE); }               // queue / node pool exhausted: the host re-renders with smaller batches
     qbase = __shfl_sync(0xffffffffu, qbase, 31);
   }
   long long at = (long long)qbase + (incl - nChild);
@@ -468,21 +469,13 @@ namespace drt {
 // ---------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------
-template <class T> struct DBuf {
-  T* p = nullptr; size_t cap = 0;
-  void ensure(size_t n, cudaStream_t st, bool keep = false) {
-    if (n <= cap) return;
-    size_t nc = n + n / 4 + 1024; T* q = nullptr; CK(cudaMalloc(&q, nc * sizeof(T)));
-    if (keep && p && cap) CK(cudaMemcpyAsync(q, p, cap * sizeof(T), cudaMemcpyDeviceToDevice, st));
-    if (p) { CK(cudaStreamSynchronize(st)); CK(cudaFree(p)); }
-    p = q; cap = nc;
-  }
-  void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
-};
 // Scene arrays live in ONE device arena fed from ONE pinned host staging buffer (grow-only): a re-upload is a host memcpy per array plus a
 // single H2D DMA -- no cudaMalloc / cudaFree on the per-frame path.
 struct SceneArena {
   char* dev = nullptr; char* host = nullptr; size_t cap = 0, used = 0;
+  SceneArena() = default;
+  SceneArena(const SceneArena&) = delete; SceneArena& operator=(const SceneArena&) = delete;
+  ~SceneArena() { if (dev) cudaFree(dev); if (host) cudaFreeHost(host); }
   void reserve(size_t bytes, cudaStream_t st) {
     if (bytes <= cap) return;
     CK(cudaStreamSynchronize(st)); if (dev) cudaFree(dev); if (host) cudaFreeHost(host);
@@ -498,53 +491,45 @@ struct SceneArena {
   }
   template <class T> static size_t need(const std::vector<T>& v) { return ((v.size() ? v.size() : 1) * sizeof(T) + 255) & ~(size_t)255; }
   void flush(cudaStream_t st) { if (used) CK(cudaMemcpyAsync(dev, host, used, cudaMemcpyHostToDevice, st)); }
-  void release() { if (dev) cudaFree(dev); if (host) cudaFreeHost(host); dev = host = nullptr; cap = used = 0; }
 };
 
+// Everything the renderer allocates on its device; created with that device current, freed with the renderer.
 struct Renderer::Impl {
   DScene ds; SceneArena arena; DBuf<FNode> lbvhNodeBuf; DBuf<FNode32> lbvhNode32Buf; DBuf<FTri> lbvhTriBuf; LbvhScratch lbvhScratch; RefBvhScratch refScratch;
   DBuf<RayRec> rays[2]; DBuf<Hit> hits; DBuf<Hit> hits0; DBuf<SurfRec> surf; DBuf<NodeRec> nodes; DBuf<double> lightPos; Counters* ctr = nullptr; Counters* ctrHost = nullptr;
   DBuf<uint32_t> deferT, deferL;                 // deferral lists of the lean trace / light kernels (ray indices of one level)
-  std::vector<cudaEvent_t> evPool;               // stage timing of a whole frame without a host sync per level
+  std::vector<DEvent> evPool;                    // stage timing of a whole frame without a host sync per level
   int shape = TF_ALL;                            // kernel variant the uploaded scene runs with (see chooseShape)
   bool anySecondary = false;                     // some shader can spawn reflection / refraction rays
   int depthHint = 0;                             // levels the last frame of this scene needed (0 = unknown: launch the full depth)
   double capHint = 0;                            // queue-capacity factor the last frame of this scene ended up with (0 = default)
   int numSMs = 148;
-  cudaEvent_t pev(size_t k) { while (evPool.size() <= k) { cudaEvent_t e; CK(cudaEventCreate(&e)); evPool.push_back(e); } return evPool[k]; }
+  cudaEvent_t pev(size_t k) { while (evPool.size() <= k) evPool.emplace_back(); return evPool[k]; }
   DBuf<int32_t> oArgb, oPrim, oInst; DBuf<double> oRgb, oT;
-  cudaEvent_t ev[8];
-  PhotonMap photons; PhotonMap::Scratch xCnt, xMine, xAll;      // photon record exchange of drt_render_distributed
+  DBuf<double> probeIn[2], probeOut[2];          // inputs and outputs of the parity probes
+  DEvent lbvhEv[2];
+  PhotonMap photons; DBuf<unsigned long long> xCnt; DBuf<PhotonRec> xMine, xAll;      // photon record exchange of drt_render_distributed
   size_t sceneBytes = 0;
   float lbvhMs = 0; long long lbvhTris = 0, lbvhNodes = 0;
   std::vector<FBvh> bvhsUploaded;                // host copy of the FBvh array as uploaded (fastRoot points at the LBVH nodes in DRT_ACCEL_LBVH mode)
+  Impl() { CK(cudaMalloc(&ctr, sizeof(Counters))); CK(cudaMallocHost(&ctrHost, sizeof(Counters))); }
+  ~Impl() { cudaFree(ctr); cudaFreeHost(ctrHost); }
 };
 
-Renderer::Renderer(int device) : impl_(new Impl), device_(device) {
+Renderer::Renderer(int device) : device_(device) {
   int cnt = 0; cudaError_t e = cudaGetDeviceCount(&cnt);
-  if (e != cudaSuccess || cnt == 0) { delete impl_; throw std::runtime_error("no CUDA device available: this renderer has no CPU fallback"); }
+  if (e != cudaSuccess || cnt == 0) throw std::runtime_error("no CUDA device available: this renderer has no CPU fallback");
   CK(cudaSetDevice(device));
-  if (const char* sl = getenv("DRT_STACK_LIMIT")) CK(cudaDeviceSetLimit(cudaLimitStackSize, (size_t)atol(sl)));     // debugging aid
-  cudaStream_t st; CK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking)); stream_ = st;
-  CK(cudaMalloc(&impl_->ctr, sizeof(Counters))); CK(cudaMallocHost(&impl_->ctrHost, sizeof(Counters)));
+  impl_.reset(new Impl);
   { cudaDeviceProp pr; CK(cudaGetDeviceProperties(&pr, device)); impl_->numSMs = pr.multiProcessorCount; }
-  for (auto& e2 : impl_->ev) CK(cudaEventCreate(&e2));
   std::memset(&impl_->ds, 0, sizeof(DScene)); std::memset(&g_, 0, sizeof(g_));
   static const unsigned char p[256] = {151,160,137,91,90,15,131,13,201,95,96,53,194,233,7,225,140,36,103,30,69,142,8,99,37,240,21,10,23,190,6,148,247,120,234,75,0,26,197,62,94,252,219,203,117,35,11,32,57,177,33,88,237,149,56,87,174,20,125,136,171,168,68,175,74,165,71,134,139,48,27,166,77,146,158,231,83,111,229,122,60,211,133,230,220,105,92,41,55,46,245,40,244,102,143,54,65,25,63,161,1,216,80,73,209,76,132,187,208,89,18,169,200,196,135,130,116,188,159,86,164,100,109,198,173,186,3,64,52,217,226,250,124,123,5,202,38,147,118,126,255,82,85,212,207,206,59,227,47,16,58,17,182,189,28,42,223,183,170,213,119,248,152,2,44,154,163,70,221,153,101,155,167,43,172,9,129,22,39,253,19,98,108,110,79,113,224,232,178,185,112,104,218,246,97,228,251,34,242,193,238,210,144,12,191,179,162,241,81,51,145,235,249,14,239,107,49,192,214,31,181,199,106,157,184,84,204,176,115,121,50,45,127,4,150,254,138,236,205,93,222,114,67,29,24,72,243,141,128,195,78,66,215,61,156,180};
   unsigned char perm[512]; for (int i = 0; i < 512; ++i) perm[i] = p[i & 255];
   CK(cudaMemcpyToSymbol(c_perm, perm, 512));
+  cudaStream_t st; CK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking)); stream_ = st;
 }
-Renderer::~Renderer() {
-  cudaSetDevice(device_);
-  impl_->arena.release(); impl_->lbvhNodeBuf.release(); impl_->lbvhNode32Buf.release(); impl_->lbvhTriBuf.release(); impl_->lbvhScratch.release(); impl_->refScratch.release();
-  impl_->rays[0].release(); impl_->rays[1].release(); impl_->hits.release(); impl_->hits0.release(); impl_->surf.release(); impl_->nodes.release(); impl_->lightPos.release();
-  impl_->oArgb.release(); impl_->oPrim.release(); impl_->oInst.release(); impl_->oRgb.release(); impl_->oT.release();
-  impl_->deferT.release(); impl_->deferL.release(); for (auto& e : impl_->evPool) cudaEventDestroy(e);
-  impl_->photons.release(); impl_->xCnt.release(); impl_->xMine.release(); impl_->xAll.release();
-  cudaFree(impl_->ctr); cudaFreeHost(impl_->ctrHost);
-  for (auto& e : impl_->ev) cudaEventDestroy(e);
-  cudaStreamDestroy((cudaStream_t)stream_); delete impl_;
-}
+// impl_ is destroyed after the body, with the device still current
+Renderer::~Renderer() { cudaSetDevice(device_); commDestroy(); cudaStreamDestroy((cudaStream_t)stream_); }
 
 // object order of the reference-topology median-split tree on the device (refbvh.cuh); false = the host recursion has to do it
 bool Renderer::orderBvh(int n, const double* keys, int32_t* ord, double* ms) {
@@ -567,7 +552,7 @@ void Renderer::upload(const HostScene& hs, bool sameScene) {
   }
   DScene& d = impl_->ds; SceneArena& A = impl_->arena;
   std::vector<FBvh> bv = hs.bvhs;
-  d.accelMode = traceMode_ & 3; d.padA = 0;
+  d.accelMode = accelMode_; d.padA = 0;
   // DRT_ACCEL_LBVH: every qualifying pure-triangle BVH is rebuilt on the GPU (lbvh.cuh) after the copy. Node slots: the reference nodes
   // first (instance-level trees, BVHs that do not qualify, rays whose units forbid reordering keep using them), LBVH nodes appended.
   size_t extra = 0;
@@ -581,7 +566,7 @@ void Renderer::upload(const HostScene& hs, bool sameScene) {
   // drt_scene_reupload of the scene that is already staged: the pinned buffer still holds it byte for byte, so the host-side copies are skipped
   // and only the H2D DMA is repeated (e2e timing: "host -> device copy of the step's inputs from pinned host memory")
   const size_t needBytes = SceneArena::need(hs.xforms) + SceneArena::need(hs.prims) + SceneArena::need(hs.pdata) + SceneArena::need(hs.children) + SceneArena::need(hs.nodes) + SceneArena::need(hs.tris) + SceneArena::need(hs.texels);
-  A.fill = !(sameScene && A.stagedScene == (const void*)&hs && A.stagedUsed == needBytes && !getenv("DRT_RESTAGE"));
+  A.fill = !(sameScene && A.stagedScene == (const void*)&hs && A.stagedUsed == needBytes);
   A.begin();
   d.xforms = A.put(hs.xforms); d.prims = A.put(hs.prims); d.pdata = A.put(hs.pdata); d.top = A.put(hs.top); d.children = A.put(hs.children); d.instances = A.put(hs.instances);
   d.lists = A.put(hs.lists); d.nodes = A.put(hs.nodes); d.fnodes32 = A.put(hs.nodes32); d.tris = A.put(hs.tris); d.bvhs = A.put(bv); d.lights = A.put(hs.lights); d.shaders = A.put(hs.shaders);
@@ -596,14 +581,14 @@ void Renderer::upload(const HostScene& hs, bool sameScene) {
     FNode* ln = impl_->lbvhNodeBuf.p; FTri* lt = impl_->lbvhTriBuf.p;
     if (n0) CK(cudaMemcpyAsync(ln, d.nodes, n0 * sizeof(FNode), cudaMemcpyDeviceToDevice, st));
     CK(cudaMemcpyAsync(lt, d.tris, hs.tris.size() * sizeof(FTri), cudaMemcpyDeviceToDevice, st));
-    { size_t mx = 0; for (const FBvh& B : bv) if (B.fast && B.fastRoot != B.root) mx = std::max(mx, (size_t)B.triCount); impl_->lbvhScratch.ensure(mx); }   // scratch is grow-only and allocated outside the timed build
-    CK(cudaEventRecord(impl_->ev[6], st));
+    { size_t mx = 0; for (const FBvh& B : bv) if (B.fast && B.fastRoot != B.root) mx = std::max(mx, (size_t)B.triCount); impl_->lbvhScratch.ensure(mx, st); }   // scratch is grow-only and allocated outside the timed build
+    CK(cudaEventRecord(impl_->lbvhEv[0], st));
     for (const FBvh& B : bv) if (B.fast && B.fastRoot != B.root) {
       const int wrote = lbvhBuild(lt, B.triStart, B.triCount, B.bmin, B.bmax, ln + B.fastRoot, B.fastRoot, impl_->lbvhScratch, st);
       if (wrote != (B.triCount + 3) / 4 - 1) throw std::runtime_error("LBVH node count mismatch");
       impl_->lbvhTris += B.triCount; impl_->lbvhNodes += wrote;
     }
-    CK(cudaEventRecord(impl_->ev[7], st)); CK(cudaStreamSynchronize(st)); CK(cudaGetLastError()); CK(cudaEventElapsedTime(&impl_->lbvhMs, impl_->ev[6], impl_->ev[7]));
+    CK(cudaEventRecord(impl_->lbvhEv[1], st)); CK(cudaStreamSynchronize(st)); CK(cudaGetLastError()); CK(cudaEventElapsedTime(&impl_->lbvhMs, impl_->lbvhEv[0], impl_->lbvhEv[1]));
     impl_->lbvhNode32Buf.ensure(n0 + extra, st);
     k_nodes32<<<(unsigned)((n0 + extra + 255) / 256), 256, 0, st>>>(ln, (long long)(n0 + extra), impl_->lbvhNode32Buf.p); ++g_kernelLaunches;
     CK(cudaStreamSynchronize(st)); CK(cudaGetLastError());
@@ -651,7 +636,12 @@ void Renderer::renderChunks(long long pix0, long long pix1, int world, int rank,
   if (g_.photonKind != 0 && !I.photons.built) { devErrorReset(st); if (!I.photons.emitted) I.photons.emitRange(I.ds, 0, g_.numPhotonsCast, I.ctr, I.ctrHost, st); I.photons.buildGrid(I.ds, st); devErrorCheck(st); }
   const int spp = g_.spp < 1 ? 1 : g_.spp;
   const int fullDepth = I.anySecondary ? std::max(1, std::min(g_.numRays - 1, DRT_MAX_LEVELS)) : 1;      // children spawn while gen < numRays - 2
-  const bool generic = counters_ || I.shape == TF_ALL || (traceMode_ & (256 | 512)) != 0;
+  // kernels of the closest-hit and light passes: the generic kernel alone (counters on, or a scene shape only it serves), or a lean variant
+  // followed by the generic kernel as the fix-up pass over what the lean one deferred
+  using TraceK = decltype(&k_trace<false, TF_ALL>); using LightK = decltype(&k_light<false, TF_ALL>);
+  const bool generic = counters_ || I.shape == TF_ALL;
+  const TraceK traceAll = counters_ ? &k_trace<true, TF_ALL> : &k_trace<false, TF_ALL>, traceLean = generic ? nullptr : I.shape == 0 ? &k_trace<false, 0> : &k_trace<false, TF_LITERAL1>;
+  const LightK lightAll = counters_ ? &k_light<true, TF_ALL> : &k_light<false, TF_ALL>, lightLean = generic ? nullptr : I.shape == 0 ? &k_light<false, 0> : &k_light<false, TF_LITERAL1>;
   long long batchRays = batchRays_; int levels = (I.depthHint > 0) ? std::min(fullDepth, I.depthHint + 1) : fullDepth;
   // queue capacity of a level relative to the batch's primary rays.  2 is the true bound for level 1 and ample for every shipped scene; the true
   // bound of level L is 2^L (binary Fresnel splits), so an overflow doubles the factor (and halves the batch: same memory) and renders again
@@ -674,62 +664,50 @@ void Renderer::renderChunks(long long pix0, long long pix1, int world, int rank,
     devErrorReset(st);
     CK(cudaMemsetAsync(I.ctr, 0, sizeof(Counters), st));
     static const bool syncDebug = getenv("DRT_SYNC_DEBUG") != nullptr;      // debugging aid: locate a faulting kernel
-    auto dbg = [&](const char* what, int level) { if (!syncDebug) return; cudaError_t e = cudaStreamSynchronize(st); if (e == cudaSuccess) e = cudaGetLastError();
-      if (e != cudaSuccess) throw std::runtime_error(std::string("DRT_SYNC_DEBUG: ") + what + " level " + std::to_string(level) + ": " + cudaGetErrorString(e)); };
+    auto launched = [&](const char* what, int level, const char* variant = "") { ++rs.kernelLaunches; if (!syncDebug) return;
+      cudaError_t e = cudaStreamSynchronize(st); if (e == cudaSuccess) e = cudaGetLastError();
+      if (e != cudaSuccess) throw std::runtime_error(std::string("DRT_SYNC_DEBUG: ") + what + variant + " level " + std::to_string(level) + ": " + cudaGetErrorString(e)); };
+    // one closest-hit or light pass of a level; `list` receives what the lean kernel defers.  args: the kernels' arguments before (work, deferOut)
+    auto pass = [&](const char* what, int level, auto lean, auto all, uint32_t* list, unsigned grid, auto... args) {
+      if (!lean) { all<<<grid, 128, 0, st>>>(args..., nullptr, nullptr); launched(what, level, " generic"); return; }
+      lean<<<grid, 128, 0, st>>>(args..., nullptr, list); launched(what, level, " lean");
+      all<<<fixGrid, 128, 0, st>>>(args..., list, nullptr); launched(what, level, " fix-up");
+    };
     size_t evN = 0; std::vector<size_t> evIdx;      // 4 events per (batch, level): before trace, after trace, after shade (+gather), after light
     CK(cudaEventRecord(I.pev(evN), st)); const size_t evStart = evN++;
     for (long long b0 = pix0; b0 < pix1; b0 += pixPerBatch) {
       const long long nPix = std::min(pixPerBatch, pix1 - b0), n0 = nPix * spp;
+      auto wave = [&](int level) { Wave w; w.n0 = n0; w.rayCap = rayCap; w.nodeCap = nodeCap; w.level = level; w.launchedLevels = levels; return w; };
       CK(cudaMemsetAsync(&I.ctr->levelCount, 0, sizeof(Counters) - offsetof(Counters, levelCount), st));
       for (int level = 0; level < levels; ++level) {
-        Wave w; w.n0 = n0; w.rayCap = rayCap; w.nodeCap = nodeCap; w.level = level; w.launchedLevels = levels;
+        const Wave w = wave(level);
         const RayRec* rays = (level == 0) ? nullptr : I.rays[level & 1].p; RayRec* nextRays = I.rays[(level + 1) & 1].p;
         Hit* hitBuf = (level == 0) ? I.hits0.p : I.hits.p;
         const unsigned grid = (level == 0) ? gridFor(n0, 128) : persist;
         CK(cudaEventRecord(I.pev(evN), st)); evIdx.push_back(evN++);
-        if (generic) {
-          if (counters_ || (traceMode_ & 512)) k_trace<true, TF_ALL><<<grid, 128, 0, st>>>(I.ds, w, pm, b0, rays, hitBuf, I.ctr, nullptr, nullptr);
-          else k_trace<false, TF_ALL><<<grid, 128, 0, st>>>(I.ds, w, pm, b0, rays, hitBuf, I.ctr, nullptr, nullptr);
-          ++rs.kernelLaunches; dbg("k_trace generic", level);
-        } else {
-          if (I.shape == 0) k_trace<false, 0><<<grid, 128, 0, st>>>(I.ds, w, pm, b0, rays, hitBuf, I.ctr, nullptr, I.deferT.p);
-          else k_trace<false, TF_LITERAL1><<<grid, 128, 0, st>>>(I.ds, w, pm, b0, rays, hitBuf, I.ctr, nullptr, I.deferT.p);
-          dbg("k_trace lean", level);
-          k_trace<false, TF_ALL><<<fixGrid, 128, 0, st>>>(I.ds, w, pm, b0, rays, hitBuf, I.ctr, I.deferT.p, nullptr);
-          rs.kernelLaunches += 2; dbg("k_trace fix-up", level);
-        }
+        pass("k_trace", level, traceLean, traceAll, I.deferT.p, grid, I.ds, w, pm, b0, rays, hitBuf, I.ctr);
         CK(cudaEventRecord(I.pev(evN++), st));
         if (level == 0) k_shade<true><<<grid, 128, 0, st>>>(I.ds, w, pm, b0, rays, hitBuf, I.surf.p, I.nodes.p, nextRays, I.ctr);
         else k_shade<false><<<grid, 128, 0, st>>>(I.ds, w, pm, b0, rays, hitBuf, I.surf.p, I.nodes.p, nextRays, I.ctr);
-        ++rs.kernelLaunches; dbg("k_shade", level);
-        if (I.ds.numPhotons > 0) { k_photon_gather_lane<<<grid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr); k_photon_gather_warp<<<grid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr); rs.kernelLaunches += 2; dbg("k_photon_gather", level); }
-        CK(cudaEventRecord(I.pev(evN++), st));
-        if (generic) {
-          if (counters_ || (traceMode_ & 256)) k_light<true, TF_ALL><<<grid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr, nullptr, nullptr);
-          else k_light<false, TF_ALL><<<grid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr, nullptr, nullptr);
-          ++rs.kernelLaunches; dbg("k_light generic", level);
-        } else {
-          if (I.shape == 0) k_light<false, 0><<<grid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr, nullptr, I.deferL.p);
-          else k_light<false, TF_LITERAL1><<<grid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr, nullptr, I.deferL.p);
-          dbg("k_light lean", level);
-          k_light<false, TF_ALL><<<fixGrid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr, I.deferL.p, nullptr);
-          rs.kernelLaunches += 2; dbg("k_light fix-up", level);
+        launched("k_shade", level);
+        if (I.ds.numPhotons > 0) {
+          k_photon_gather_lane<<<grid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr); launched("k_photon_gather_lane", level);
+          k_photon_gather_warp<<<grid, 128, 0, st>>>(I.ds, w, I.surf.p, I.nodes.p, I.ctr); launched("k_photon_gather_warp", level);
         }
         CK(cudaEventRecord(I.pev(evN++), st));
+        pass("k_light", level, lightLean, lightAll, I.deferL.p, grid, I.ds, w, I.surf.p, I.nodes.p, I.ctr);
+        CK(cudaEventRecord(I.pev(evN++), st));
       }
-      for (int level = levels - 1; level >= 1; --level) {
-        Wave w; w.n0 = n0; w.rayCap = rayCap; w.nodeCap = nodeCap; w.level = level; w.launchedLevels = levels;
-        k_resolve<<<persist, 256, 0, st>>>(w, I.nodes.p, I.ctr); ++rs.kernelLaunches; dbg("k_resolve", level);
-      }
-      k_finish<<<gridFor(nPix, 256), 256, 0, st>>>(I.ds, pm, b0, nPix, I.nodes.p, I.hits0.p, out); ++rs.kernelLaunches; dbg("k_finish", 0);
+      for (int level = levels - 1; level >= 1; --level) { k_resolve<<<persist, 256, 0, st>>>(wave(level), I.nodes.p, I.ctr); launched("k_resolve", level); }
+      k_finish<<<gridFor(nPix, 256), 256, 0, st>>>(I.ds, pm, b0, nPix, I.nodes.p, I.hits0.p, out); launched("k_finish", 0);
     }
     CK(cudaEventRecord(I.pev(evN), st)); const size_t evEnd = evN++;
     CK(cudaMemcpyAsync(I.ctrHost, I.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, st));
-    unsigned int devErr = 0; CK(cudaMemcpyFromSymbolAsync(&devErr, g_devError, sizeof(devErr), 0, cudaMemcpyDeviceToHost, st));
+    unsigned int devErr = 0; devErrorFetch(&devErr, st);
     CK(cudaStreamSynchronize(st)); CK(cudaGetLastError()); ++rs.hostSyncs;
-    if (devErr & 1u) throw std::runtime_error(kDevIncomplete);
-    if (devErr & 4u) { if (levels >= fullDepth) throw std::runtime_error("internal error: bounce depth beyond numRays"); levels = fullDepth; ++retries; continue; }
-    if (devErr & 2u) { if (capFactor >= 64.0) throw std::runtime_error("internal error: secondary-ray queues overflow at their upper bound"); capFactor = std::min(64.0, capFactor * 2); if (capFactor > 2.0) batchRays = std::max<long long>(65536, batchRays / 2); ++retries; continue; }
+    throwIfIncomplete(devErr);
+    if (devErr & DEV_ERR_DEPTH) { if (levels >= fullDepth) throw std::runtime_error("internal error: bounce depth beyond numRays"); levels = fullDepth; ++retries; continue; }
+    if (devErr & DEV_ERR_QUEUE) { if (capFactor >= 64.0) throw std::runtime_error("internal error: secondary-ray queues overflow at their upper bound"); capFactor = std::min(64.0, capFactor * 2); if (capFactor > 2.0) batchRays = std::max<long long>(65536, batchRays / 2); ++retries; continue; }
     float msT = 0, msS = 0, msL = 0, tot = 0;
     for (size_t k : evIdx) { float a, b2, c; CK(cudaEventElapsedTime(&a, I.evPool[k], I.evPool[k + 1])); CK(cudaEventElapsedTime(&b2, I.evPool[k + 1], I.evPool[k + 2])); CK(cudaEventElapsedTime(&c, I.evPool[k + 2], I.evPool[k + 3])); msT += a; msS += b2; msL += c; }
     CK(cudaEventElapsedTime(&tot, I.evPool[evStart], I.evPool[evEnd]));
@@ -752,10 +730,6 @@ void Renderer::renderToHost(int32_t* argbHost, int32_t* hitPrimHost, int32_t* hi
   if (argbHost) { I.oArgb.ensure(np, st); o.argb = I.oArgb.p; } if (hitPrimHost) { I.oPrim.ensure(np, st); o.hitPrim = I.oPrim.p; }
   if (hitInstHost) { I.oInst.ensure(np, st); o.hitInst = I.oInst.p; } if (rgbHost) { I.oRgb.ensure(3 * np, st); o.rgb = I.oRgb.p; } if (tHost) { I.oT.ensure(np, st); o.t = I.oT.p; }
   renderRange(0, (long long)np, o, stats);
-  if (const char* dump = getenv("DRT_DUMP_HITS")) {   // debugging aid
-    std::vector<Hit> hh(np * (g_.spp < 1 ? 1 : g_.spp)); CK(cudaMemcpy(hh.data(), I.hits0.p, hh.size() * sizeof(Hit), cudaMemcpyDeviceToHost));
-    FILE* f = fopen(dump, "wb"); if (f) { fwrite(hh.data(), sizeof(Hit), hh.size(), f); fclose(f); }
-  }
   if (argbHost) CK(cudaMemcpyAsync(argbHost, o.argb, np * 4, cudaMemcpyDeviceToHost, st));
   if (hitPrimHost) CK(cudaMemcpyAsync(hitPrimHost, o.hitPrim, np * 4, cudaMemcpyDeviceToHost, st));
   if (hitInstHost) CK(cudaMemcpyAsync(hitInstHost, o.hitInst, np * 4, cudaMemcpyDeviceToHost, st));
@@ -786,7 +760,7 @@ void Renderer::emitPhotonsRange(long long i0, long long i1, RenderStats* stats) 
 long long Renderer::exportPhotonsDevice(double* dst6Dev, long long cap) {
   CK(cudaSetDevice(device_)); Impl& I = *impl_; cudaStream_t st = (cudaStream_t)stream_;
   long long n = std::min<long long>((long long)I.photons.count, cap);
-  if (n > 0 && dst6Dev) { CK(cudaMemcpyAsync(dst6Dev, I.photons.rec, (size_t)n * sizeof(PhotonRec), cudaMemcpyDeviceToDevice, st)); CK(cudaStreamSynchronize(st)); }
+  if (n > 0 && dst6Dev) { CK(cudaMemcpyAsync(dst6Dev, I.photons.rec.p, (size_t)n * sizeof(PhotonRec), cudaMemcpyDeviceToDevice, st)); CK(cudaStreamSynchronize(st)); }
   return (long long)I.photons.count;
 }
 void Renderer::buildPhotonsFromDevice(const double* src6Dev, long long n, RenderStats* stats) {
@@ -796,15 +770,25 @@ void Renderer::buildPhotonsFromDevice(const double* src6Dev, long long n, Render
   I.photons.setRecords(reinterpret_cast<const PhotonRec*>(src6Dev), (unsigned long long)n, st); I.photons.buildGrid(I.ds, st);
   if (stats) { stats->kernelLaunches = g_kernelLaunches - l0; stats->photonsStored = I.photons.count; stats->msOther = I.photons.msBuild; stats->msTotal = I.photons.msBuild; }
 }
+// Parity probes: n items, each input and output `w` doubles per item (at most two of each), through the renderer's grow-only probe buffers.
+// Resets the device error word, uploads the inputs, zeroes the outputs, runs launch(in, out), downloads the outputs, synchronises once and
+// fails the call if a device search ran beyond its capacity.
+struct ProbeIn { const void* host; size_t w; };
+struct ProbeOut { void* host; size_t w; };
+template <class L> static void probe(Renderer::Impl& I, cudaStream_t st, long long n, std::initializer_list<ProbeIn> ins, std::initializer_list<ProbeOut> outs, L launch) {
+  double* in[2] = {nullptr, nullptr}; double* out[2] = {nullptr, nullptr}; int k = 0;
+  devErrorReset(st);
+  for (const ProbeIn& a : ins) { in[k] = I.probeIn[k].ensure(n * a.w, st); CK(cudaMemcpyAsync(in[k], a.host, n * a.w * 8, cudaMemcpyHostToDevice, st)); ++k; }
+  k = 0; for (const ProbeOut& a : outs) { out[k] = I.probeOut[k].ensure(n * a.w, st); CK(cudaMemsetAsync(out[k], 0, n * a.w * 8, st)); ++k; }
+  launch(in, out);
+  k = 0; for (const ProbeOut& a : outs) { CK(cudaMemcpyAsync(a.host, out[k], n * a.w * 8, cudaMemcpyDeviceToHost, st)); ++k; }
+  unsigned int e = 0; devErrorFetch(&e, st);
+  CK(cudaStreamSynchronize(st)); CK(cudaGetLastError()); throwIfIncomplete(e);
+}
 void Renderer::probePhotons(long long n, const double* ptsHost, double* out5Host) {
   CK(cudaSetDevice(device_)); Impl& I = *impl_; cudaStream_t st = (cudaStream_t)stream_;
-  devErrorReset(st);
-  if (g_.photonKind != 0 && !I.photons.built) I.photons.emitAndBuild(I.ds, I.ctr, I.ctrHost, st);
-  double *a, *b; CK(cudaMalloc(&a, n * 24)); CK(cudaMalloc(&b, n * 40));
-  CK(cudaMemcpyAsync(a, ptsHost, n * 24, cudaMemcpyHostToDevice, st)); CK(cudaMemsetAsync(b, 0, n * 40, st));
-  if (I.ds.numPhotons > 0) k_photon_probe<<<gridFor(n, 128), 128, 0, st>>>(I.ds, n, a, b);
-  CK(cudaMemcpyAsync(out5Host, b, n * 40, cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st)); CK(cudaGetLastError());
-  cudaFree(a); cudaFree(b); devErrorCheck(st);
+  if (g_.photonKind != 0 && !I.photons.built) { devErrorReset(st); I.photons.emitAndBuild(I.ds, I.ctr, I.ctrHost, st); devErrorCheck(st); }
+  probe(I, st, n, {{ptsHost, 3}}, {{out5Host, 5}}, [&](double* const* in, double* const* o) { if (I.ds.numPhotons > 0) k_photon_probe<<<gridFor(n, 128), 128, 0, st>>>(I.ds, n, in[0], o[0]); });
 }
 // parity probe: the resident packed triangles of fast BVH `fastIndex` and, in DRT_ACCEL_LBVH mode, its GPU-built nodes
 long long Renderer::probeFastBvh(int fastIndex, std::vector<FTri>& tris, std::vector<FNode>& nodes, int32_t info[4]) {
@@ -821,25 +805,15 @@ void Renderer::accelInfo(double out[4]) const { out[0] = impl_->lbvhMs; out[1] =
 long long Renderer::getPhotons(double* out6Host, long long cap) { CK(cudaSetDevice(device_)); return impl_->photons.download(out6Host, cap, (cudaStream_t)stream_); }
 
 void Renderer::traceRays(long long n, const double* orgHost, const double* dirHost, int32_t* idsHost, double* tHost) {
-  CK(cudaSetDevice(device_)); cudaStream_t st = (cudaStream_t)stream_;
-  devErrorReset(st);
-  double *o, *d, *t; int32_t* ids; CK(cudaMalloc(&o, n * 24)); CK(cudaMalloc(&d, n * 24)); CK(cudaMalloc(&t, n * 8)); CK(cudaMalloc(&ids, n * 8));
-  CK(cudaMemcpyAsync(o, orgHost, n * 24, cudaMemcpyHostToDevice, st)); CK(cudaMemcpyAsync(d, dirHost, n * 24, cudaMemcpyHostToDevice, st));
-  if (counters_) k_trace_explicit<true><<<gridFor(n, 128), 128, 0, st>>>(impl_->ds, n, o, d, ids, t);
-  else k_trace_explicit<false><<<gridFor(n, 128), 128, 0, st>>>(impl_->ds, n, o, d, ids, t);
-  CK(cudaMemcpyAsync(idsHost, ids, n * 8, cudaMemcpyDeviceToHost, st)); CK(cudaMemcpyAsync(tHost, t, n * 8, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st)); CK(cudaGetLastError()); devErrorCheck(st);
-  cudaFree(o); cudaFree(d); cudaFree(t); cudaFree(ids);
+  CK(cudaSetDevice(device_)); cudaStream_t st = (cudaStream_t)stream_; const auto k = counters_ ? &k_trace_explicit<true> : &k_trace_explicit<false>;
+  probe(*impl_, st, n, {{orgHost, 3}, {dirHost, 3}}, {{idsHost, 1}, {tHost, 1}},       // ids: two int32 per ray
+        [&](double* const* in, double* const* o) { k<<<gridFor(n, 128), 128, 0, st>>>(impl_->ds, n, in[0], in[1], reinterpret_cast<int32_t*>(o[0]), o[1]); });
 }
 void Renderer::evalTexture(int shaderIdx, long long n, const double* hitLocHost, const double* fwdLocHost, double* outHost) {
   CK(cudaSetDevice(device_)); cudaStream_t st = (cudaStream_t)stream_;
-  double *a, *b, *c; CK(cudaMalloc(&a, n * 24)); CK(cudaMalloc(&b, n * 24)); CK(cudaMalloc(&c, n * 24));
-  CK(cudaMemcpyAsync(a, hitLocHost, n * 24, cudaMemcpyHostToDevice, st)); CK(cudaMemcpyAsync(b, fwdLocHost, n * 24, cudaMemcpyHostToDevice, st));
-  k_eval_texture<<<gridFor(n, 128), 128, 0, st>>>(impl_->ds, shaderIdx, n, a, b, c);
-  CK(cudaMemcpyAsync(outHost, c, n * 24, cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st)); CK(cudaGetLastError());
-  cudaFree(a); cudaFree(b); cudaFree(c);
+  probe(*impl_, st, n, {{hitLocHost, 3}, {fwdLocHost, 3}}, {{outHost, 3}},
+        [&](double* const* in, double* const* o) { k_eval_texture<<<gridFor(n, 128), 128, 0, st>>>(impl_->ds, shaderIdx, n, in[0], in[1], o[0]); });
 }
-
 
 // ---------------------------------------------------------------------------------------------------------------
 // Multi-GPU inside the library (SURVEY 8(b)/(e)): one context per GPU, the frame split in interleaved row chunks, photon emission split by
@@ -918,18 +892,17 @@ void Renderer::renderDistributed(int32_t* argbHostRank0, int32_t* argbDevRank0, 
     long long pr[2]; distPhotonRange(g_.numPhotonsCast, world, rank, pr); const long long i0 = pr[0], i1 = pr[1];
     devErrorReset(st); I.photons.emitRange(I.ds, i0, i1, I.ctr, I.ctrHost, st); devErrorCheck(st);
     if (world > 1) {
-      // (exchange buffers are grow-only members: a cudaMalloc / cudaFree pair per frame costs tens to hundreds of ms on this driver)
-      unsigned long long* cnt = I.xCnt.get<unsigned long long>((size_t)world + 1);
+      unsigned long long* cnt = I.xCnt.ensure((size_t)world + 1, st);
       k_store_u64<<<1, 1, 0, st>>>(cnt + world, I.photons.count);
       NK(nccl().AllGather(cnt + world, cnt, 1, ncclUint64, (ncclComm_t)comm_, st));
       std::vector<unsigned long long> counts(world); CK(cudaMemcpyAsync(counts.data(), cnt, sizeof(unsigned long long) * world, cudaMemcpyDeviceToHost, st)); CK(cudaStreamSynchronize(st));
       unsigned long long mx = 1, total = 0, segs = I.photons.segments; for (auto c : counts) { mx = std::max(mx, c); total += c; }
-      PhotonRec* mine = I.xMine.get<PhotonRec>((size_t)mx); PhotonRec* all = I.xAll.get<PhotonRec>((size_t)mx * world);
+      PhotonRec* mine = I.xMine.ensure((size_t)mx, st); PhotonRec* all = I.xAll.ensure((size_t)mx * world, st);
       CK(cudaMemsetAsync(mine, 0, mx * sizeof(PhotonRec), st));
-      if (I.photons.count) CK(cudaMemcpyAsync(mine, I.photons.rec, I.photons.count * sizeof(PhotonRec), cudaMemcpyDeviceToDevice, st));
+      if (I.photons.count) CK(cudaMemcpyAsync(mine, I.photons.rec.p, I.photons.count * sizeof(PhotonRec), cudaMemcpyDeviceToDevice, st));
       NK(nccl().AllGather(mine, all, mx * sizeof(PhotonRec), ncclChar, (ncclComm_t)comm_, st));
-      I.photons.built = false; I.photons.emitted = true; I.photons.count = 0; I.photons.ensureRec((size_t)total, st);
-      unsigned long long at = 0; for (int r = 0; r < world; ++r) { if (counts[r]) CK(cudaMemcpyAsync(I.photons.rec + at, all + (size_t)r * mx, counts[r] * sizeof(PhotonRec), cudaMemcpyDeviceToDevice, st)); at += counts[r]; }
+      I.photons.built = false; I.photons.emitted = true; I.photons.count = 0; I.photons.rec.ensure((size_t)total, st);
+      unsigned long long at = 0; for (int r = 0; r < world; ++r) { if (counts[r]) CK(cudaMemcpyAsync(I.photons.rec.p + at, all + (size_t)r * mx, counts[r] * sizeof(PhotonRec), cudaMemcpyDeviceToDevice, st)); at += counts[r]; }
       I.photons.count = total; I.photons.segments = segs; CK(cudaStreamSynchronize(st));
     }
     I.photons.buildGrid(I.ds, st);

@@ -1,6 +1,7 @@
 // Host-side handle of the wavefront renderer (device memory owner + kernel launcher).
 #pragma once
 #include "host_scene.h"
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -28,7 +29,7 @@ class Renderer {
   bool orderBvh(int n, const double* keys3n, int32_t* ord, double* msDevice);   // device twin of HostScene::refOrderHost (csrc/refbvh.cuh)
   void setBatchRays(long long n) { batchRays_ = n; }
   void setCounters(bool on) { counters_ = on; }
-  void setTraceMode(int m) { traceMode_ = m; }
+  void setAccelMode(int m) { accelMode_ = m; }              // DRT_ACCEL_*: takes effect at the next upload
   // render pixels [pix0, pix1) (row-major pixel indices) into the device buffers of `out` (indexed by absolute pixel)
   void renderRange(long long pix0, long long pix1, const RenderOutputs& out, RenderStats* stats);
   void renderChunks(long long pix0, long long pix1, int world, int rank, int chunkRows, const RenderOutputs& out, RenderStats* stats);
@@ -66,13 +67,13 @@ class Renderer {
   struct Impl;
 
  private:
-  Impl* impl_;
+  std::unique_ptr<Impl> impl_;
   FGlobals g_;
   int device_;
   void* stream_;
   long long batchRays_ = 8ll << 20;
   bool counters_ = false;
-  int traceMode_ = 0;
+  int accelMode_ = 0;
   bool keepDepthHint_ = false;
   void* comm_ = nullptr; int world_ = 1, rank_ = 0;
 };

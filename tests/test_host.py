@@ -174,6 +174,16 @@ def test_unknown_accel_mode_is_rejected(drt):
     ctx.close()
 
 
+def test_finalize_rejects_unknown_accel_modes(drt):
+    """drt_scene_finalize takes exactly DRT_ACCEL_REFERENCE (0), DRT_ACCEL_REFERENCE_FAST (1) and DRT_ACCEL_LBVH (2): no value outside
+    them, flag bits included, is accepted."""
+    ctx = drt.Context(device=-1)
+    for m in (3, 4, -1, 256, 512, 257):
+        with pytest.raises(drt.DrtError, match="unknown acceleration mode"):
+            drt.Scene.from_cli(ctx, "t01.cli", accel=m)
+    ctx.close()
+
+
 def test_vertex_fast_path_keeps_the_token_rules(drt):
     """`vertex` lines are parsed in place (no token list); the rules must stay those of PApplet.splitTokens(line, " ") + Java number parsing as the
     general path applies them: any number of blanks, trailing tokens ignored, f / d suffixes accepted, a missing or malformed number is an error
