@@ -12,6 +12,8 @@ interface for the path:
     `write` -> myScene.draw()  (java :86-93)        Scene.draw()  -> ARGB ints == PImage.pixels
     PImage.save                                     Scene.save(path)
 
+Scene.intersect / Scene.occluded answer closest-hit and occlusion queries for the caller's own rays on CUDA tensors.
+
 There is no CPU fallback: without the built library or without a CUDA device every render call raises.
 """
-from .host import Context, Scene, RTFileReader, DrtError, lib_path, load_library, refine_steps, refine_pass, SCENES_DIR, ACCEL_REFERENCE, ACCEL_REFERENCE_FAST, ACCEL_LBVH  # noqa: F401
+from .host import Context, Scene, Stats, RTFileReader, DrtError, lib_path, load_library, refine_steps, refine_pass, SCENES_DIR, ACCEL_REFERENCE, ACCEL_REFERENCE_FAST, ACCEL_LBVH  # noqa: F401

@@ -7,6 +7,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <memory>
 #include <stdexcept>
 #include <zlib.h>
@@ -189,6 +190,23 @@ int drt_save_png(const char* path, const int32_t* argb, int32_t cols, int32_t ro
 }
 
 int drt_trace_rays(drt_ctx* ctx, int64_t n, const double* org, const double* dir, int32_t* ids2, double* t) { NEED_DEV(ctx) GUARD(ctx, { if (!ctx->finalized) throw std::runtime_error("scene not finalized"); ctx->renderer->traceRays(n, org, dir, ids2, t); }, DRT_ERR_CUDA) }
+// shared argument checks of the ray queries: device, finalized scene, n >= 0, required pointers present when there are rays
+static int queryArgs(drt_ctx* ctx, int64_t n, std::initializer_list<const void*> required) {
+  if (!ctx) return DRT_ERR_BAD_ARG;
+  NEED_DEV(ctx)
+  if (!ctx->finalized) { ctx->err = "scene not finalized"; return DRT_ERR_STATE; }
+  if (n < 0) { ctx->err = "negative ray count"; return DRT_ERR_BAD_ARG; }
+  if (n > 0) for (const void* p : required) if (!p) { ctx->err = "a required ray or output buffer is NULL"; return DRT_ERR_BAD_ARG; }
+  return DRT_OK;
+}
+int drt_query_closest(drt_ctx* ctx, int64_t n, const double* org3, const double* dir3, const double* tmax, int32_t* ids2, double* t, double* pos3, double* nrm3, drt_stats* stats) {
+  if (const int rc = queryArgs(ctx, n, {org3, dir3, ids2, t})) return rc;
+  GUARD(ctx, { RenderStats rs; ctx->renderer->queryClosest(n, org3, dir3, tmax, ids2, t, pos3, nrm3, &rs); toStats(rs, stats); }, DRT_ERR_CUDA)
+}
+int drt_query_occluded(drt_ctx* ctx, int64_t n, const double* org3, const double* dir3, const double* dist, uint8_t* occluded, drt_stats* stats) {
+  if (const int rc = queryArgs(ctx, n, {org3, dir3, dist, occluded})) return rc;
+  GUARD(ctx, { RenderStats rs; ctx->renderer->queryOccluded(n, org3, dir3, dist, occluded, &rs); toStats(rs, stats); }, DRT_ERR_CUDA)
+}
 int drt_eval_texture(drt_ctx* ctx, int32_t serial, int64_t n, const double* hl, const double* fl, double* rgb) {
   NEED_DEV(ctx) GUARD(ctx, { if (!ctx->finalized) throw std::runtime_error("scene not finalized"); if (serial < 0 || serial >= (int)ctx->scene->shaderOfSerial.size()) throw std::runtime_error("no such shader"); ctx->renderer->evalTexture(ctx->scene->shaderOfSerial[serial], n, hl, fl ? fl : hl, rgb); }, DRT_ERR_CUDA)
 }

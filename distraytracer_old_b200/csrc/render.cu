@@ -441,6 +441,73 @@ __global__ void k_nodes32(const FNode* __restrict__ in, long long n, FNode32* __
   m.left = a.left; m.right = a.right; m.triL = a.triL; m.triR = a.triR; out[i] = m;
 }
 
+// caller ray queries (drt_query_closest / drt_query_occluded) -----------------------------------------------------
+// One thread = one caller ray (FP64 origin and direction, 3 doubles each, ray time 0).  F / work / deferOut as in k_trace: the scene's lean
+// variant defers what it cannot serve to `deferOut` (count in Counters::deferTrace[0] / deferLight[0]), the generic variant serves everything
+// and is the fix-up pass over that list.  A ray is traced only if origin and direction are finite and the direction's FP64 length is finite
+// and nonzero; any other ray is a miss / not occluded.
+__device__ __forceinline__ bool queryRay(const double* __restrict__ org, const double* __restrict__ dir, long long i, Ray& ray) {
+  const D3 o = d3(org[3 * i], org[3 * i + 1], org[3 * i + 2]), d = d3(dir[3 * i], dir[3 * i + 1], dir[3 * i + 2]);
+  const double m = mag3(d);
+  if (!(isfinite(o.x) && isfinite(o.y) && isfinite(o.z) && isfinite(d.x) && isfinite(d.y) && isfinite(d.z) && isfinite(m) && m > 0)) return false;
+  ray = makeRay(o, norm3(d)); return true;
+}
+// closest hit, reported as a miss unless t < tmax[i] (tmax == null: +inf).  The search itself is the unbounded one.  pos / nrm (optional): the
+// world hit point and unit normal k_shade shades with (0 on a miss)
+template <int F>
+__global__ void __launch_bounds__(128, (F == TF_ALL) ? DRT_TRACE_MINBLOCKS : (F == TF_LITERAL1) ? DRT_L1_MINBLOCKS : DRT_LTRACE_MINBLOCKS)
+k_query_closest(const __grid_constant__ DScene S, long long nRays, const double* __restrict__ org, const double* __restrict__ dir, const double* __restrict__ tmax,
+                int32_t* __restrict__ ids, double* __restrict__ tOut, double* __restrict__ pos, double* __restrict__ nrm, Counters* ctr, const uint32_t* __restrict__ work, uint32_t* __restrict__ deferOut) {
+  const long long n = work ? (long long)ctr->deferTrace[0] : nRays;
+  if (work && n > 0 && blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&ctr->deferredTotal, (unsigned long long)n);
+  for (long long base = (long long)blockIdx.x * blockDim.x; base < n; base += (long long)gridDim.x * blockDim.x) {
+    long long i = base + threadIdx.x; bool defer = false;
+    if (i < n) {
+      if (work) i = work[i];
+      Hit h; hitReset(h); Ray ray;
+      if (queryRay(org, dir, i, ray)) {
+        const int got = closestHitT<F>(S, ray, 0.0, h, nullptr);
+        if (F != TF_ALL && got < 0) defer = true;
+      }
+      if (!defer) {
+        const bool hit = h.prim >= 0 && (!tmax || h.t < tmax[i]);
+        ids[2 * i] = hit ? S.prims[h.prim].serial : -1; ids[2 * i + 1] = hit ? h.inst : -1; tOut[i] = hit ? h.t : 0;
+        if (pos || nrm) {
+          D3 p = d3(0, 0, 0), q = p;
+          if (hit) {
+            const FPrim P = S.prims[h.prim]; const FXform& X = S.xforms[h.hitXform];
+            p = xfPoint(X.m, h.loc); q = norm3(xfVector(X.adj, primNormal(S, P, h.loc, h.arg0, h.arg1, h.state)));
+          }
+          if (pos) { pos[3 * i] = p.x; pos[3 * i + 1] = p.y; pos[3 * i + 2] = p.z; }
+          if (nrm) { nrm[3 * i] = q.x; nrm[3 * i + 1] = q.y; nrm[3 * i + 2] = q.z; }
+        }
+      }
+    }
+    if (F != TF_ALL) deferAppend(defer, (uint32_t)i, &ctr->deferTrace[0], deferOut);
+  }
+}
+// occlusion: the renderer's shadow test (anyHitT: something hit with (dist - t) > DRT_EPS).  dist may be +inf; a NaN dist is not occluded
+template <int F>
+__global__ void __launch_bounds__(128, (F == TF_ALL) ? DRT_LIGHT_MINBLOCKS : (F == TF_LITERAL1) ? DRT_L1_MINBLOCKS : DRT_LLIGHT_MINBLOCKS)
+k_query_any(const __grid_constant__ DScene S, long long nRays, const double* __restrict__ org, const double* __restrict__ dir, const double* __restrict__ dist,
+            uint8_t* __restrict__ occluded, Counters* ctr, const uint32_t* __restrict__ work, uint32_t* __restrict__ deferOut) {
+  const long long n = work ? (long long)ctr->deferLight[0] : nRays;
+  if (work && n > 0 && blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&ctr->deferredTotal, (unsigned long long)n);
+  for (long long base = (long long)blockIdx.x * blockDim.x; base < n; base += (long long)gridDim.x * blockDim.x) {
+    long long i = base + threadIdx.x; bool defer = false;
+    if (i < n) {
+      if (work) i = work[i];
+      const double d = dist[i]; int got = 0; Ray ray;
+      if (d == d && queryRay(org, dir, i, ray)) {
+        got = anyHitT<F>(S, ray, 0.0, d, nullptr);
+        if (F != TF_ALL && got < 0) defer = true;
+      }
+      if (!defer) occluded[i] = got > 0 ? 1 : 0;
+    }
+    if (F != TF_ALL) deferAppend(defer, (uint32_t)i, &ctr->deferLight[0], deferOut);
+  }
+}
+
 // parity helpers ------------------------------------------------------------------------------------------------
 template <bool COUNT>
 __global__ void k_trace_explicit(const __grid_constant__ DScene S, long long n, const double* __restrict__ org, const double* __restrict__ dir, int32_t* __restrict__ ids, double* __restrict__ tOut) {
@@ -618,6 +685,26 @@ void Renderer::upload(const HostScene& hs, bool sameScene) {
 
 static inline unsigned gridFor(long long n, int block) { return (unsigned)((n + block - 1) / block); }
 
+// Kernel launches of one call on `st`: counts them into *launches and, with DRT_SYNC_DEBUG set, synchronises after each one (debugging aid:
+// locate a faulting kernel).  operator(): one closest-hit or light pass -- the generic kernel alone (lean == null), or the lean kernel, which
+// appends what it defers to `list`, followed by the generic kernel as the fix-up pass over that list.  args: the kernels' arguments before
+// (work, deferOut).
+struct PassLauncher {
+  cudaStream_t st; unsigned fixGrid; unsigned long long* launches;
+  void launched(const char* what, int level, const char* variant = "") const {
+    ++*launches;
+    static const bool syncDebug = getenv("DRT_SYNC_DEBUG") != nullptr;
+    if (!syncDebug) return;
+    cudaError_t e = cudaStreamSynchronize(st); if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) throw std::runtime_error(std::string("DRT_SYNC_DEBUG: ") + what + variant + " level " + std::to_string(level) + ": " + cudaGetErrorString(e));
+  }
+  template <class K, class... A> void operator()(const char* what, int level, K lean, K all, uint32_t* list, unsigned grid, A... args) const {
+    if (!lean) { all<<<grid, 128, 0, st>>>(args..., nullptr, nullptr); launched(what, level, " generic"); return; }
+    lean<<<grid, 128, 0, st>>>(args..., nullptr, list); launched(what, level, " lean");
+    all<<<fixGrid, 128, 0, st>>>(args..., list, nullptr); launched(what, level, " fix-up");
+  }
+};
+
 void Renderer::renderRange(long long pix0, long long pix1, const RenderOutputs& out, RenderStats* stats) { renderChunks(pix0, pix1, 1, 0, 0, out, stats); }
 
 // world > 1: compact pixel p of this rank maps to interleaved row chunks (chunkRows rows each, chunk c of the rank = absolute chunk c*world+rank)
@@ -663,16 +750,9 @@ void Renderer::renderChunks(long long pix0, long long pix1, int world, int rank,
     const unsigned persist = (unsigned)std::min<long long>(gridFor(rayCap, 128), (long long)I.numSMs * 16), fixGrid = (unsigned)I.numSMs * 4;
     devErrorReset(st);
     CK(cudaMemsetAsync(I.ctr, 0, sizeof(Counters), st));
-    static const bool syncDebug = getenv("DRT_SYNC_DEBUG") != nullptr;      // debugging aid: locate a faulting kernel
-    auto launched = [&](const char* what, int level, const char* variant = "") { ++rs.kernelLaunches; if (!syncDebug) return;
-      cudaError_t e = cudaStreamSynchronize(st); if (e == cudaSuccess) e = cudaGetLastError();
-      if (e != cudaSuccess) throw std::runtime_error(std::string("DRT_SYNC_DEBUG: ") + what + variant + " level " + std::to_string(level) + ": " + cudaGetErrorString(e)); };
-    // one closest-hit or light pass of a level; `list` receives what the lean kernel defers.  args: the kernels' arguments before (work, deferOut)
-    auto pass = [&](const char* what, int level, auto lean, auto all, uint32_t* list, unsigned grid, auto... args) {
-      if (!lean) { all<<<grid, 128, 0, st>>>(args..., nullptr, nullptr); launched(what, level, " generic"); return; }
-      lean<<<grid, 128, 0, st>>>(args..., nullptr, list); launched(what, level, " lean");
-      all<<<fixGrid, 128, 0, st>>>(args..., list, nullptr); launched(what, level, " fix-up");
-    };
+    // one closest-hit or light pass of a level; `list` receives what the lean kernel defers
+    const PassLauncher pass{st, fixGrid, &rs.kernelLaunches};
+    auto launched = [&](const char* what, int level) { pass.launched(what, level); };
     size_t evN = 0; std::vector<size_t> evIdx;      // 4 events per (batch, level): before trace, after trace, after shade (+gather), after light
     CK(cudaEventRecord(I.pev(evN), st)); const size_t evStart = evN++;
     for (long long b0 = pix0; b0 < pix1; b0 += pixPerBatch) {
@@ -808,6 +888,50 @@ void Renderer::traceRays(long long n, const double* orgHost, const double* dirHo
   CK(cudaSetDevice(device_)); cudaStream_t st = (cudaStream_t)stream_; const auto k = counters_ ? &k_trace_explicit<true> : &k_trace_explicit<false>;
   probe(*impl_, st, n, {{orgHost, 3}, {dirHost, 3}}, {{idsHost, 1}, {tHost, 1}},       // ids: two int32 per ray
         [&](double* const* in, double* const* o) { k<<<gridFor(n, 128), 128, 0, st>>>(impl_->ds, n, in[0], in[1], reinterpret_cast<int32_t*>(o[0]), o[1]); });
+}
+// Caller rays against the uploaded scene, device arrays in and out.  The rays run through the scene's kernel variant (Impl::shape) with the
+// generic kernel as the fix-up pass, in launches of at most 2^31 - 1 rays (the deferral list holds 32-bit indices); one host sync at the end,
+// after which the device error word is checked.  Uses the renderer's counters and deferral list as scratch; the frame speculation (depth and
+// capacity hints) and the photon map are not touched.  launch(pass, lean, i0, m) queues the pass of rays [i0, i0 + m).
+template <class L> static void runQuery(Renderer::Impl& I, cudaStream_t st, long long n, DBuf<uint32_t>& list, bool lean, double RenderStats::*ms, RenderStats* stats, L launch) {
+  RenderStats rs; std::memset(&rs, 0, sizeof(rs));
+  if (n > 0) {
+    const long long per = std::min<long long>(n, INT32_MAX);
+    if (lean) list.ensure((size_t)per, st);
+    const PassLauncher pass{st, (unsigned)I.numSMs * 4, &rs.kernelLaunches};
+    devErrorReset(st);
+    CK(cudaMemsetAsync(I.ctr, 0, sizeof(Counters), st));
+    CK(cudaEventRecord(I.pev(0), st));
+    for (long long i0 = 0; i0 < n; i0 += per) {
+      if (i0 > 0) CK(cudaMemsetAsync(&I.ctr->levelCount, 0, sizeof(Counters) - offsetof(Counters, levelCount), st));
+      launch(pass, i0, std::min(per, n - i0));
+    }
+    CK(cudaEventRecord(I.pev(1), st));
+    CK(cudaMemcpyAsync(I.ctrHost, I.ctr, sizeof(Counters), cudaMemcpyDeviceToHost, st));
+    unsigned int e = 0; devErrorFetch(&e, st);
+    CK(cudaStreamSynchronize(st)); CK(cudaGetLastError()); ++rs.hostSyncs;
+    throwIfIncomplete(e);
+    float t = 0; CK(cudaEventElapsedTime(&t, I.pev(0), I.pev(1)));
+    rs.*ms = t; rs.msTotal = t; rs.deferred = I.ctrHost->deferredTotal;
+  }
+  if (stats) *stats = rs;
+}
+void Renderer::queryClosest(long long n, const double* org, const double* dir, const double* tmax, int32_t* ids, double* t, double* pos, double* nrm, RenderStats* stats) {
+  CK(cudaSetDevice(device_)); Impl& I = *impl_; cudaStream_t st = (cudaStream_t)stream_;
+  using K = decltype(&k_query_closest<TF_ALL>);
+  const K all = &k_query_closest<TF_ALL>, lean = I.shape == TF_ALL ? nullptr : I.shape == 0 ? &k_query_closest<0> : &k_query_closest<TF_LITERAL1>;
+  runQuery(I, st, n, I.deferT, lean != nullptr, &RenderStats::msTrace, stats, [&](const PassLauncher& pass, long long i0, long long m) {
+    pass("k_query_closest", 0, lean, all, I.deferT.p, gridFor(m, 128), I.ds, m, org + 3 * i0, dir + 3 * i0, tmax ? tmax + i0 : nullptr, ids + 2 * i0, t + i0,
+         pos ? pos + 3 * i0 : nullptr, nrm ? nrm + 3 * i0 : nullptr, I.ctr);
+  });
+}
+void Renderer::queryOccluded(long long n, const double* org, const double* dir, const double* dist, uint8_t* occluded, RenderStats* stats) {
+  CK(cudaSetDevice(device_)); Impl& I = *impl_; cudaStream_t st = (cudaStream_t)stream_;
+  using K = decltype(&k_query_any<TF_ALL>);
+  const K all = &k_query_any<TF_ALL>, lean = I.shape == TF_ALL ? nullptr : I.shape == 0 ? &k_query_any<0> : &k_query_any<TF_LITERAL1>;
+  runQuery(I, st, n, I.deferL, lean != nullptr, &RenderStats::msLight, stats, [&](const PassLauncher& pass, long long i0, long long m) {
+    pass("k_query_any", 0, lean, all, I.deferL.p, gridFor(m, 128), I.ds, m, org + 3 * i0, dir + 3 * i0, dist + i0, occluded + i0, I.ctr);
+  });
 }
 void Renderer::evalTexture(int shaderIdx, long long n, const double* hitLocHost, const double* fwdLocHost, double* outHost) {
   CK(cudaSetDevice(device_)); cudaStream_t st = (cudaStream_t)stream_;

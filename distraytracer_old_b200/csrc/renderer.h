@@ -37,6 +37,10 @@ class Renderer {
   void renderToHost(int32_t* argbHost, int32_t* hitPrimHost, int32_t* hitInstHost, double* rgbHost, double* tHost, RenderStats* stats);
   // explicit world-space rays (closest hit only) for parity tests: ids = {primSerial, instSerial} per ray
   void traceRays(long long n, const double* orgHost, const double* dirHost, int32_t* idsHost, double* tHost);
+  // caller rays in DEVICE memory (include/drt.h drt_query_closest / drt_query_occluded); every pointer is a device pointer, optional ones may
+  // be null (tmax: +inf; pos, nrm: not written).  Complete when the call returns; stats: launches, deferred rays, one host sync, event ms
+  void queryClosest(long long n, const double* org, const double* dir, const double* tmax, int32_t* ids, double* t, double* pos, double* nrm, RenderStats* stats);
+  void queryOccluded(long long n, const double* org, const double* dir, const double* dist, uint8_t* occluded, RenderStats* stats);
   void evalTexture(int shaderIdx, long long n, const double* hitLocHost, const double* fwdLocHost, double* outHost);
   void emitPhotons(RenderStats* stats);               // builds the photon map if the scene asks for one
   long long getPhotons(double* out6Host, long long cap);

@@ -1,5 +1,5 @@
-"""ctypes host over include/drt.h.  No torch types cross the boundary; torch is only used by callers that
-want device-resident outputs (multi-GPU tile gather)."""
+"""ctypes host over include/drt.h.  No torch types cross the boundary: the ray queries (Scene.intersect / Scene.occluded) take CUDA tensors
+and pass their device pointers; elsewhere torch is only used by callers that want device-resident outputs (multi-GPU tile gather)."""
 import ctypes as C
 import os
 
@@ -83,6 +83,8 @@ def load_library():
         "drt_render_device_chunks": (C.c_int, [vp, i32, i32, i32, vp, C.POINTER(Stats)]),
         "drt_save_png": (C.c_int, [C.c_char_p, vp, i32, i32]),
         "drt_trace_rays": (C.c_int, [vp, i64, vp, vp, vp, vp]),
+        "drt_query_closest": (C.c_int, [vp, i64, vp, vp, vp, vp, vp, vp, vp, C.POINTER(Stats)]),
+        "drt_query_occluded": (C.c_int, [vp, i64, vp, vp, vp, vp, C.POINTER(Stats)]),
         "drt_eval_texture": (C.c_int, [vp, i32, i64, vp, vp, vp]),
         "drt_dump_bvh": (i64, [vp, i32, vp, i64, vp]),
         "drt_obj_ctm": (C.c_int, [vp, i32, vp]),
@@ -111,7 +113,7 @@ def load_library():
 EXPORTS = ["drt_create", "drt_destroy", "drt_last_error", "drt_set_image_loader", "drt_set_texture_dir", "drt_scene_reset",
            "drt_scene_command", "drt_scene_load_cli", "drt_scene_override", "drt_scene_finalize", "drt_scene_reupload",
            "drt_scene_info", "drt_scene_counts", "drt_build_info", "drt_bvh_order", "drt_lbvh_probe", "drt_scene_refine", "drt_refine_steps", "drt_refine_pass", "drt_accel_info", "drt_emit_photons", "drt_render", "drt_render_aov", "drt_render_device", "drt_render_device_chunks", "drt_save_png",
-           "drt_trace_rays", "drt_eval_texture", "drt_dump_bvh", "drt_obj_ctm", "drt_sample_u01", "drt_get_photons",
+           "drt_trace_rays", "drt_query_closest", "drt_query_occluded", "drt_eval_texture", "drt_dump_bvh", "drt_obj_ctm", "drt_sample_u01", "drt_get_photons",
            "drt_emit_photons_range", "drt_photons_export_device", "drt_photons_build_device", "drt_photon_probe",
            "drt_comm_unique_id", "drt_comm_init", "drt_comm_destroy", "drt_render_distributed",
            "drt_dist_rank_pixels", "drt_dist_abs_pixel", "drt_dist_photon_range"]
@@ -359,6 +361,54 @@ class Scene:
         rc = self.L.drt_save_png(path.encode(), a.ctypes.data, a.shape[1], a.shape[0])
         if rc != 0:
             raise DrtError("drt_save_png failed")
+
+    # ---- ray queries on CUDA tensors (drt_query_closest / drt_query_occluded)
+    def _device_arrays(self, *specs):
+        """specs: (tensor, name, cols).  Each must be a float64 torch tensor of shape (n, cols) (cols None: (n,)), contiguous, and on this
+        context's CUDA device, with the same n: it is passed as is, never copied.  Form and device are checked in that order."""
+        import torch
+        for x, name, cols in specs:
+            if not isinstance(x, torch.Tensor):
+                raise ValueError("%s must be a torch.Tensor on cuda:%d, got %s" % (name, self.ctx.device, type(x).__name__))
+            if x.dtype != torch.float64:
+                raise ValueError("%s must be torch.float64, got %s" % (name, x.dtype))
+            if (x.dim() != 2 or x.shape[1] != cols) if cols else x.dim() != 1:
+                raise ValueError("%s must have shape %s, got %s" % (name, "(n, %d)" % cols if cols else "(n,)", tuple(x.shape)))
+            if not x.is_contiguous():
+                raise ValueError("%s must be contiguous" % name)
+            if x.shape[0] != specs[0][0].shape[0]:
+                raise ValueError("%s holds %d rows for %d rays" % (name, x.shape[0], specs[0][0].shape[0]))
+        for x, name, _ in specs:
+            if x.device.type != "cuda" or x.device.index != self.ctx.device:
+                raise ValueError("%s must be on cuda:%d (the context's device), got %s" % (name, self.ctx.device, x.device))
+        return specs[0][0].shape[0]
+
+    def intersect(self, org, dirs, tmax=None, frame=False, stats=None):
+        """Closest hit of n caller rays (CUDA float64 tensors (n, 3)): ids int32 (n, 2) = (primitive serial, instance serial), -1 on a miss,
+        and t float64 (n,), 0 on a miss; a hit counts only when t < tmax (float64 (n,), None = +inf).  frame=True also returns the world hit
+        point and unit normal the renderer shades with, (n, 3) each.  stats: a Stats to fill."""
+        import torch
+        n = self._device_arrays((org, "org", 3), (dirs, "dirs", 3), *([(tmax, "tmax", None)] if tmax is not None else []))
+        ids = torch.empty((n, 2), dtype=torch.int32, device=org.device)
+        t = torch.empty(n, dtype=torch.float64, device=org.device)
+        pos = torch.empty((n, 3), dtype=torch.float64, device=org.device) if frame else None
+        nrm = torch.empty((n, 3), dtype=torch.float64, device=org.device) if frame else None
+        torch.cuda.current_stream(org.device).synchronize()        # the library's stream does not wait on torch's
+        ptr = lambda a: a.data_ptr() if a is not None else None
+        st = stats if stats is not None else Stats()
+        self.ctx._ck(self.L.drt_query_closest(self.ctx.h, n, ptr(org), ptr(dirs), ptr(tmax), ptr(ids), ptr(t), ptr(pos), ptr(nrm), C.byref(st)))
+        return (ids, t, pos, nrm) if frame else (ids, t)
+
+    def occluded(self, org, dirs, dist, stats=None):
+        """Shadow test of n caller rays (CUDA float64 tensors (n, 3)) against distances dist (float64 (n,), +inf allowed): torch.bool (n,),
+        True when something is hit with dist - t > 1e-7 (the renderer's shadow rule).  stats: a Stats to fill."""
+        import torch
+        n = self._device_arrays((org, "org", 3), (dirs, "dirs", 3), (dist, "dist", None))
+        occ = torch.empty(n, dtype=torch.bool, device=org.device)          # one byte per ray, written 0 / 1 by the library
+        torch.cuda.current_stream(org.device).synchronize()
+        st = stats if stats is not None else Stats()
+        self.ctx._ck(self.L.drt_query_occluded(self.ctx.h, n, org.data_ptr(), dirs.data_ptr(), dist.data_ptr(), occ.data_ptr(), C.byref(st)))
+        return occ
 
     # ---- parity probes
     def trace_rays(self, org, dirs):

@@ -124,6 +124,27 @@ int drt_scene_refine(drt_ctx* ctx);
 int32_t drt_refine_steps(int32_t cols, int32_t rows, int32_t* steps16);
 int drt_refine_pass(const int32_t* argb_full, int32_t cols, int32_t rows, int32_t step, int32_t* argb_out);
 
+/* ---- ray queries: the caller's own rays against the finalized scene (visibility, ambient occlusion, picking, depth / normal buffers).
+ * Every pointer is DEVICE memory of the context's GPU; n rays, origin org3[3i..] and direction dir3[3i..] in FP64 world space (the direction
+ * is normalised on the device; it need not be unit length).  Ray time is 0: moving spheres are queried at their start position.  A ray whose
+ * origin or direction is not finite, or whose direction has a zero (or non-finite) FP64 length, is not traced: a miss / not occluded.
+ * The rays run through the same traversal, kernel variants and fix-up pass as the renderer's closest-hit and shadow rays, on the context's
+ * stream; the call returns when the outputs are complete (one host sync).  The caller makes its own producers of the inputs finish first.
+ * Returns DRT_ERR_NO_DEVICE on a host-only context, DRT_ERR_STATE before drt_scene_finalize, DRT_ERR_BAD_ARG for n < 0 or a required pointer
+ * that is NULL while n > 0; n == 0 does nothing.  stats (may be NULL): kernel_launches, rays_deferred (rays the lean kernel left to the generic
+ * one), host_syncs, ms_trace (closest) or ms_light (occlusion) and ms_total (CUDA events); every other field is 0.
+ *
+ * drt_query_closest: the closest hit, reported as a miss unless t < tmax[i] (tmax NULL = +inf; a NaN tmax is a miss).  ids2[2i] = primitive
+ * serial, ids2[2i+1] = instance serial (-1, -1 on a miss), t[i] (0 on a miss) -- the conventions of drt_trace_rays, whose ids and t these are
+ * bit for bit.  Optional pos3 / nrm3 (NULL: skipped): the world hit point and unit normal the renderer shades with (0 on a miss).  SURVEY Q6/Q7
+ * apply: for a mesh in a transformed BVH pos is the reference's CTM-applied-twice point, and through a scaled instance t is measured in the
+ * instance's direction units, so pos is not org + t * dir in general.
+ * drt_query_occluded: occluded[i] = 1 when something is hit with (dist[i] - t) > 1e-7 -- the renderer's shadow test (box rules and instance
+ * trees included) -- else 0.  dist may be +inf; a NaN dist is not occluded.
+ * No Java binding covers these entry points (device pointers). */
+int drt_query_closest(drt_ctx* ctx, int64_t n, const double* org3, const double* dir3, const double* tmax, int32_t* ids2, double* t, double* pos3, double* nrm3, drt_stats* stats);
+int drt_query_occluded(drt_ctx* ctx, int64_t n, const double* org3, const double* dir3, const double* dist, uint8_t* occluded, drt_stats* stats);
+
 /* ---- parity probes (used by tests; not needed by a host) ---- */
 int drt_trace_rays(drt_ctx* ctx, int64_t n, const double* org, const double* dir, int32_t* ids2, double* t);
 int drt_eval_texture(drt_ctx* ctx, int32_t shader_serial, int64_t n, const double* hit_loc, const double* fwd_loc, double* rgb);
