@@ -912,7 +912,6 @@ __device__ __forceinline__ int anyHitT(const DScene& S, Ray& ray, double time, d
   }
   return 0;
 }
-__device__ __forceinline__ bool anyHit(const DScene& S, Ray& ray, double time, double dist, TraceCounters* tc) { return anyHitT<TF_ALL>(S, ray, time, dist, tc) > 0; }
 
 
 }  // namespace drt

@@ -168,11 +168,33 @@ __device__ __forceinline__ double rayTime(const DScene& S, uint32_t stream, uint
 #ifndef DRT_L1_MINBLOCKS
 #define DRT_L1_MINBLOCKS 6           // lean variants for scenes with instanced meshes (F == TF_LITERAL1)
 #endif
+// __launch_bounds__ min-blocks of the closest-hit kernels (k_trace, k_query_closest) and the shadow-ray kernels (k_light, k_query_any)
+constexpr int traceMinBlocks(int F) { return (F == TF_ALL) ? DRT_TRACE_MINBLOCKS : (F == TF_LITERAL1) ? DRT_L1_MINBLOCKS : DRT_LTRACE_MINBLOCKS; }
+constexpr int lightMinBlocks(int F) { return (F == TF_ALL) ? DRT_LIGHT_MINBLOCKS : (F == TF_LITERAL1) ? DRT_L1_MINBLOCKS : DRT_LLIGHT_MINBLOCKS; }
+
+// The query kernels' loop over the rays of a launch (F: dev_isect.cuh).  Direct launch (work == null): rays [0, n).  Fix-up launch (the
+// generic kernel, work != null): the *deferCount rays listed in `work`, counted once into Counters::deferredTotal.  body(i) returns whether
+// ray i is deferred; a lean variant appends those, warp-collectively, to deferOut / *deferCount, which its fix-up launch reads.  The bodies
+// are always_inline lambdas (optimised on their own first, they spill more).  k_trace / k_light write this loop out: through it they ran slower.
+template <int F, class Body>
+__device__ __forceinline__ void rayLoop(long long n, const uint32_t* work, unsigned long long* deferCount, uint32_t* deferOut, Counters* ctr, Body body) {
+  if (work) n = (long long)*deferCount;
+  if (work && n > 0 && blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&ctr->deferredTotal, (unsigned long long)n);
+  for (long long base = (long long)blockIdx.x * blockDim.x; base < n; base += (long long)gridDim.x * blockDim.x) {
+    long long i = base + threadIdx.x; bool defer = false;
+    if (i < n) {
+      if (work) i = work[i];
+      defer = body(i);
+    }
+    if (F != TF_ALL) deferAppend(defer, (uint32_t)i, deferCount, deferOut);
+  }
+}
+
 // Closest-hit pass of one level.  F = compile-time feature set (dev_isect.cuh): the lean variants defer what they cannot serve to `deferOut`;
 // the generic variant (TF_ALL) serves everything and is also the fix-up pass over such a list (`work` != null: ray indices to trace).
 // rays == null: level 0, the primary ray is generated from the index.
 template <bool COUNT, int F>
-__global__ void __launch_bounds__(128, (F == TF_ALL) ? DRT_TRACE_MINBLOCKS : (F == TF_LITERAL1) ? DRT_L1_MINBLOCKS : DRT_LTRACE_MINBLOCKS)
+__global__ void __launch_bounds__(128, traceMinBlocks(F))
 k_trace(const __grid_constant__ DScene S, Wave w, PixMap pm, long long pix0, const RayRec* __restrict__ rays, Hit* __restrict__ hits, Counters* ctr, const uint32_t* __restrict__ work, uint32_t* __restrict__ deferOut) {
   const long long n = work ? (long long)ctr->deferTrace[w.level] : waveCount(w, ctr);
   if (w.level == 0 && !work && blockIdx.x == 0 && threadIdx.x == 0) ctr->levelCount[0] = (unsigned long long)w.n0;
@@ -334,7 +356,7 @@ __global__ void __launch_bounds__(128, DRT_SHADE_MINBLOCKS) k_shade(const __grid
 // across it at the 80-register cap, they were spilled to local memory and written back through L2 on every light.
 __device__ __forceinline__ D3 ldgD3(const double* p) { return d3(__ldg(p), __ldg(p + 1), __ldg(p + 2)); }
 template <bool COUNT, int F>
-__global__ void __launch_bounds__(128, (F == TF_ALL) ? DRT_LIGHT_MINBLOCKS : (F == TF_LITERAL1) ? DRT_L1_MINBLOCKS : DRT_LLIGHT_MINBLOCKS)
+__global__ void __launch_bounds__(128, lightMinBlocks(F))
 k_light(const __grid_constant__ DScene S, Wave w, const SurfRec* __restrict__ surf, NodeRec* __restrict__ nodesBase, Counters* ctr, const uint32_t* __restrict__ work, uint32_t* __restrict__ deferOut) {
   const long long n = work ? (long long)ctr->deferLight[w.level] : waveCount(w, ctr);
   NodeRec* __restrict__ nodes = nodesBase + ((w.level == 0) ? 0 : waveNodeOffset(w, ctr, w.level));
@@ -442,10 +464,10 @@ __global__ void k_nodes32(const FNode* __restrict__ in, long long n, FNode32* __
 }
 
 // caller ray queries (drt_query_closest / drt_query_occluded) -----------------------------------------------------
-// One thread = one caller ray (FP64 origin and direction, 3 doubles each, ray time 0).  F / work / deferOut as in k_trace: the scene's lean
-// variant defers what it cannot serve to `deferOut` (count in Counters::deferTrace[0] / deferLight[0]), the generic variant serves everything
-// and is the fix-up pass over that list.  A ray is traced only if origin and direction are finite and the direction's FP64 length is finite
-// and nonzero; any other ray is a miss / not occluded.
+// One thread = one caller ray (FP64 origin and direction, 3 doubles each, ray time 0), through rayLoop: the scene's lean variant defers what
+// it cannot serve to `deferOut` (count in Counters::deferTrace[0] / deferLight[0]), the generic variant serves everything and is the fix-up
+// pass over that list.  A ray is traced only if origin and direction are finite and the direction's FP64 length is finite and nonzero; any
+// other ray is a miss / not occluded.
 __device__ __forceinline__ bool queryRay(const double* __restrict__ org, const double* __restrict__ dir, long long i, Ray& ray) {
   const D3 o = d3(org[3 * i], org[3 * i + 1], org[3 * i + 2]), d = d3(dir[3 * i], dir[3 * i + 1], dir[3 * i + 2]);
   const double m = mag3(d);
@@ -453,71 +475,50 @@ __device__ __forceinline__ bool queryRay(const double* __restrict__ org, const d
   ray = makeRay(o, norm3(d)); return true;
 }
 // closest hit, reported as a miss unless t < tmax[i] (tmax == null: +inf).  The search itself is the unbounded one.  pos / nrm (optional): the
-// world hit point and unit normal k_shade shades with (0 on a miss)
+// world hit point and unit normal k_shade shades with (0 on a miss).  k_query_closest<TF_ALL> is also the drt_trace_rays probe.
 template <int F>
-__global__ void __launch_bounds__(128, (F == TF_ALL) ? DRT_TRACE_MINBLOCKS : (F == TF_LITERAL1) ? DRT_L1_MINBLOCKS : DRT_LTRACE_MINBLOCKS)
+__global__ void __launch_bounds__(128, traceMinBlocks(F))
 k_query_closest(const __grid_constant__ DScene S, long long nRays, const double* __restrict__ org, const double* __restrict__ dir, const double* __restrict__ tmax,
                 int32_t* __restrict__ ids, double* __restrict__ tOut, double* __restrict__ pos, double* __restrict__ nrm, Counters* ctr, const uint32_t* __restrict__ work, uint32_t* __restrict__ deferOut) {
-  const long long n = work ? (long long)ctr->deferTrace[0] : nRays;
-  if (work && n > 0 && blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&ctr->deferredTotal, (unsigned long long)n);
-  for (long long base = (long long)blockIdx.x * blockDim.x; base < n; base += (long long)gridDim.x * blockDim.x) {
-    long long i = base + threadIdx.x; bool defer = false;
-    if (i < n) {
-      if (work) i = work[i];
-      Hit h; hitReset(h); Ray ray;
-      if (queryRay(org, dir, i, ray)) {
-        const int got = closestHitT<F>(S, ray, 0.0, h, nullptr);
-        if (F != TF_ALL && got < 0) defer = true;
-      }
-      if (!defer) {
-        const bool hit = h.prim >= 0 && (!tmax || h.t < tmax[i]);
-        ids[2 * i] = hit ? S.prims[h.prim].serial : -1; ids[2 * i + 1] = hit ? h.inst : -1; tOut[i] = hit ? h.t : 0;
-        if (pos || nrm) {
-          D3 p = d3(0, 0, 0), q = p;
-          if (hit) {
-            const FPrim P = S.prims[h.prim]; const FXform& X = S.xforms[h.hitXform];
-            p = xfPoint(X.m, h.loc); q = norm3(xfVector(X.adj, primNormal(S, P, h.loc, h.arg0, h.arg1, h.state)));
-          }
-          if (pos) { pos[3 * i] = p.x; pos[3 * i + 1] = p.y; pos[3 * i + 2] = p.z; }
-          if (nrm) { nrm[3 * i] = q.x; nrm[3 * i + 1] = q.y; nrm[3 * i + 2] = q.z; }
+  rayLoop<F>(nRays, work, &ctr->deferTrace[0], deferOut, ctr, [&](long long i) __attribute__((always_inline)) {
+    Hit h; hitReset(h); Ray ray; bool defer = false;
+    if (queryRay(org, dir, i, ray)) {
+      const int got = closestHitT<F>(S, ray, 0.0, h, nullptr);
+      if (F != TF_ALL && got < 0) defer = true;
+    }
+    if (!defer) {
+      const bool hit = h.prim >= 0 && (!tmax || h.t < tmax[i]);
+      ids[2 * i] = hit ? S.prims[h.prim].serial : -1; ids[2 * i + 1] = hit ? h.inst : -1; tOut[i] = hit ? h.t : 0;
+      if (pos || nrm) {
+        D3 p = d3(0, 0, 0), q = p;
+        if (hit) {
+          const FPrim P = S.prims[h.prim]; const FXform& X = S.xforms[h.hitXform];
+          p = xfPoint(X.m, h.loc); q = norm3(xfVector(X.adj, primNormal(S, P, h.loc, h.arg0, h.arg1, h.state)));
         }
+        if (pos) { pos[3 * i] = p.x; pos[3 * i + 1] = p.y; pos[3 * i + 2] = p.z; }
+        if (nrm) { nrm[3 * i] = q.x; nrm[3 * i + 1] = q.y; nrm[3 * i + 2] = q.z; }
       }
     }
-    if (F != TF_ALL) deferAppend(defer, (uint32_t)i, &ctr->deferTrace[0], deferOut);
-  }
+    return defer;
+  });
 }
 // occlusion: the renderer's shadow test (anyHitT: something hit with (dist - t) > DRT_EPS).  dist may be +inf; a NaN dist is not occluded
 template <int F>
-__global__ void __launch_bounds__(128, (F == TF_ALL) ? DRT_LIGHT_MINBLOCKS : (F == TF_LITERAL1) ? DRT_L1_MINBLOCKS : DRT_LLIGHT_MINBLOCKS)
+__global__ void __launch_bounds__(128, lightMinBlocks(F))
 k_query_any(const __grid_constant__ DScene S, long long nRays, const double* __restrict__ org, const double* __restrict__ dir, const double* __restrict__ dist,
             uint8_t* __restrict__ occluded, Counters* ctr, const uint32_t* __restrict__ work, uint32_t* __restrict__ deferOut) {
-  const long long n = work ? (long long)ctr->deferLight[0] : nRays;
-  if (work && n > 0 && blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&ctr->deferredTotal, (unsigned long long)n);
-  for (long long base = (long long)blockIdx.x * blockDim.x; base < n; base += (long long)gridDim.x * blockDim.x) {
-    long long i = base + threadIdx.x; bool defer = false;
-    if (i < n) {
-      if (work) i = work[i];
-      const double d = dist[i]; int got = 0; Ray ray;
-      if (d == d && queryRay(org, dir, i, ray)) {
-        got = anyHitT<F>(S, ray, 0.0, d, nullptr);
-        if (F != TF_ALL && got < 0) defer = true;
-      }
-      if (!defer) occluded[i] = got > 0 ? 1 : 0;
+  rayLoop<F>(nRays, work, &ctr->deferLight[0], deferOut, ctr, [&](long long i) __attribute__((always_inline)) {
+    const double d = dist[i]; int got = 0; Ray ray; bool defer = false;
+    if (d == d && queryRay(org, dir, i, ray)) {
+      got = anyHitT<F>(S, ray, 0.0, d, nullptr);
+      if (F != TF_ALL && got < 0) defer = true;
     }
-    if (F != TF_ALL) deferAppend(defer, (uint32_t)i, &ctr->deferLight[0], deferOut);
-  }
+    if (!defer) occluded[i] = got > 0 ? 1 : 0;
+    return defer;
+  });
 }
 
-// parity helpers ------------------------------------------------------------------------------------------------
-template <bool COUNT>
-__global__ void k_trace_explicit(const __grid_constant__ DScene S, long long n, const double* __restrict__ org, const double* __restrict__ dir, int32_t* __restrict__ ids, double* __restrict__ tOut) {
-  long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; if (i >= n) return;
-  Ray ray = makeRay(d3(org[3 * i], org[3 * i + 1], org[3 * i + 2]), norm3(d3(dir[3 * i], dir[3 * i + 1], dir[3 * i + 2])));
-  TraceCounters tc; tc.box = 0; tc.prim = 0;
-  Hit h; closestHit(S, ray, 0.0, h, COUNT ? &tc : nullptr);
-  if (COUNT && tc.box == 0xFFFFFFFFFFFFull) ids[0] = 0;
-  ids[2 * i] = h.prim >= 0 ? S.prims[h.prim].serial : -1; ids[2 * i + 1] = h.prim >= 0 ? h.inst : -1; tOut[i] = h.prim >= 0 ? h.t : 0;
-}
+// parity helper ------------------------------------------------------------------------------------------------
 __global__ void k_eval_texture(const __grid_constant__ DScene S, int shader, long long n, const double* __restrict__ hl, const double* __restrict__ fl, double* __restrict__ out) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; if (i >= n) return;
   FPrim P; P.type = PT_BOX; P.flags = 0; P.xform = 0; P.shader = shader; P.data = 0; P.serial = 0; P.pad0 = P.pad1 = 0;   // no image textures through this probe
@@ -567,6 +568,8 @@ struct Renderer::Impl {
   DBuf<uint32_t> deferT, deferL;                 // deferral lists of the lean trace / light kernels (ray indices of one level)
   std::vector<DEvent> evPool;                    // stage timing of a whole frame without a host sync per level
   int shape = TF_ALL;                            // kernel variant the uploaded scene runs with (see chooseShape)
+  // the lean kernel of a pass for `shape`, given its F = 0 and F = TF_LITERAL1 instances; null when only the generic kernel serves the scene
+  template <class K> K lean(K shape0, K literal1) const { return shape == TF_ALL ? nullptr : shape == 0 ? shape0 : literal1; }
   bool anySecondary = false;                     // some shader can spawn reflection / refraction rays
   int depthHint = 0;                             // levels the last frame of this scene needed (0 = unknown: launch the full depth)
   double capHint = 0;                            // queue-capacity factor the last frame of this scene ended up with (0 = default)
@@ -726,9 +729,8 @@ void Renderer::renderChunks(long long pix0, long long pix1, int world, int rank,
   // kernels of the closest-hit and light passes: the generic kernel alone (counters on, or a scene shape only it serves), or a lean variant
   // followed by the generic kernel as the fix-up pass over what the lean one deferred
   using TraceK = decltype(&k_trace<false, TF_ALL>); using LightK = decltype(&k_light<false, TF_ALL>);
-  const bool generic = counters_ || I.shape == TF_ALL;
-  const TraceK traceAll = counters_ ? &k_trace<true, TF_ALL> : &k_trace<false, TF_ALL>, traceLean = generic ? nullptr : I.shape == 0 ? &k_trace<false, 0> : &k_trace<false, TF_LITERAL1>;
-  const LightK lightAll = counters_ ? &k_light<true, TF_ALL> : &k_light<false, TF_ALL>, lightLean = generic ? nullptr : I.shape == 0 ? &k_light<false, 0> : &k_light<false, TF_LITERAL1>;
+  const TraceK traceAll = counters_ ? &k_trace<true, TF_ALL> : &k_trace<false, TF_ALL>, traceLean = counters_ ? nullptr : I.lean(&k_trace<false, 0>, &k_trace<false, TF_LITERAL1>);
+  const LightK lightAll = counters_ ? &k_light<true, TF_ALL> : &k_light<false, TF_ALL>, lightLean = counters_ ? nullptr : I.lean(&k_light<false, 0>, &k_light<false, TF_LITERAL1>);
   long long batchRays = batchRays_; int levels = (I.depthHint > 0) ? std::min(fullDepth, I.depthHint + 1) : fullDepth;
   // queue capacity of a level relative to the batch's primary rays.  2 is the true bound for level 1 and ample for every shipped scene; the true
   // bound of level L is 2^L (binary Fresnel splits), so an overflow doubles the factor (and halves the batch: same memory) and renders again
@@ -746,7 +748,7 @@ void Renderer::renderChunks(long long pix0, long long pix1, int world, int rank,
     const long long nodeCap = (levels > 1) ? maxN0 + ((capFactor >= 64.0) ? 126 * maxN0 : std::max<long long>(64, (long long)(3.0 * capFactor * (double)maxN0))) : maxN0;
     I.hits0.ensure(maxN0, st); I.surf.ensure(std::max(maxN0, rayCap), st); I.nodes.ensure(nodeCap, st);
     if (levels > 1) { I.rays[0].ensure(rayCap, st); I.rays[1].ensure(rayCap, st); I.hits.ensure(rayCap, st); }
-    if (!generic) { I.deferT.ensure(std::max(maxN0, rayCap), st); I.deferL.ensure(std::max(maxN0, rayCap), st); }
+    if (traceLean) { I.deferT.ensure(std::max(maxN0, rayCap), st); I.deferL.ensure(std::max(maxN0, rayCap), st); }
     const unsigned persist = (unsigned)std::min<long long>(gridFor(rayCap, 128), (long long)I.numSMs * 16), fixGrid = (unsigned)I.numSMs * 4;
     devErrorReset(st);
     CK(cudaMemsetAsync(I.ctr, 0, sizeof(Counters), st));
@@ -884,10 +886,13 @@ long long Renderer::probeFastBvh(int fastIndex, std::vector<FTri>& tris, std::ve
 void Renderer::accelInfo(double out[4]) const { out[0] = impl_->lbvhMs; out[1] = (double)impl_->lbvhTris; out[2] = (double)impl_->lbvhNodes; out[3] = (double)impl_->sceneBytes; }
 long long Renderer::getPhotons(double* out6Host, long long cap) { CK(cudaSetDevice(device_)); return impl_->photons.download(out6Host, cap, (cudaStream_t)stream_); }
 
+// parity probe of the closest-hit search: host arrays through the generic query kernel alone (no tmax, hit point or normal, no deferral)
 void Renderer::traceRays(long long n, const double* orgHost, const double* dirHost, int32_t* idsHost, double* tHost) {
-  CK(cudaSetDevice(device_)); cudaStream_t st = (cudaStream_t)stream_; const auto k = counters_ ? &k_trace_explicit<true> : &k_trace_explicit<false>;
-  probe(*impl_, st, n, {{orgHost, 3}, {dirHost, 3}}, {{idsHost, 1}, {tHost, 1}},       // ids: two int32 per ray
-        [&](double* const* in, double* const* o) { k<<<gridFor(n, 128), 128, 0, st>>>(impl_->ds, n, in[0], in[1], reinterpret_cast<int32_t*>(o[0]), o[1]); });
+  CK(cudaSetDevice(device_)); cudaStream_t st = (cudaStream_t)stream_; Impl& I = *impl_;
+  probe(I, st, n, {{orgHost, 3}, {dirHost, 3}}, {{idsHost, 1}, {tHost, 1}},       // ids: two int32 per ray
+        [&](double* const* in, double* const* o) {
+          k_query_closest<TF_ALL><<<gridFor(n, 128), 128, 0, st>>>(I.ds, n, in[0], in[1], nullptr, reinterpret_cast<int32_t*>(o[0]), o[1], nullptr, nullptr, I.ctr, nullptr, nullptr);
+        });
 }
 // Caller rays against the uploaded scene, device arrays in and out.  The rays run through the scene's kernel variant (Impl::shape) with the
 // generic kernel as the fix-up pass, in launches of at most 2^31 - 1 rays (the deferral list holds 32-bit indices); one host sync at the end,
@@ -918,8 +923,7 @@ template <class L> static void runQuery(Renderer::Impl& I, cudaStream_t st, long
 }
 void Renderer::queryClosest(long long n, const double* org, const double* dir, const double* tmax, int32_t* ids, double* t, double* pos, double* nrm, RenderStats* stats) {
   CK(cudaSetDevice(device_)); Impl& I = *impl_; cudaStream_t st = (cudaStream_t)stream_;
-  using K = decltype(&k_query_closest<TF_ALL>);
-  const K all = &k_query_closest<TF_ALL>, lean = I.shape == TF_ALL ? nullptr : I.shape == 0 ? &k_query_closest<0> : &k_query_closest<TF_LITERAL1>;
+  const auto all = &k_query_closest<TF_ALL>, lean = I.lean(&k_query_closest<0>, &k_query_closest<TF_LITERAL1>);
   runQuery(I, st, n, I.deferT, lean != nullptr, &RenderStats::msTrace, stats, [&](const PassLauncher& pass, long long i0, long long m) {
     pass("k_query_closest", 0, lean, all, I.deferT.p, gridFor(m, 128), I.ds, m, org + 3 * i0, dir + 3 * i0, tmax ? tmax + i0 : nullptr, ids + 2 * i0, t + i0,
          pos ? pos + 3 * i0 : nullptr, nrm ? nrm + 3 * i0 : nullptr, I.ctr);
@@ -927,8 +931,7 @@ void Renderer::queryClosest(long long n, const double* org, const double* dir, c
 }
 void Renderer::queryOccluded(long long n, const double* org, const double* dir, const double* dist, uint8_t* occluded, RenderStats* stats) {
   CK(cudaSetDevice(device_)); Impl& I = *impl_; cudaStream_t st = (cudaStream_t)stream_;
-  using K = decltype(&k_query_any<TF_ALL>);
-  const K all = &k_query_any<TF_ALL>, lean = I.shape == TF_ALL ? nullptr : I.shape == 0 ? &k_query_any<0> : &k_query_any<TF_LITERAL1>;
+  const auto all = &k_query_any<TF_ALL>, lean = I.lean(&k_query_any<0>, &k_query_any<TF_LITERAL1>);
   runQuery(I, st, n, I.deferL, lean != nullptr, &RenderStats::msLight, stats, [&](const PassLauncher& pass, long long i0, long long m) {
     pass("k_query_any", 0, lean, all, I.deferL.p, gridFor(m, 128), I.ds, m, org + 3 * i0, dir + 3 * i0, dist + i0, occluded + i0, I.ctr);
   });

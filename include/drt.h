@@ -146,6 +146,8 @@ int drt_query_closest(drt_ctx* ctx, int64_t n, const double* org3, const double*
 int drt_query_occluded(drt_ctx* ctx, int64_t n, const double* org3, const double* dir3, const double* dist, uint8_t* occluded, drt_stats* stats);
 
 /* ---- parity probes (used by tests; not needed by a host) ---- */
+/* drt_trace_rays: drt_query_closest's generic kernel on HOST arrays, without tmax, pos3 / nrm3 or the lean kernel variants: the same ids2 and
+ * t.  So a ray whose origin or direction is not finite, or whose direction has a zero (or non-finite) FP64 length, is a miss (-1, -1, 0). */
 int drt_trace_rays(drt_ctx* ctx, int64_t n, const double* org, const double* dir, int32_t* ids2, double* t);
 int drt_eval_texture(drt_ctx* ctx, int32_t shader_serial, int64_t n, const double* hit_loc, const double* fwd_loc, double* rgb);
 int64_t drt_dump_bvh(drt_ctx* ctx, int32_t top_index, int32_t* out, int64_t cap, double* root_box6);

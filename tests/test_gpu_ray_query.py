@@ -293,8 +293,9 @@ def test_edges_and_return_codes(drt, gpu_ctx_factory, monkeypatch):
     org = np.array([[0, 0, 0], [nan, 0, 0], [0, inf, 0], [0, 0, 0], [0, 0, 0], [0, 0, 0], [0, 0, 0], [0, 0, 0], [0, 0, 0]], dtype=np.float64)
     d = np.array([[0, 0, -1], [0, 0, -1], [0, 0, -1], [0, 0, 0], [nan, 0, -1], [0, -inf, -1], [1e-300, 0, -1e-300], [1e300, 0, -1e300], [0, 0, -1]], dtype=np.float64)
     (ids, t, pos, nrm), _ = query(drt, s, org, d, frame=True)
-    pi, pt = s.trace_rays(org[:1], d[:1])
-    assert pi[0, 0] >= 0 and np.array_equal(ids[0], pi[0]) and np.array_equal(ids[-1], pi[0]) and t[0] == pt[0] == t[-1]
+    pi, pt = s.trace_rays(org, d)          # the probe follows the same rule: every ray, traced or not, gives the query's ids and t
+    assert np.array_equal(ids, pi) and np.array_equal(t.view(np.int64), pt.view(np.int64))
+    assert pi[0, 0] >= 0 and np.array_equal(ids[-1], pi[0]) and t[0] == pt[0] == t[-1]
     assert np.all(ids[1:-1] == -1) and np.all(t[1:-1] == 0) and np.all(pos[1:-1] == 0) and np.all(nrm[1:-1] == 0)
     dist = np.full(len(org), np.inf); dist[-1] = nan           # the last ray is a normal one, but a NaN distance is not occluded
     occ, _ = occl(drt, s, org, d, dist)
